@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...   # the reference's CPU path (oracle port)
+    python bench.py ... --dump-outputs DIR                    # also write the last timed step's outputs to DIR/*.npy
 
 A "step" is one pass of the depth-guidance hot path (reference mask2former/utils/custom_model.py:324-355:
 ratio predictor -> depth decomposition -> 3 DSAM stages -> DGGM injection + branch sum) over one batch of
@@ -21,8 +22,10 @@ configs[3] restricted to the hot path (fwd + bwd + NCCL gradient all-reduce, bat
 from __future__ import annotations
 
 import argparse
+import ctypes
 import json
 import os
+import signal
 import subprocess
 import sys
 import tempfile
@@ -48,6 +51,7 @@ FLOP_DSAM = sum(5 * 2.0 * (H // (2 * s)) * (W // (2 * s)) * co * 9 * ci
 FEAT_ELEMS = sum(c * (H // s) * (W // s) for c, s in zip(CHANS, STRIDES))      # 3 456 000
 BYTES_DGGM = 3 * 4 * FEAT_ELEMS + 4 * 4 * H * W               # read colour + branch-1, write fused, read grad+mask
 POST_THRESHOLD = 0.0     # the reference's Evaluator(threshold=0.0) (finetuning.py:95): every candidate segment is painted
+DUMP_BYTES = 64 * 10**6  # --dump-outputs writes at most this much in all
 
 
 WORKLOAD = "configs[1]: batch-32/GPU inference, 480x640 RGB-D, Swin-T pyramid, depth-guidance hot path"
@@ -185,7 +189,7 @@ def run_reference(args):
         return
     steps, warmup = max(args.steps, 1), max(args.warmup, 1)
     base, sec_per_step = cpu_hot_path(steps, warmup)
-    whole, whole_sec = cpu_whole_model(min(steps, 10), min(warmup, 2))
+    whole, whole_sec = cpu_whole_model(steps, min(warmup, 2))
     line = {
         "impl": "reference", "metric": METRIC, "value": base["value"], "unit": UNIT, "n_gpus": args.gpus,
         "steps": args.steps, "warmup": args.warmup, "ms_per_step": sec_per_step * 1e3, "higher_is_better": True,
@@ -204,6 +208,9 @@ def run_reference(args):
 # --------------------------------------------------------------------------------------------------------
 # own arm
 # --------------------------------------------------------------------------------------------------------
+PR_SET_PDEATHSIG = 1     # prctl(2) option: signal this process when its parent ends
+
+
 class ClockSampler:
     def __init__(self, index: int):
         self.index = index
@@ -211,9 +218,15 @@ class ClockSampler:
         q = ("index,clocks.sm,clocks.max.sm,power.draw,clocks_event_reasons.hw_slowdown,"
              "clocks_event_reasons.hw_thermal_slowdown,clocks_event_reasons.sw_thermal_slowdown,"
              "clocks_event_reasons.sw_power_cap")
+        prctl, parent = ctypes.CDLL(None, use_errno=True).prctl, os.getpid()
+
+        def die_with_parent():                 # in the child, before exec: SIGKILL when bench.py ends, however it ends
+            prctl(PR_SET_PDEATHSIG, signal.SIGKILL)
+            if os.getppid() != parent:         # bench.py ended before the line above took effect
+                os._exit(1)
         try:
             self.p = subprocess.Popen(["nvidia-smi", f"--query-gpu={q}", "--format=csv,noheader,nounits", "-lms", "50",
-                                       "-i", str(index)], stdout=self.f, stderr=subprocess.DEVNULL)
+                                       "-i", str(index)], stdout=self.f, stderr=subprocess.DEVNULL, preexec_fn=die_with_parent)
         except OSError:
             self.p = None
 
@@ -350,9 +363,11 @@ def run_own(args):
     barrier()
     e0.record()
     for _ in range(args.steps):
-        step()
+        fused = step()
     e1.record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, fused)
     launches = launches_per_step * args.steps          # kernels of this library executed inside the timed region
     elapsed = parallel.max_over_ranks(e0.elapsed_time(e1) / 1e3, dev)
     value = frames_per_step * args.steps / elapsed
@@ -366,11 +381,11 @@ def run_own(args):
             g1()
         torch.cuda.synchronize()
         e0.record()
-        for _ in range(20):
+        for _ in range(args.steps):
             g1()
         e1.record()
         torch.cuda.synchronize()
-        latency = {"batch": 1, "ms_per_frame": e0.elapsed_time(e1) / 20, "launch": "CUDA graph replay"}
+        latency = {"batch": 1, "ms_per_frame": e0.elapsed_time(e1) / args.steps, "steps": args.steps, "launch": "CUDA graph replay"}
         del g1
     except Exception as e:                                   # reported, never fatal
         latency = {"error": repr(e)}
@@ -518,7 +533,7 @@ def run_own(args):
     # ---- the decoder_ops kernels at this workload's shapes (live CUDA-event timings; reported, never part of `value`)
     if not args.no_whole_model:
         try:
-            extra.extend(decoder_ops_rooflines(B, pkv, dev))
+            extra.extend(decoder_ops_rooflines(B, pkv, dev, args.steps))
         except Exception as e:                               # reported, never fatal for the headline line
             extra.append({"kernel": "decoder_ops kernels", "error": repr(e)})
 
@@ -570,6 +585,21 @@ def run_own(args):
         emit(line)
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir: str, fused) -> None:
+    """--dump-outputs: what the last timed step returned -- the four fused feature maps handed to the pixel decoder -- as
+    float32 ``fused<i>.npy``.  A map larger than its share of DUMP_BYTES is stored as a fixed sample of its elements (flat
+    indices drawn from a generator seeded with ``i``, in increasing order), so runs with the same arguments store the same
+    elements."""
+    os.makedirs(out_dir, exist_ok=True)
+    per_map = (DUMP_BYTES // len(fused) - 128) // 4          # elements; 128 bytes of .npy header
+    for i, t in enumerate(fused):
+        t = t.detach()
+        if t.numel() > per_map:
+            idx = np.sort(np.random.default_rng(i).choice(t.numel(), per_map, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(out_dir, f"fused{i}.npy"), t.float().cpu().numpy())
 
 
 def hot_path_host_features(args, model, B, rgb_host, depth_host, feats, pv, dev, barrier, world, frames_per_step):
@@ -766,7 +796,7 @@ def train_whole_model_record(args, dev, rank, world, barrier):
         return out.loss
 
     import warnings
-    steps = max(3, min(args.steps, 5))
+    steps = args.steps
     with warnings.catch_warnings():
         warnings.simplefilter("ignore")
         for _ in range(2):
@@ -795,7 +825,7 @@ def train_whole_model_record(args, dev, rank, world, barrier):
                         "labels, HF Mask2FormerLoss, bucketed NCCL gradient all-reduce overlapped with the backward, AdamW"}
 
 
-def decoder_ops_rooflines(B, pkv, dev):
+def decoder_ops_rooflines(B, pkv, dev, steps):
     """Live timings of the decoder_ops kernels that carry most bytes, at the shapes the whole model gives them for this workload
     (deformable attention of the pixel decoder's three coarse levels; LayerNorm of the pixel decoder's token stream)."""
     from rgbd_b200 import functional as Fn
@@ -809,7 +839,7 @@ def decoder_ops_rooflines(B, pkv, dev):
     x = torch.randn(B * S, 256, device=dev, generator=g)
     w, b = torch.ones(256, device=dev), torch.zeros(256, device=dev)
 
-    def timed(fn, n=10):
+    def timed(fn, n=steps):
         fn()
         torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -838,7 +868,7 @@ class PerKernel:
     """Times the stages of one hot-path step separately with CUDA events (same inputs, same stream)."""
 
     def __init__(self, model, pv, feats, steps):
-        self.m, self.pv, self.feats, self.steps = model, pv, feats, max(steps, 3)
+        self.m, self.pv, self.feats, self.steps = model, pv, feats, steps
 
     def _time(self, fn):
         fn()
@@ -941,7 +971,14 @@ def main():
     ap.add_argument("--no-graph", dest="graph", action="store_false",
                     help="launch the ~22 kernels of a step one by one instead of replaying the step as one CUDA graph")
     ap.set_defaults(graph=True)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the fused feature maps of the last one as DIR/fused<i>.npy (float32; "
+                         "rank 0; a seeded sample of each map's elements where all of them would pass 64 MB in total)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "own":
+        ap.error("--dump-outputs writes the outputs of this repo's CUDA path (--impl own)")
     set_workload(args.workload)
     args.batch = args.batch or BATCH
     if args.impl == "reference":

@@ -20,6 +20,37 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REF = "/root/reference"
 GOLD = os.path.join(ROOT, "tests", "golden")
+# Every wiring golden is computed from the same colour-encoder features (one seed, one config) and both depth-encoder versions
+# from the same depth-encoder features: each set is stored once, beside the per-version outputs, so no file grows past 1 MB.
+WIRING_INPUTS = {"feat": "wiring_feat.npz", "dfeat": "wiring_dfeat.npz"}
+
+
+def save_wiring(name, out, gold=GOLD):
+    """Write the wiring golden ``name`` (``fused*``, ``ratios``) and the encoder features (``feat*``, ``dfeat*``) in ``out``.
+    Features already stored by another wiring golden must be equal to the ones given here: the other goldens' outputs were
+    computed from them."""
+    out = dict(out)
+    for prefix, shared in WIRING_INPUTS.items():
+        feats = {k: out.pop(k) for k in [k for k in out if k.rstrip("0123456789") == prefix]}
+        if not feats:
+            continue
+        path = os.path.join(gold, shared)
+        if os.path.exists(path):
+            old = np.load(path)
+            if sorted(old.files) != sorted(feats) or not all(np.array_equal(old[k], v) for k, v in feats.items()):
+                raise ValueError(f"{name}: its {prefix}* differ from those in {shared}, which other wiring goldens were made "
+                                 f"from; remove {shared} and regenerate every wiring golden")
+        else:
+            np.savez_compressed(path, **feats)
+    np.savez_compressed(os.path.join(gold, name), **out)
+
+
+def load_wiring(gold, name):
+    """The wiring golden ``name`` together with the encoder features it was computed from (``feat*``, ``dfeat*``)."""
+    g = dict(np.load(os.path.join(gold, name)))
+    for shared in WIRING_INPUTS.values():
+        g.update(np.load(os.path.join(gold, shared)))
+    return g
 
 
 def import_reference():
@@ -193,7 +224,7 @@ def main():
     for i in range(4):
         out[f"feat{i}"] = captured["feats"][i].numpy()
         out[f"fused{i}"] = captured["fused"][i].numpy()
-    np.savez_compressed(os.path.join(GOLD, "wiring.npz"), **out)
+    save_wiring("wiring.npz", out)
     # ---- 8. other version branches that reuse DGGM / DSAM (CM:156-163, CM:234-256) ---------------------------
     for version, nch in (("0.0.3", 7), ("0.1.2", 6)):
         torch.manual_seed(42)
@@ -214,7 +245,7 @@ def main():
         for i in range(4):
             out[f"feat{i}"] = cap["feats"][i].numpy()
             out[f"fused{i}"] = cap["fused"][i].numpy()
-        np.savez_compressed(os.path.join(GOLD, f"wiring_v{version.replace('.', '')}.npz"), **out)
+        save_wiring(f"wiring_v{version.replace('.', '')}.npz", out)
     for f in sorted(os.listdir(GOLD)):
         print(f, os.path.getsize(os.path.join(GOLD, f)))
 

@@ -1,6 +1,7 @@
 """Golden vectors of the version 0.1.3 / 0.3.0 branches (CM:258-322) from the REFERENCE module itself ->
-tests/golden/wiring_v013.npz, wiring_v030.npz: colour-encoder features, depth-encoder features, predicted ratios and the
-list handed to the pixel decoder.  Run in the build container: ``python oracle/make_golden_versions.py``."""
+tests/golden/wiring_v013.npz, wiring_v030.npz: predicted ratios and the list handed to the pixel decoder; the colour- and
+depth-encoder features go to the shared wiring_feat.npz / wiring_dfeat.npz.  Run where the reference project is importable:
+``python oracle/make_golden_versions.py``."""
 import os
 import sys
 
@@ -9,7 +10,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-from oracle.make_golden import GOLD, REF, import_reference, load_pkg      # noqa: E402
+from oracle.make_golden import GOLD, REF, import_reference, load_pkg, save_wiring      # noqa: E402
 
 
 def main():
@@ -45,7 +46,7 @@ def main():
             out[f"dfeat{i}"] = cap["dfeats"][i].numpy()
             out[f"fused{i}"] = cap["fused"][i].numpy()
         path = os.path.join(GOLD, f"wiring_v{version.replace('.', '')}.npz")
-        np.savez_compressed(path, **out)
+        save_wiring(os.path.basename(path), out)
         print(path, os.path.getsize(path), out["ratios"].ravel())
 
 

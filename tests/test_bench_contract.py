@@ -29,13 +29,38 @@ def test_reference_arm_prints_one_contract_line():
     assert d["value"] > 0 and "workload" in d["config"] and "model" not in d["config"]
 
 
+import numpy as np  # noqa: E402
 import pytest  # noqa: E402
+import torch  # noqa: E402
+
+
+def test_dump_outputs_keeps_to_64_mb_and_stores_the_same_elements_every_run(tmp_path):
+    """--dump-outputs: float32 files, at most 64 MB in all; maps that fit whole, larger ones as a fixed sample.  Each map holds
+    its own flat indices, so a sample shows which elements it kept."""
+    import bench
+    B = 8
+    fused = [torch.arange(B * c * (bench.H // s) * (bench.W // s), dtype=torch.float32).view(B, c, bench.H // s, bench.W // s)
+             for c, s in zip(bench.CHANS, bench.STRIDES)]
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), fused)
+    assert sorted(p.name for p in (tmp_path / "a").iterdir()) == [f"fused{i}.npy" for i in range(4)]
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= 64 * 10**6
+    whole = []
+    for i, t in enumerate(fused):
+        a, b = np.load(tmp_path / "a" / f"fused{i}.npy"), np.load(tmp_path / "b" / f"fused{i}.npy")
+        assert a.dtype == np.float32 and np.array_equal(a, b)
+        whole.append(a.shape == tuple(t.shape))
+        if whole[-1]:
+            assert np.array_equal(a, t.numpy())
+        else:
+            assert a.ndim == 1 and 0 < a.size < t.numel() and (np.diff(a) > 0).all() and 0 <= a[0] and a[-1] < t.numel()
+    assert whole == [False, False, True, True]
 
 
 @pytest.mark.gpu
-def test_own_arm_prints_one_contract_line():
+def test_own_arm_prints_one_contract_line(tmp_path):
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "3", "--warmup", "3", "--batch", "4",
-                        "--cpu-steps", "1"], capture_output=True, text=True, timeout=900, cwd=ROOT)
+                        "--cpu-steps", "1", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=900, cwd=ROOT)
     assert r.returncode == 0, r.stderr[-3000:]
     lines = [ln for ln in r.stdout.splitlines() if ln.strip()]
     assert len(lines) == 1, lines
@@ -60,3 +85,7 @@ def test_own_arm_prints_one_contract_line():
     tr = d["train"]
     assert tr["value"] > 0 and tr["batch_per_gpu"] == 8 and tr["ms_per_step"] > 0
     assert cb["detail"]["hot_path_1_thread_frames_per_s"] > 0 and cb["detail"]["whole_model_plus_postprocess_frames_per_s"] > 0
+    # --dump-outputs: the last timed step's four fused maps (batch 4: the largest as a sample, the others whole)
+    dumped = [np.load(tmp_path / f"fused{i}.npy") for i in range(4)]
+    assert [a.shape for a in dumped[1:]] == [(4, c, 480 // s, 640 // s) for c, s in ((192, 8), (384, 16), (768, 32))]
+    assert dumped[0].ndim == 1 and all(a.dtype == np.float32 and np.isfinite(a).all() for a in dumped)

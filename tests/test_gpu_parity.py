@@ -13,7 +13,7 @@ import rgbd_b200  # noqa: F401
 from rgbd_b200 import synthetic
 from oracle import hotpath as O
 from oracle import weights as OW
-from oracle.make_golden import decompose_cases
+from oracle.make_golden import decompose_cases, load_wiring
 from rgbd_b200 import _lib as _rgbd_lib
 
 pytestmark = pytest.mark.gpu
@@ -507,7 +507,7 @@ def test_dsam_module_fp32_precision_mode(mods, ci, co, hw, dhw):
 
 def test_depth_guidance_fp32_precision_mode(mods, golden_dir):
     """fp32 bar of the north star (1e-4 relative) on the fused features handed to the pixel decoder."""
-    g = np.load(os.path.join(golden_dir, "wiring.npz"))
+    g = load_wiring(golden_dir, "wiring.npz")
     m = mods.DepthGuidance((96, 192, 384, 768), precision="fp32")
     m.load_state_dict(OW.guidance_weights(seed=700))
     m.cuda().eval()
@@ -546,7 +546,7 @@ def test_ratio_predictor(mods, hw):
 
 
 def test_depth_guidance_wiring(mods, golden_dir):
-    g = np.load(os.path.join(golden_dir, "wiring.npz"))
+    g = load_wiring(golden_dir, "wiring.npz")
     w = OW.guidance_weights(seed=700)
     m = mods.DepthGuidance((96, 192, 384, 768))
     missing = m.load_state_dict(w, strict=True)
@@ -666,7 +666,7 @@ def test_dsam_stage_backward(mods, fn, ci, co, hw, dhw):
 def test_depth_guidance_training_gradients(mods, golden_dir):
     """Fine-tuning semantics of CM:324-355: gradients reach all DSAM and DGGM parameters, none reach the encoder
     features or the ratio predictor (SURVEY section 8a row 10)."""
-    g = np.load(os.path.join(golden_dir, "wiring.npz"))
+    g = load_wiring(golden_dir, "wiring.npz")
     w = OW.guidance_weights(seed=700)
     m = mods.DepthGuidance((96, 192, 384, 768))
     m.load_state_dict(w)
@@ -904,7 +904,7 @@ def test_full_size_dggm_and_dsam_linearity(mods, fn, full_size):
 def test_other_version_branches(mods, golden_dir, version):
     """SURVEY section 8f-4: the version branches built from the same kernels (DGGM only / DSAM cascade only)."""
     from rgbd_b200 import pixel_level
-    g = np.load(os.path.join(golden_dir, f"wiring_v{version.replace('.', '')}.npz"))
+    g = load_wiring(golden_dir, f"wiring_v{version.replace('.', '')}.npz")
     cfg = pixel_level.swin_tiny_mask2former_config(num_labels=8)
     plm = pixel_level.CustomMask2FormerPixelLevelModule(cfg, version=version)
     w = OW.guidance_weights(seed=700)
@@ -936,7 +936,7 @@ def test_other_version_branches(mods, golden_dir, version):
 def test_depth_encoder_version_branches(mods, golden_dir, version):
     """Versions with a second (depth) encoder and the feature-based RatioPredictor (CM:258-322)."""
     from rgbd_b200 import pixel_level
-    g = np.load(os.path.join(golden_dir, f"wiring_v{version.replace('.', '')}.npz"))
+    g = load_wiring(golden_dir, f"wiring_v{version.replace('.', '')}.npz")
     cfg = pixel_level.swin_tiny_mask2former_config(num_labels=8)
     torch.manual_seed(0)         # the stock (random-init) HF pixel decoder yields NaN for some seeds at this tiny size
     plm = pixel_level.CustomMask2FormerPixelLevelModule(cfg, version=version)

@@ -195,18 +195,37 @@ def test_state_dict_keys_match_the_reference_layout():
     assert keys == ref, keys ^ ref
 
 
-def test_state_dict_keys_match_the_live_reference_modules():
+def test_state_dict_keys_match_the_live_reference_modules(golden_dir):
+    """Key -> shape / dtype of each mirror against the reference modules' tables (tests/golden/state_dict_layout.json,
+    oracle/make_golden_layout.py), and checkpoints of that layout load strictly and come back unchanged; where the
+    reference project is importable, also against the live reference modules."""
+    import json
     from oracle import make_golden as MG
+    layout = json.load(open(os.path.join(golden_dir, "state_dict_layout.json")))
+    own = {"DepthGradientInjectionResidual([96, 192, 384, 768], 3)": modules.DepthGradientInjectionResidual([96, 192, 384, 768], 3),
+           "DSAModule(96, 192, 3)": modules.DSAModule(96, 192, 3), "DSAModule(64, 64, 3)": modules.DSAModule(64, 64, 3),
+           "EnhancedDepthImageRatioPredictor(3)": modules.EnhancedDepthImageRatioPredictor(3)}
+    assert sorted(own) == sorted(layout)
+    g = torch.Generator().manual_seed(0)
+    for name, own_m in own.items():
+        b = {k: {"shape": list(v.shape), "dtype": str(v.dtype).replace("torch.", "")} for k, v in own_m.state_dict().items()}
+        assert b == layout[name], (name, set(map(str, b.items())) ^ set(map(str, layout[name].items())))
+        ckpt = {k: (torch.randn(t["shape"], generator=g) if t["dtype"] == "float32" else
+                    torch.full(t["shape"], 3, dtype=getattr(torch, t["dtype"]))) for k, t in layout[name].items()}
+        own_m.load_state_dict(ckpt)                         # strict
+        back = own_m.state_dict()
+        assert all(torch.equal(back[k], v) for k, v in ckpt.items()), name
     if not os.path.isdir(os.path.join(MG.REF, "mask2former")):
-        pytest.skip("the reference tree is only present in the build container")
+        return
     cm, _ = MG.import_reference()
     pairs = [(cm.DepthGradientInjectionResidual([96, 192, 384, 768], 3), modules.DepthGradientInjectionResidual([96, 192, 384, 768], 3)),
              (cm.DSAModule(96, 192, 3), modules.DSAModule(96, 192, 3)), (cm.DSAModule(64, 64, 3), modules.DSAModule(64, 64, 3)),
              (cm.EnhancedDepthImageRatioPredictor(3), modules.EnhancedDepthImageRatioPredictor(3))]
-    for ref_m, own_m in pairs:
+    for name, (ref_m, own_m) in zip(own, pairs):
         a = {k: tuple(v.shape) for k, v in ref_m.state_dict().items()}
         b = {k: tuple(v.shape) for k, v in own_m.state_dict().items()}
         assert a == b, (type(ref_m).__name__, set(a.items()) ^ set(b.items()))
+        assert a == {k: tuple(t["shape"]) for k, t in layout[name].items()}, name     # the stored table is the reference's
         own_m.load_state_dict(ref_m.state_dict())          # checkpoints move both ways
         ref_m.load_state_dict(own_m.state_dict())
 

@@ -9,7 +9,7 @@ import rgbd_b200  # noqa: F401
 from rgbd_b200 import synthetic
 from oracle import hotpath as O
 from oracle import weights as OW
-from oracle.make_golden import decompose_cases
+from oracle.make_golden import decompose_cases, load_wiring
 
 
 def _load(golden_dir, name):
@@ -139,7 +139,7 @@ def test_ratio_predictor(golden_dir):
 
 
 def test_wiring(golden_dir):
-    g = _load(golden_dir, "wiring.npz")
+    g = load_wiring(golden_dir, "wiring.npz")
     w = OW.guidance_weights(seed=700)
     pvs = []
     for j in range(2):
@@ -156,7 +156,7 @@ def test_wiring(golden_dir):
 
 @pytest.mark.parametrize("version", ["0.0.3", "0.1.2"])
 def test_other_version_wiring(golden_dir, version):
-    g = _load(golden_dir, f"wiring_v{version.replace('.', '')}.npz")
+    g = load_wiring(golden_dir, f"wiring_v{version.replace('.', '')}.npz")
     w = OW.guidance_weights(seed=700)
     pvs = []
     for j in range(2):
@@ -174,7 +174,7 @@ def test_other_version_wiring(golden_dir, version):
 @pytest.mark.parametrize("version", ["0.1.3", "0.3.0"])
 def test_depth_encoder_version_wiring(golden_dir, version):
     """CM:258-322: feature-based RatioPredictor -> DSAM cascade (-> DGGM on the result for 0.3.0), reference goldens."""
-    g = _load(golden_dir, f"wiring_v{version.replace('.', '')}.npz")
+    g = load_wiring(golden_dir, f"wiring_v{version.replace('.', '')}.npz")
     w = OW.guidance_weights_feature_ratio(seed=700)
     pvs = []
     for j in range(2):
