@@ -10,9 +10,7 @@ B = int(os.environ.get("B", 32))
 dev = "cuda"
 chans = [96, 192, 384, 768]
 sizes = [(120, 160), (60, 80), (30, 40)]
-variants = os.environ.get("DSAM_TMEM_VARIANTS", "0,1,0,1").split(",")
-for i, tmem in [(i, t) for t in variants for i in range(3)]:
-    os.environ["RGBD_DSAM_TMEM"] = tmem          # read by the launcher at every call (A/B in one process)
+for i in range(3):
     torch.manual_seed(i)
     m = DSAModule(chans[i], chans[i + 1]).to(dev)
     H, W = sizes[i]
@@ -34,6 +32,6 @@ for i, tmem in [(i, t) for t in variants for i in range(3)]:
         torch.cuda.synchronize()
         ms = e0.elapsed_time(e1) / n
         flops = 2.0 * B * ((H + 1) // 2) * ((W + 1) // 2) * chans[i + 1] * 45 * chans[i]
-        print(f"tmem_a={tmem} stage {i} {mode:10s} {ms*1e3:8.1f} us  {flops/ms/1e9:7.1f} TFLOP/s (useful)")
+        print(f"stage {i} {mode:10s} {ms*1e3:8.1f} us  {flops/ms/1e9:7.1f} TFLOP/s (useful)")
     out = m._stage_forward_impl(x, codes, var)
     print(f"   checksum {float(out.double().abs().sum()):.6e}")

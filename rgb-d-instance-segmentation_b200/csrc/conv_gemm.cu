@@ -21,7 +21,7 @@
 #include "common.cuh"
 #include "rgbd_b200.h"
 #include "tc_ptx.cuh"
-#include <stdlib.h>
+#include "tma_host.cuh"
 
 namespace {
 
@@ -32,6 +32,7 @@ constexpr int kThreads = 384;        // 4 control warps + 8 epilogue warps
 constexpr int kEpiThreads = 256;
 constexpr int kEpiWarps = kEpiThreads / 32;   // arrivals per CTA on tmem_empty: one per epilogue warp
 constexpr int kTmemCols = 512;
+constexpr int kAccStages = 2;        // accumulator buffers in tensor memory: the epilogue of tile t overlaps the MMAs of tile t+1
 
 struct KParams {
     int n_img, tiles_x, tiles_y, BX, BY, out_w, out_h;
@@ -63,14 +64,13 @@ struct KParams {
     const uint8_t* next_codes;
     int next_c_pad, next_n_seg, next_masked_segs;
     int c_blocks, sa_stages, a_stage_bytes;   // conv3x3_kernel: 64-channel blocks, A-ring depth, bytes per A stage
-    int acc_stages;           // accumulator buffers in tensor memory: 2 (epilogue of tile t overlaps the MMAs of tile t+1) or 1
 };
 
 struct alignas(16) SmemCtl {
     uint64_t full[kMaxStages];
     uint64_t empty[kMaxStages];
-    uint64_t tmem_full[2];
-    uint64_t tmem_empty[2];
+    uint64_t tmem_full[kAccStages];
+    uint64_t tmem_empty[kAccStages];
     uint64_t gate_full;
     uint64_t gate_empty;
     uint64_t b_full;
@@ -97,7 +97,6 @@ __device__ __forceinline__ void decode_tile(const KParams& p, int t, int& img, i
 }
 
 struct EpiCtx {
-    uint8_t* smem;
     uint8_t* s_staging;
     uint8_t* s_gate;
     SmemCtl* ctl;
@@ -106,7 +105,16 @@ struct EpiCtx {
     uint32_t tmem_base;
     int t_begin, t_end, warp, lane;   // work units [t_begin, t_end): tiles, or tile PAIRS when pair_rank >= 0
     int pair_rank;                    // -1: one CTA per tile; 0/1: rank of this CTA in a CTA pair (see pair_tile)
-    uint32_t tmem_empty_remote[2];    // shared::cluster addresses of the leader's tmem_empty barriers (0: arrive locally)
+    uint32_t tmem_empty_remote[kAccStages];   // shared::cluster addresses of the leader's tmem_empty barriers (0: arrive locally)
+};
+
+// Slot and mbarrier phase of a ring of buffers; the phase flips each time the slot wraps to 0.
+struct Ring {
+    int i = 0;
+    uint32_t ph = 0;
+    __device__ __forceinline__ void next(int n) {
+        if (++i == n) { i = 0; ph ^= 1; }
+    }
 };
 
 // tile of CTA `rank` in pair unit u: the two CTAs take adjacent M tiles of the SAME N tile (they share the B operand)
@@ -138,8 +146,8 @@ __device__ __forceinline__ void epilogue_loop(const KParams& p, const EpiCtx& c,
     const int lx = row % p.BX, ly = row / p.BX;
     const int n_chunks = p.BLOCK_N >> 5;
     const int epi_tid = (int)threadIdx.x - 128;   // 0..255
-    int as = 0;
-    uint32_t aphase = 0, gphase = 0;
+    Ring buf;                                  // accumulator buffer
+    uint32_t gphase = 0;
     float acc[8];                              // pooled-mode running sums (lane L owns column 32*k + L)
     float acc_sq[8];                           // ... of the squares (ACT 3 only; dead code otherwise)
 #pragma unroll
@@ -169,9 +177,9 @@ __device__ __forceinline__ void epilogue_loop(const KParams& p, const EpiCtx& c,
             ss_key = want;
         }
 
-        tc::mbar_wait(&ctl->tmem_full[as], aphase);
+        tc::mbar_wait(&ctl->tmem_full[buf.i], buf.ph);
         tc::tc_fence_after();
-        const uint32_t taddr0 = c.tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(as * p.BLOCK_N);
+        const uint32_t taddr0 = c.tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(buf.i * p.BLOCK_N);
 
         int key = -1;
         bool uniform = false;
@@ -395,10 +403,10 @@ __device__ __forceinline__ void epilogue_loop(const KParams& p, const EpiCtx& c,
         // ordered by the tcgen05 fence); a cluster-scope release per thread costs a MEMBAR.ALL.GPU + ERRBAR each
         __syncwarp();
         if (lane == 0) {
-            if (c.tmem_empty_remote[as]) tc::mbar_arrive_cluster_tmem(c.tmem_empty_remote[as]);
-            else tc::mbar_arrive(&ctl->tmem_empty[as]);
+            if (c.tmem_empty_remote[buf.i]) tc::mbar_arrive_cluster_tmem(c.tmem_empty_remote[buf.i]);
+            else tc::mbar_arrive(&ctl->tmem_empty[buf.i]);
         }
-        if (++as == p.acc_stages) { as = 0; aphase ^= 1; }
+        buf.next(kAccStages);
         if (MODE == 0) {
             if (p.gate_bytes) {
                 tc::mbar_arrive(&ctl->gate_empty);
@@ -425,63 +433,170 @@ __device__ __forceinline__ void epilogue_loop(const KParams& p, const EpiCtx& c,
     }
 }
 
-template <bool STATS>
-__global__ void __launch_bounds__(kThreads, 1)
-conv_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
-                 const __grid_constant__ CUtensorMap tmap_out, const __grid_constant__ CUtensorMap tmap_gate,
-                 const __grid_constant__ KParams p) {
+// ---- the frame shared by the GEMM kernels ---------------------------------------------------------------------------------
+enum GemmKind { kGemm, kGemmPair, kConv3x3, kConv3x3Pair, kDsam };
+
+constexpr int kTile = kBlockM * 128;         // 16 KB: 128 pixels x 64 bf16 channels
+constexpr int kDsamThreads = 512;            // dsam_fwd_kernel: 4 control warps + 8 epilogue warps + 4 mask warps
+constexpr int kDsamRaw = 3;                  // dsam_fwd_kernel: raw (unmasked) tile ring, prefetched ahead of the masking
+
+// Dynamic shared memory of a GEMM kernel from its 1024-aligned start: a kernel-specific head (conv_gemm_kernel: the resident
+// weights; the 3x3 kernels: the ring of A tiles; dsam_fwd_kernel: the raw tiles and two groups of masked copies), the operand
+// ring of p.stages slots, the staged output tile and the gate tile (epilogue mode 0), the barriers, the slice table and the
+// scale / shift tables.  The host sizes the launch and the kernel places its buffers with this one function.
+// Addr: uint8_t* from the aligned start in a kernel, size_t from 0 on the host.
+template <typename Addr>
+struct SmemLayout {
+    Addr ring;                               // the operand ring
+    int stage;                               // bytes per ring slot
+    Addr staging, gate, ctl, slices, scale, shift, end;
+};
+
+template <typename Addr>
+__host__ __device__ __forceinline__ SmemLayout<Addr> smem_layout(GemmKind kind, const KParams& p, Addr base) {
+    SmemLayout<Addr> L;
+    switch (kind) {
+    case kGemm:
+        L.ring = base + p.b_res_bytes;
+        L.stage = kBlockM * p.kb_bytes + (p.b_resident ? 0 : p.BLOCK_N * p.kb_bytes);
+        break;
+    case kGemmPair:                          // A tile + this CTA's half of the B K block
+        L.ring = base;
+        L.stage = kBlockM * p.kb_bytes + (p.BLOCK_N / 2) * p.kb_bytes;
+        break;
+    case kConv3x3:
+    case kConv3x3Pair:                       // B tiles (a CTA pair: half of each per CTA)
+        L.ring = base + (size_t)p.sa_stages * p.a_stage_bytes;
+        L.stage = (kind == kConv3x3 ? p.BLOCK_N : p.BLOCK_N / 2) * 128;
+        break;
+    case kDsam:                              // half weight tiles
+        L.ring = base + (size_t)(kDsamRaw + 2 * p.m3_masked_segs) * kTile;
+        L.stage = (p.BLOCK_N / 2) * 128;
+        break;
+    }
+    L.staging = L.ring + (size_t)p.stages * L.stage;
+    L.gate = L.staging + p.staging_bytes;
+    L.ctl = L.gate + p.gate_bytes;
+    L.slices = L.ctl + sizeof(SmemCtl);
+    L.scale = L.slices + (size_t)p.n_slices * sizeof(int4);
+    L.shift = L.scale + (size_t)p.BLOCK_N * sizeof(float);
+    L.end = L.shift + (size_t)p.BLOCK_N * sizeof(float);
+    return L;
+}
+
+// dynamic shared memory aligned to 1024 bytes (the period of the 128B swizzle); keeps the shared address space
+__device__ __forceinline__ uint8_t* smem_base() {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
-    uint8_t* smem = smem_raw + ((1024u - (tc::smem_u32(smem_raw) & 1023u)) & 1023u);   // keeps the shared address space
-    const int a_bytes = kBlockM * p.kb_bytes;
-    const int b_bytes = p.BLOCK_N * p.kb_bytes;
-    const int stage_bytes = p.b_resident ? a_bytes : a_bytes + b_bytes;   // multiples of 1024 by construction
-    uint8_t* s_bres = smem;                                                  // resident weights (b_resident)
-    uint8_t* s_ring = smem + p.b_res_bytes;
-    uint8_t* s_staging = s_ring + (size_t)p.stages * stage_bytes;            // 1024-aligned
-    uint8_t* s_gate = s_staging + p.staging_bytes;                           // 1024-aligned
-    SmemCtl* ctl = reinterpret_cast<SmemCtl*>(s_gate + p.gate_bytes);
-    int4* s_slices = reinterpret_cast<int4*>(reinterpret_cast<uint8_t*>(ctl) + sizeof(SmemCtl));
-    float* s_scale = reinterpret_cast<float*>(s_slices + p.n_slices);
-    float* s_shift = s_scale + p.BLOCK_N;
+    return smem_raw + ((1024u - (tc::smem_u32(smem_raw) & 1023u)) & 1023u);
+}
 
+// Prologue of a GEMM kernel; PAIR: the CTA pair of a cluster runs tcgen05 cta_group::2.  Warp 0 prefetches the tensor maps,
+// warp 1 initialises the operand ring's barriers and the accumulator buffers' barriers (tmem_empty: one arrive per epilogue
+// warp of every CTA) and fences them together with the kernel's own, which the same thread initialised before the call;
+// warp 2 allocates the tensor memory.  Returns its base address.
+template <bool PAIR>
+__device__ __forceinline__ uint32_t gemm_prologue(SmemCtl* ctl, const KParams& p, const CUtensorMap* tmap_a,
+                                                  const CUtensorMap* tmap_b, const CUtensorMap* tmap_out,
+                                                  const CUtensorMap* tmap_gate) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-
-    for (int i = threadIdx.x; i < p.n_slices; i += blockDim.x) s_slices[i] = p.slices[i];
     if (warp == 0 && lane == 0) {
-        tc::prefetch_tmap(&tmap_a);
-        tc::prefetch_tmap(&tmap_b);
-        if (p.staging_bytes) tc::prefetch_tmap(&tmap_out);
-        if (p.gate_bytes) tc::prefetch_tmap(&tmap_gate);
+        tc::prefetch_tmap(tmap_a);
+        tc::prefetch_tmap(tmap_b);
+        if (p.staging_bytes) tc::prefetch_tmap(tmap_out);
+        if (p.gate_bytes) tc::prefetch_tmap(tmap_gate);
     }
     if (warp == 1 && lane == 0) {
         for (int s = 0; s < p.stages; ++s) {
             tc::mbar_init(&ctl->full[s], 1);
             tc::mbar_init(&ctl->empty[s], 1);
         }
-        for (int s = 0; s < 2; ++s) {
+        for (int s = 0; s < kAccStages; ++s) {
             tc::mbar_init(&ctl->tmem_full[s], 1);
-            tc::mbar_init(&ctl->tmem_empty[s], kEpiWarps);
+            tc::mbar_init(&ctl->tmem_empty[s], (PAIR ? 2 : 1) * kEpiWarps);
         }
+        tc::fence_barrier_init();
+    }
+    if (PAIR) {
+        tc::cluster_sync_all();              // the barriers of both CTAs exist before any remote use
+        if (warp == 2) tc::tmem_alloc_2cta(&ctl->tmem_base, kTmemCols);
+        tc::tc_fence_before();
+        tc::cluster_sync_all();
+    } else {
+        if (warp == 2) tc::tmem_alloc(&ctl->tmem_base, kTmemCols);
+        tc::tc_fence_before();
+        __syncthreads();
+    }
+    tc::tc_fence_after();
+    return ctl->tmem_base;
+}
+
+// Contiguous range [begin, end) of work units of this CTA (PAIR: of this CTA pair): tiles, or pair units (see pair_tile).
+// Contiguous ranges keep the pooled epilogue's partial sums in registers across tiles.
+template <bool PAIR>
+__device__ __forceinline__ void work_range(const KParams& p, int& begin, int& end) {
+    const int units = PAIR ? ((p.total_tiles / p.n_tiles_n + 1) / 2) * p.n_tiles_n : p.total_tiles;
+    const int n = PAIR ? (int)gridDim.x / 2 : (int)gridDim.x, id = PAIR ? (int)blockIdx.x / 2 : (int)blockIdx.x;
+    const int per = units / n, rem = units % n;
+    begin = id * per + min(id, rem);
+    end = begin + per + (id < rem ? 1 : 0);
+}
+
+// the epilogue warps' view; in a CTA pair they release the accumulator on the leader's tmem_empty barriers
+template <bool PAIR>
+__device__ __forceinline__ EpiCtx epi_ctx(const SmemLayout<uint8_t*>& L, SmemCtl* ctl, uint32_t tmem_base, int begin, int end) {
+    EpiCtx c{L.staging, L.gate, ctl, reinterpret_cast<float*>(L.scale), reinterpret_cast<float*>(L.shift), tmem_base, begin, end,
+             (int)threadIdx.x >> 5, (int)threadIdx.x & 31, -1, {0u, 0u}};
+    if (PAIR) {
+        c.pair_rank = (int)tc::cluster_ctarank();
+        for (int b = 0; b < kAccStages; ++b) c.tmem_empty_remote[b] = tc::mapa(tc::smem_u32(&ctl->tmem_empty[b]), 0);
+    }
+    return c;
+}
+
+template <bool PAIR>
+__device__ __forceinline__ void gemm_teardown(uint32_t tmem_base) {
+    tc::tc_fence_before();
+    if (PAIR) tc::cluster_sync_all();        // the peer's smem / TMEM stay alive until the leader's MMAs are done
+    else __syncthreads();
+    if ((threadIdx.x >> 5) == 2) {
+        tc::tc_fence_after();
+        if (PAIR) tc::tmem_dealloc_2cta(tmem_base, kTmemCols);
+        else tc::tmem_dealloc(tmem_base, kTmemCols);
+    }
+}
+
+// Every GEMM kernel takes the same parameters: A and B maps, the output and gate maps of epilogue mode 0 (placeholders
+// otherwise) and the parameter block.
+template <bool STATS>
+__global__ void __launch_bounds__(kThreads, 1)
+conv_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
+                 const __grid_constant__ CUtensorMap tmap_out, const __grid_constant__ CUtensorMap tmap_gate,
+                 const __grid_constant__ KParams p) {
+    uint8_t* smem = smem_base();
+    const SmemLayout<uint8_t*> L = smem_layout(kGemm, p, smem);
+    const int a_bytes = kBlockM * p.kb_bytes;
+    const int b_bytes = p.BLOCK_N * p.kb_bytes;
+    uint8_t* s_bres = smem;                                                  // resident weights (b_resident)
+    uint8_t* s_ring = L.ring;
+    uint8_t* s_gate = L.gate;
+    SmemCtl* ctl = reinterpret_cast<SmemCtl*>(L.ctl);
+    int4* s_slices = reinterpret_cast<int4*>(L.slices);
+
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    for (int i = threadIdx.x; i < p.n_slices; i += blockDim.x) s_slices[i] = p.slices[i];
+    if (warp == 1 && lane == 0) {
         tc::mbar_init(&ctl->b_full, 1);
         tc::mbar_init(&ctl->gate_full, 1);
         tc::mbar_init(&ctl->gate_empty, kEpiThreads);
-        tc::fence_barrier_init();
     }
-    if (warp == 2) tc::tmem_alloc(&ctl->tmem_base, kTmemCols);
-    tc::tc_fence_before();
-    __syncthreads();
-    tc::tc_fence_after();
-    const uint32_t tmem_base = ctl->tmem_base;
-
-    // contiguous tile range per CTA (keeps pooled partial sums in registers across tiles)
-    const int per = p.total_tiles / gridDim.x, rem = p.total_tiles % gridDim.x;
-    const int t_begin = blockIdx.x * per + min((int)blockIdx.x, rem);
-    const int t_end = t_begin + per + ((int)blockIdx.x < rem ? 1 : 0);
+    const uint32_t tmem_base = gemm_prologue<false>(ctl, p, &tmap_a, &tmap_b, &tmap_out, &tmap_gate);
+    int t_begin, t_end;
+    work_range<false>(p, t_begin, t_end);
 
     if (warp == 0 && lane == 0) {
         // ================= TMA producer =================
-        int stage = 0;
-        uint32_t phase = 0, gphase = 0;
+        Ring st;
+        uint32_t gphase = 0;
         if (p.b_resident) {
             tc::mbar_expect_tx(&ctl->b_full, (uint32_t)p.b_res_bytes);
             for (int j = 0; j < p.n_slices; ++j)
@@ -500,51 +615,48 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
                 gphase ^= 1;
             }
             for (int j = 0; j < p.n_slices; ++j) {
-                tc::mbar_wait(&ctl->empty[stage], phase ^ 1);
-                uint8_t* sa = s_ring + (size_t)stage * stage_bytes;
+                tc::mbar_wait(&ctl->empty[st.i], st.ph ^ 1);
+                uint8_t* sa = s_ring + (size_t)st.i * L.stage;
                 uint8_t* sb = sa + a_bytes;
-                tc::mbar_expect_tx(&ctl->full[stage], (uint32_t)stage_bytes);
+                tc::mbar_expect_tx(&ctl->full[st.i], (uint32_t)L.stage);
                 const int4 sl = s_slices[j];
-                tc::tma_load_4d(sa, &tmap_a, &ctl->full[stage], sl.x, x0 + sl.y, y0 + sl.z, pl0 + sl.w);
+                tc::tma_load_4d(sa, &tmap_a, &ctl->full[st.i], sl.x, x0 + sl.y, y0 + sl.z, pl0 + sl.w);
                 if (!p.b_resident)
-                    tc::tma_load_2d(sb, &tmap_b, &ctl->full[stage], j * (p.kb_bytes >> 1), nt * p.BLOCK_N);
-                if (++stage == p.stages) { stage = 0; phase ^= 1; }
+                    tc::tma_load_2d(sb, &tmap_b, &ctl->full[st.i], j * (p.kb_bytes >> 1), nt * p.BLOCK_N);
+                st.next(p.stages);
             }
         }
     } else if (warp == 1) {
         // ================= MMA issuer: whole warp in uniform control flow, one elected lane issues =================
         const uint32_t idesc = tc::make_idesc_bf16(kBlockM, p.BLOCK_N);
         const int k_per_block = p.kb_bytes >> 5;           // UMMA_K = 16 bf16 = 32 bytes
-        int stage = 0;
-        uint32_t phase = 0;
-        int as = 0;
-        uint32_t aphase = 0;
+        Ring st, buf;
         if (p.b_resident) tc::mbar_wait(&ctl->b_full, 0);
         for (int t = t_begin; t < t_end; ++t) {
-            tc::mbar_wait(&ctl->tmem_empty[as], aphase ^ 1);
+            tc::mbar_wait(&ctl->tmem_empty[buf.i], buf.ph ^ 1);
             tc::tc_fence_after();
-            const uint32_t d_tmem = tmem_base + (uint32_t)(as * p.BLOCK_N);
+            const uint32_t d_tmem = tmem_base + (uint32_t)(buf.i * p.BLOCK_N);
             for (int j = 0; j < p.n_slices; ++j) {
-                tc::mbar_wait(&ctl->full[stage], phase);
+                tc::mbar_wait(&ctl->full[st.i], st.ph);
                 tc::tc_fence_after();
-                const uint32_t sa = tc::smem_u32(s_ring + (size_t)stage * stage_bytes);
+                const uint32_t sa = tc::smem_u32(s_ring + (size_t)st.i * L.stage);
                 const uint32_t sb = p.b_resident ? tc::smem_u32(s_bres + (size_t)j * b_bytes) : sa + a_bytes;
                 const uint64_t adesc = tc::make_kmajor_desc(sa, p.kb_bytes);
                 const uint64_t bdesc = tc::make_kmajor_desc(sb, p.kb_bytes);
                 if (tc::elect_one()) {
                     for (int k = 0; k < k_per_block; ++k)
                         tc::umma_bf16(d_tmem, adesc + (uint64_t)(k * 2), bdesc + (uint64_t)(k * 2), idesc, (j | k) != 0);
-                    tc::umma_commit(&ctl->empty[stage]);
-                    if (j == p.n_slices - 1) tc::umma_commit(&ctl->tmem_full[as]);
+                    tc::umma_commit(&ctl->empty[st.i]);
+                    if (j == p.n_slices - 1) tc::umma_commit(&ctl->tmem_full[buf.i]);
                 }
                 __syncwarp();
-                if (++stage == p.stages) { stage = 0; phase ^= 1; }
+                st.next(p.stages);
             }
-            if (++as == p.acc_stages) { as = 0; aphase ^= 1; }
+            buf.next(kAccStages);
         }
     } else if (warp >= 4) {
         // ================= epilogue =================
-        EpiCtx c{smem, s_staging, s_gate, ctl, s_scale, s_shift, tmem_base, t_begin, t_end, warp, lane, -1, {0u, 0u}};
+        const EpiCtx c = epi_ctx<false>(L, ctl, tmem_base, t_begin, t_end);
         const bool sc = p.scale != nullptr;
         if (p.epi_mode == 0) {
             if (p.act == 2) epilogue_loop<0, 2, false>(p, c, &tmap_out);
@@ -563,13 +675,7 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
             else epilogue_loop<2, 1, false>(p, c, &tmap_out);
         }
     }
-
-    tc::tc_fence_before();
-    __syncthreads();
-    if (warp == 2) {
-        tc::tc_fence_after();
-        tc::tmem_dealloc(tmem_base, kTmemCols);
-    }
+    gemm_teardown<false>(tmem_base);
 }
 
 
@@ -584,71 +690,44 @@ __global__ void __launch_bounds__(kThreads, 1)
 conv3x3_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                const __grid_constant__ CUtensorMap tmap_out, const __grid_constant__ CUtensorMap tmap_gate,
                const __grid_constant__ KParams p) {
-    extern __shared__ __align__(1024) uint8_t smem_raw[];
-    uint8_t* smem = smem_raw + ((1024u - (tc::smem_u32(smem_raw) & 1023u)) & 1023u);
-    const int b_bytes = p.BLOCK_N * 128;
+    uint8_t* smem = smem_base();
+    const SmemLayout<uint8_t*> L = smem_layout(kConv3x3, p, smem);
     uint8_t* s_a = smem;
-    uint8_t* s_b = s_a + (size_t)p.sa_stages * p.a_stage_bytes;
-    uint8_t* s_staging = s_b + (size_t)p.stages * b_bytes;
-    uint8_t* s_gate = s_staging + p.staging_bytes;
-    SmemCtl* ctl = reinterpret_cast<SmemCtl*>(s_gate + p.gate_bytes);
-    int4* s_slices = reinterpret_cast<int4*>(reinterpret_cast<uint8_t*>(ctl) + sizeof(SmemCtl));
-    float* s_scale = reinterpret_cast<float*>(s_slices + p.n_slices);
-    float* s_shift = s_scale + p.BLOCK_N;
+    uint8_t* s_b = L.ring;
+    SmemCtl* ctl = reinterpret_cast<SmemCtl*>(L.ctl);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    if (warp == 0 && lane == 0) {
-        tc::prefetch_tmap(&tmap_a);
-        tc::prefetch_tmap(&tmap_b);
-        if (p.staging_bytes) tc::prefetch_tmap(&tmap_out);
-    }
     if (warp == 1 && lane == 0) {
-        for (int s = 0; s < p.stages; ++s) {
-            tc::mbar_init(&ctl->full[s], 1);
-            tc::mbar_init(&ctl->empty[s], 1);
-        }
         for (int s = 0; s < p.sa_stages; ++s) {
             tc::mbar_init(&ctl->a_full[s], 1);
             tc::mbar_init(&ctl->a_empty[s], 1);
         }
-        for (int s = 0; s < 2; ++s) {
-            tc::mbar_init(&ctl->tmem_full[s], 1);
-            tc::mbar_init(&ctl->tmem_empty[s], kEpiWarps);
-        }
         tc::mbar_init(&ctl->gate_full, 1);
         tc::mbar_init(&ctl->gate_empty, kEpiThreads);
-        tc::fence_barrier_init();
     }
-    if (warp == 2) tc::tmem_alloc(&ctl->tmem_base, kTmemCols);
-    tc::tc_fence_before();
-    __syncthreads();
-    tc::tc_fence_after();
-    const uint32_t tmem_base = ctl->tmem_base;
-
-    const int per = p.total_tiles / gridDim.x, rem = p.total_tiles % gridDim.x;
-    const int t_begin = blockIdx.x * per + min((int)blockIdx.x, rem);
-    const int t_end = t_begin + per + ((int)blockIdx.x < rem ? 1 : 0);
+    const uint32_t tmem_base = gemm_prologue<false>(ctl, p, &tmap_a, &tmap_b, &tmap_out, &tmap_gate);
+    int t_begin, t_end;
+    work_range<false>(p, t_begin, t_end);
 
     if (warp == 0 && lane == 0) {
         // ================= TMA producer =================
-        int sa = 0, sb = 0;
-        uint32_t pa = 0, pb = 0;
+        Ring ra, rb;
         for (int t = t_begin; t < t_end; ++t) {
             int img, ty, tx, nt;
             decode_tile(p, t, img, ty, tx, nt);
             const int x0 = tx * p.BX, y0 = ty;
             for (int dy = 0; dy < 3; ++dy) {
                 for (int cb = 0; cb < p.c_blocks; ++cb) {
-                    tc::mbar_wait(&ctl->a_empty[sa], pa ^ 1);
-                    tc::mbar_expect_tx(&ctl->a_full[sa], (uint32_t)((kBlockM + 2) * 128));
-                    tc::tma_load_4d(s_a + (size_t)sa * p.a_stage_bytes, &tmap_a, &ctl->a_full[sa], cb * 64, x0 - 1, y0 + dy - 1, img);
-                    if (++sa == p.sa_stages) { sa = 0; pa ^= 1; }
+                    tc::mbar_wait(&ctl->a_empty[ra.i], ra.ph ^ 1);
+                    tc::mbar_expect_tx(&ctl->a_full[ra.i], (uint32_t)((kBlockM + 2) * 128));
+                    tc::tma_load_4d(s_a + (size_t)ra.i * p.a_stage_bytes, &tmap_a, &ctl->a_full[ra.i], cb * 64, x0 - 1, y0 + dy - 1, img);
+                    ra.next(p.sa_stages);
                     for (int dx = 0; dx < 3; ++dx) {
-                        tc::mbar_wait(&ctl->empty[sb], pb ^ 1);
-                        tc::mbar_expect_tx(&ctl->full[sb], (uint32_t)b_bytes);
-                        tc::tma_load_2d(s_b + (size_t)sb * b_bytes, &tmap_b, &ctl->full[sb],
+                        tc::mbar_wait(&ctl->empty[rb.i], rb.ph ^ 1);
+                        tc::mbar_expect_tx(&ctl->full[rb.i], (uint32_t)L.stage);
+                        tc::tma_load_2d(s_b + (size_t)rb.i * L.stage, &tmap_b, &ctl->full[rb.i],
                                         ((dy * 3 + dx) * p.c_blocks + cb) * 64, nt * p.BLOCK_N);
-                        if (++sb == p.stages) { sb = 0; pb ^= 1; }
+                        rb.next(p.stages);
                     }
                 }
             }
@@ -656,43 +735,42 @@ conv3x3_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
     } else if (warp == 1) {
         // ================= MMA issuer: whole warp in uniform control flow, one elected lane issues =================
         const uint32_t idesc = tc::make_idesc_bf16(kBlockM, p.BLOCK_N);
-        int sa = 0, sb = 0, as = 0;
-        uint32_t pa = 0, pb = 0, aphase = 0;
+        Ring ra, rb, buf;
         for (int t = t_begin; t < t_end; ++t) {
-            tc::mbar_wait(&ctl->tmem_empty[as], aphase ^ 1);
+            tc::mbar_wait(&ctl->tmem_empty[buf.i], buf.ph ^ 1);
             tc::tc_fence_after();
-            const uint32_t d_tmem = tmem_base + (uint32_t)(as * p.BLOCK_N);
+            const uint32_t d_tmem = tmem_base + (uint32_t)(buf.i * p.BLOCK_N);
             uint32_t first = 0;                 // 0 until the tile's first MMA (overwrites the accumulator)
             for (int dy = 0; dy < 3; ++dy) {
                 for (int cb = 0; cb < p.c_blocks; ++cb) {
-                    tc::mbar_wait(&ctl->a_full[sa], pa);
-                    const uint32_t a_base = tc::smem_u32(s_a + (size_t)sa * p.a_stage_bytes);
+                    tc::mbar_wait(&ctl->a_full[ra.i], ra.ph);
+                    const uint32_t a_base = tc::smem_u32(s_a + (size_t)ra.i * p.a_stage_bytes);
                     for (int dx = 0; dx < 3; ++dx) {
-                        tc::mbar_wait(&ctl->full[sb], pb);
+                        tc::mbar_wait(&ctl->full[rb.i], rb.ph);
                         tc::tc_fence_after();
                         const uint64_t adesc = tc::make_kmajor_desc(a_base + (uint32_t)(dx * 128), 128);
-                        const uint64_t bdesc = tc::make_kmajor_desc(tc::smem_u32(s_b + (size_t)sb * b_bytes), 128);
+                        const uint64_t bdesc = tc::make_kmajor_desc(tc::smem_u32(s_b + (size_t)rb.i * L.stage), 128);
                         if (tc::elect_one()) {
 #pragma unroll
                             for (int k = 0; k < 4; ++k)
                                 tc::umma_bf16(d_tmem, adesc + (uint64_t)(k * 2), bdesc + (uint64_t)(k * 2), idesc, (first | k) ? 1u : 0u);
-                            tc::umma_commit(&ctl->empty[sb]);
+                            tc::umma_commit(&ctl->empty[rb.i]);
                             if (dx == 2) {
-                                tc::umma_commit(&ctl->a_empty[sa]);
-                                if (dy == 2 && cb == p.c_blocks - 1) tc::umma_commit(&ctl->tmem_full[as]);
+                                tc::umma_commit(&ctl->a_empty[ra.i]);
+                                if (dy == 2 && cb == p.c_blocks - 1) tc::umma_commit(&ctl->tmem_full[buf.i]);
                             }
                         }
                         __syncwarp();
                         first = 1;
-                        if (++sb == p.stages) { sb = 0; pb ^= 1; }
+                        rb.next(p.stages);
                     }
-                    if (++sa == p.sa_stages) { sa = 0; pa ^= 1; }
+                    ra.next(p.sa_stages);
                 }
             }
-            if (++as == p.acc_stages) { as = 0; aphase ^= 1; }
+            buf.next(kAccStages);
         }
     } else if (warp >= 4) {
-        EpiCtx c{smem, s_staging, s_gate, ctl, s_scale, s_shift, tmem_base, t_begin, t_end, warp, lane, -1, {0u, 0u}};
+        const EpiCtx c = epi_ctx<false>(L, ctl, tmem_base, t_begin, t_end);
         const bool sc = p.scale != nullptr;
         if (p.epi_mode == 0) {
             if (p.act == 1 && !sc) epilogue_loop<0, 1, false>(p, c, &tmap_out);
@@ -705,13 +783,7 @@ conv3x3_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
             else epilogue_loop<2, 1, false>(p, c, &tmap_out);
         }
     }
-
-    tc::tc_fence_before();
-    __syncthreads();
-    if (warp == 2) {
-        tc::tc_fence_after();
-        tc::tmem_dealloc(tmem_base, kTmemCols);
-    }
+    gemm_teardown<false>(tmem_base);
 }
 
 // DSAModule.forward (CM:683-696) without the five-fold masked operand in HBM: the UNMASKED feature tile of a
@@ -721,43 +793,23 @@ conv3x3_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
 // against the five weight tiles.  Versus conv_gemm on a pre-masked operand this loads 128 + 5*BLOCK_N/2 TMA rows per
 // 5 K blocks instead of 5*(128 + BLOCK_N/2) and the pack kernel writes one copy instead of five.  CTA pairs
 // (cta_group::2): every CTA masks its own tile, the weight tiles are split between the two CTAs.
-constexpr int kDsamThreads = 512;            // 4 control warps + 8 epilogue warps + 4 mask warps
-constexpr int kDsamRaw = 3;                  // raw (unmasked) tile ring: prefetched ahead of the masking
-// TMEM_A: the masked copies live in TENSOR MEMORY instead of shared memory (tcgen05.st by the mask warps, tcgen05.mma with
-// the A operand in TMEM): the 64 KB of masked-copy writes and the 64 KB of A reads per (tap, channel block) group leave the
-// shared-memory port, which bounded the kernel at N = 192 (154 B/clk wanted of 128 B/clk, profiles/r01_notes.md).  Tensor
-// memory then holds ONE accumulator buffer [0, BLOCK_N) and two groups of four 32-column bf16 operands at [256, 512): the
-// epilogue no longer overlaps the next tile's MMAs (~3 k of ~40 k cycles per tile).
-constexpr uint32_t kDsamTmemA = 256;
-template <bool TMEM_A>
 __global__ void __launch_bounds__(kDsamThreads, 1)
 dsam_fwd_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
+                const __grid_constant__ CUtensorMap tmap_out, const __grid_constant__ CUtensorMap tmap_gate,
                 const __grid_constant__ KParams p) {
-    extern __shared__ __align__(1024) uint8_t smem_raw[];
-    uint8_t* smem = smem_raw + ((1024u - (tc::smem_u32(smem_raw) & 1023u)) & 1023u);
-    constexpr int kTile = kBlockM * 128;                       // 16 KB: 128 pixels x 64 channels
+    uint8_t* smem = smem_base();
+    const SmemLayout<uint8_t*> L = smem_layout(kDsam, p, smem);
     const int n_seg = p.m3_n_seg;                              // 5: four masked segments + the projection copy
     const int n_msk = p.m3_masked_segs;
-    const int b_bytes = (p.BLOCK_N / 2) * 128;
     uint8_t* s_rawt = smem;                                    // kDsamRaw raw tiles (TMA targets; also the projection operand)
-    uint8_t* s_msk = s_rawt + kDsamRaw * kTile;                // 2 groups x n_msk masked copies (not with TMEM_A)
-    uint8_t* s_b = s_msk + (TMEM_A ? 0 : 2 * n_msk * kTile);
-    SmemCtl* ctl = reinterpret_cast<SmemCtl*>(s_b + (size_t)p.stages * b_bytes);
-    float* s_scale = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(ctl) + sizeof(SmemCtl));
-    float* s_shift = s_scale + p.BLOCK_N;
+    uint8_t* s_msk = s_rawt + kDsamRaw * kTile;                // 2 groups x n_msk masked copies
+    uint8_t* s_b = L.ring;
+    SmemCtl* ctl = reinterpret_cast<SmemCtl*>(L.ctl);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t rank = tc::cluster_ctarank();
     const bool leader = rank == 0;
-    if (warp == 0 && lane == 0) {
-        tc::prefetch_tmap(&tmap_a);
-        tc::prefetch_tmap(&tmap_b);
-    }
     if (warp == 1 && lane == 0) {
-        for (int s = 0; s < p.stages; ++s) {
-            tc::mbar_init(&ctl->full[s], 1);
-            tc::mbar_init(&ctl->empty[s], 1);
-        }
         for (int r = 0; r < kDsamRaw; ++r) {
             tc::mbar_init(&ctl->a_full[r], 1);                 // raw tile landed (local TMA)
             tc::mbar_init(&ctl->a_empty[r], 1);                // released by the pair's MMAs (multicast commit)
@@ -765,46 +817,31 @@ dsam_fwd_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constan
         for (int g = 0; g < 2; ++g) {
             tc::mbar_init(&ctl->masked_full[g], 2 * 4);        // one arrive per mask warp of BOTH CTAs (counted in the leader)
             tc::mbar_init(&ctl->masked_empty[g], 1);           // multicast commit
-            tc::mbar_init(&ctl->tmem_full[g], 1);
-            tc::mbar_init(&ctl->tmem_empty[g], 2 * kEpiWarps);
         }
-        tc::fence_barrier_init();
     }
-    tc::cluster_sync_all();
-    if (warp == 2) tc::tmem_alloc_2cta(&ctl->tmem_base, kTmemCols);
-    tc::tc_fence_before();
-    tc::cluster_sync_all();
-    tc::tc_fence_after();
-    const uint32_t tmem_base = ctl->tmem_base;
-
-    const int total_m = p.total_tiles / p.n_tiles_n;
-    const int n_units = ((total_m + 1) / 2) * p.n_tiles_n;
-    const int n_clusters = gridDim.x / 2, cid = blockIdx.x / 2;
-    const int per = n_units / n_clusters, rem = n_units % n_clusters;
-    const int u_begin = cid * per + min(cid, rem);
-    const int u_end = u_begin + per + (cid < rem ? 1 : 0);
+    const uint32_t tmem_base = gemm_prologue<true>(ctl, p, &tmap_a, &tmap_b, &tmap_out, &tmap_gate);
+    int u_begin, u_end;
+    work_range<true>(p, u_begin, u_end);
     const int groups_per_tile = p.dsam_taps * p.c_blocks;
 
     if (warp == 0 && lane == 0) {
         // ================= TMA producer: weight tiles =================
-        int sb = 0;
-        uint32_t pb = 0;
+        Ring rb;
         for (int u = u_begin; u < u_end; ++u) {
             const int nt = pair_tile(p, u, (int)rank) % p.n_tiles_n;
             for (int gi = 0; gi < groups_per_tile; ++gi) {
                 for (int sg = 0; sg < n_seg; ++sg) {
-                    tc::mbar_wait(&ctl->empty[sb], pb ^ 1);
-                    if (leader) tc::mbar_expect_tx(&ctl->full[sb], 2u * (uint32_t)b_bytes);
-                    tc::tma_load_2d_2cta(s_b + (size_t)sb * b_bytes, &tmap_b, &ctl->full[sb], (gi * n_seg + sg) * 64,
+                    tc::mbar_wait(&ctl->empty[rb.i], rb.ph ^ 1);
+                    if (leader) tc::mbar_expect_tx(&ctl->full[rb.i], 2u * (uint32_t)L.stage);
+                    tc::tma_load_2d_2cta(s_b + (size_t)rb.i * L.stage, &tmap_b, &ctl->full[rb.i], (gi * n_seg + sg) * 64,
                                          nt * p.BLOCK_N + (int)rank * (p.BLOCK_N / 2));
-                    if (++sb == p.stages) { sb = 0; pb ^= 1; }
+                    rb.next(p.stages);
                 }
             }
         }
     } else if (warp == 3 && lane == 0) {
         // ================= TMA producer: raw feature tiles (own ring, runs ahead of the masking) =================
-        int r = 0;
-        uint32_t pr = 0;
+        Ring raw;
         for (int u = u_begin; u < u_end; ++u) {
             int img, ty, tx, nt;
             decode_tile(p, pair_tile(p, u, (int)rank), img, ty, tx, nt);
@@ -815,10 +852,10 @@ dsam_fwd_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constan
                 const int par = (dy == 1 ? 0 : 2) + (dx == 1 ? 0 : 1);
                 const int yo = dy == 0 ? -1 : 0, xo = dx == 0 ? -1 : 0;
                 for (int cb = 0; cb < p.c_blocks; ++cb) {
-                    tc::mbar_wait(&ctl->a_empty[r], pr ^ 1);
-                    tc::mbar_expect_tx(&ctl->a_full[r], kTile);
-                    tc::tma_load_4d(s_rawt + (size_t)r * kTile, &tmap_a, &ctl->a_full[r], cb * 64, x0 + xo, y0 + yo, img * 4 + par);
-                    if (++r == kDsamRaw) { r = 0; pr ^= 1; }
+                    tc::mbar_wait(&ctl->a_empty[raw.i], raw.ph ^ 1);
+                    tc::mbar_expect_tx(&ctl->a_full[raw.i], kTile);
+                    tc::tma_load_4d(s_rawt + (size_t)raw.i * kTile, &tmap_a, &ctl->a_full[raw.i], cb * 64, x0 + xo, y0 + yo, img * 4 + par);
+                    raw.next(kDsamRaw);
                 }
             }
         }
@@ -826,46 +863,40 @@ dsam_fwd_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constan
         // ================= MMA issuer (leader): the whole warp runs the uniform control flow so the descriptors stay in
         // uniform registers (no per-MMA ELECT/R2UR waterfall); one elected lane issues =================
         const uint32_t idesc = tc::make_idesc_bf16(2 * kBlockM, p.BLOCK_N);
-        int g = 0, r = 0, sb = 0, as = 0;
-        uint32_t pg = 0, pb = 0, aphase = 0;
+        Ring grp, raw, rb, buf;
         for (int u = u_begin; u < u_end; ++u) {
-            tc::mbar_wait(&ctl->tmem_empty[as], aphase ^ 1);
+            tc::mbar_wait(&ctl->tmem_empty[buf.i], buf.ph ^ 1);
             tc::tc_fence_after();
-            const uint32_t d_tmem = tmem_base + (uint32_t)(as * p.BLOCK_N);
+            const uint32_t d_tmem = tmem_base + (uint32_t)(buf.i * p.BLOCK_N);
             uint32_t first = 0;                                 // 0 until the tile's first MMA (overwrites the accumulator)
             for (int gi = 0; gi < groups_per_tile; ++gi) {
-                tc::mbar_wait(&ctl->masked_full[g], pg);       // both CTAs: raw tile landed and masked copies written
+                tc::mbar_wait(&ctl->masked_full[grp.i], grp.ph);   // both CTAs: raw tile landed and masked copies written
                 tc::tc_fence_after();
                 for (int sg = 0; sg < n_seg; ++sg) {
-                    tc::mbar_wait(&ctl->full[sb], pb);
+                    tc::mbar_wait(&ctl->full[rb.i], rb.ph);
                     tc::tc_fence_after();
-                    const uint8_t* a_tile = sg < n_msk ? s_msk + (size_t)(g * n_msk + sg) * kTile : s_rawt + (size_t)r * kTile;
+                    const uint8_t* a_tile = sg < n_msk ? s_msk + (size_t)(grp.i * n_msk + sg) * kTile : s_rawt + (size_t)raw.i * kTile;
                     const uint64_t adesc = tc::make_kmajor_desc(tc::smem_u32(a_tile), 128);
-                    const uint64_t bdesc = tc::make_kmajor_desc(tc::smem_u32(s_b + (size_t)sb * b_bytes), 128);
-                    const uint32_t a_tmem = tmem_base + kDsamTmemA + (uint32_t)((g * 4 + sg) * 32);
+                    const uint64_t bdesc = tc::make_kmajor_desc(tc::smem_u32(s_b + (size_t)rb.i * L.stage), 128);
                     if (tc::elect_one()) {
 #pragma unroll
-                        for (int k = 0; k < 4; ++k) {
-                            if (TMEM_A && sg < n_msk)
-                                tc::umma_bf16_ts_2cta(d_tmem, a_tmem + (uint32_t)(k * 8), bdesc + (uint64_t)(k * 2), idesc, (first | k) ? 1u : 0u);
-                            else
-                                tc::umma_bf16_2cta(d_tmem, adesc + (uint64_t)(k * 2), bdesc + (uint64_t)(k * 2), idesc, (first | k) ? 1u : 0u);
-                        }
-                        tc::umma_commit_2cta(&ctl->empty[sb]);
+                        for (int k = 0; k < 4; ++k)
+                            tc::umma_bf16_2cta(d_tmem, adesc + (uint64_t)(k * 2), bdesc + (uint64_t)(k * 2), idesc, (first | k) ? 1u : 0u);
+                        tc::umma_commit_2cta(&ctl->empty[rb.i]);
                         if (sg == n_seg - 1) {
-                            tc::umma_commit_2cta(&ctl->masked_empty[g]);
-                            tc::umma_commit_2cta(&ctl->a_empty[r]);
-                            if (gi == groups_per_tile - 1) tc::umma_commit_2cta(&ctl->tmem_full[as]);
+                            tc::umma_commit_2cta(&ctl->masked_empty[grp.i]);
+                            tc::umma_commit_2cta(&ctl->a_empty[raw.i]);
+                            if (gi == groups_per_tile - 1) tc::umma_commit_2cta(&ctl->tmem_full[buf.i]);
                         }
                     }
                     __syncwarp();
                     first = 1;
-                    if (++sb == p.stages) { sb = 0; pb ^= 1; }
+                    rb.next(p.stages);
                 }
-                if (++g == 2) { g = 0; pg ^= 1; }
-                if (++r == kDsamRaw) r = 0;
+                grp.next(2);
+                raw.next(kDsamRaw);
             }
-            if (++as == p.acc_stages) { as = 0; aphase ^= 1; }
+            buf.next(kAccStages);
         }
     } else if (warp >= 12) {
         // ================= mask warps: masked copies of the raw tile =================
@@ -873,8 +904,7 @@ dsam_fwd_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constan
         const int lx = row % p.BX, ly = row / p.BX;
         const uint32_t masked_full_remote[2] = {tc::mapa(tc::smem_u32(&ctl->masked_full[0]), 0),
                                                 tc::mapa(tc::smem_u32(&ctl->masked_full[1]), 0)};
-        int g = 0, r = 0;
-        uint32_t pg = 0, pr = 0;
+        Ring grp, raw;
         for (int u = u_begin; u < u_end; ++u) {
             int img, ty, tx, nt;
             decode_tile(p, pair_tile(p, u, (int)rank), img, ty, tx, nt);
@@ -886,172 +916,106 @@ dsam_fwd_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constan
                 if (img_ok && iy >= 0 && iy < p.in_h && ix >= 0 && ix < p.in_w)
                     code = p.codes[((size_t)img * p.in_h + iy) * p.in_w + ix];
                 for (int cb = 0; cb < p.c_blocks; ++cb) {
-                    tc::mbar_wait(&ctl->a_full[r], pr);
-                    const uint8_t* src = s_rawt + (size_t)r * kTile + row * 128;
+                    tc::mbar_wait(&ctl->a_full[raw.i], raw.ph);
+                    const uint8_t* src = s_rawt + (size_t)raw.i * kTile + row * 128;
                     uint4 v[8];
-                    if (TMEM_A) {
-                        // logical order (16-byte piece j of the row sits at chunk j ^ (row & 7) of the 128B-swizzled tile; the XOR
-                        // keeps the eight lanes of a quarter-warp on distinct chunks): words 4j .. 4j+3 = channels 8j .. 8j+7
 #pragma unroll
-                        for (int j = 0; j < 8; ++j) v[j] = *reinterpret_cast<const uint4*>(src + (((j ^ row) & 7) << 4));
-                        tc::mbar_wait(&ctl->masked_empty[g], pg ^ 1);
-                        tc::tc_fence_after();                  // the MMAs that read this group's columns have completed
-                        const uint32_t t0 = tmem_base + ((uint32_t)((warp - 12) * 32) << 16) + kDsamTmemA + (uint32_t)(g * 4 * 32);
-                        for (int sg = 0; sg < n_msk; ++sg) {
-                            const bool keep = (code >> sg) & 1u;
-                            uint32_t w[32];
+                    for (int j = 0; j < 8; ++j) v[j] = *reinterpret_cast<const uint4*>(src + (((j + row) & 7) << 4));   // rotated: bank-conflict free
+                    tc::mbar_wait(&ctl->masked_empty[grp.i], grp.ph ^ 1);
+                    const uint4 zero = make_uint4(0u, 0u, 0u, 0u);
+                    for (int sg = 0; sg < n_msk; ++sg) {
+                        uint8_t* dst = s_msk + (size_t)(grp.i * n_msk + sg) * kTile + row * 128;
+                        const bool keep = (code >> sg) & 1u;
 #pragma unroll
-                            for (int j = 0; j < 8; ++j) {
-                                w[4 * j] = keep ? v[j].x : 0u; w[4 * j + 1] = keep ? v[j].y : 0u;
-                                w[4 * j + 2] = keep ? v[j].z : 0u; w[4 * j + 3] = keep ? v[j].w : 0u;
-                            }
-                            tc::tmem_st_32x32(t0 + (uint32_t)(sg * 32), w);
-                        }
-                        tc::tmem_st_wait();
-                        tc::tc_fence_before();
-                    } else {
-#pragma unroll
-                        for (int j = 0; j < 8; ++j) v[j] = *reinterpret_cast<const uint4*>(src + (((j + row) & 7) << 4));   // rotated: bank-conflict free
-                        tc::mbar_wait(&ctl->masked_empty[g], pg ^ 1);
-                        const uint4 zero = make_uint4(0u, 0u, 0u, 0u);
-                        for (int sg = 0; sg < n_msk; ++sg) {
-                            uint8_t* dst = s_msk + (size_t)(g * n_msk + sg) * kTile + row * 128;
-                            const bool keep = (code >> sg) & 1u;
-#pragma unroll
-                            for (int j = 0; j < 8; ++j) *reinterpret_cast<uint4*>(dst + (((j + row) & 7) << 4)) = keep ? v[j] : zero;
-                        }
-                        tc::fence_proxy_async();               // generic-proxy writes -> visible to the tensor core's smem reads
+                        for (int j = 0; j < 8; ++j) *reinterpret_cast<uint4*>(dst + (((j + row) & 7) << 4)) = keep ? v[j] : zero;
                     }
+                    tc::fence_proxy_async();                   // generic-proxy writes -> visible to the tensor core's smem reads
                     __syncwarp();
                     // one arrive per warp, CTA-scope release: the copies are read by THIS CTA's tensor core (async proxy,
                     // ordered by the fence above); the remote barrier only signals the leader's MMA thread
-                    if (lane == 0) tc::mbar_arrive_cluster_tmem(masked_full_remote[g]);
-                    if (++g == 2) { g = 0; pg ^= 1; }
-                    if (++r == kDsamRaw) { r = 0; pr ^= 1; }
+                    if (lane == 0) tc::mbar_arrive_cluster_tmem(masked_full_remote[grp.i]);
+                    grp.next(2);
+                    raw.next(kDsamRaw);
                 }
             }
         }
     } else if (warp >= 4 && warp < 12) {
-        EpiCtx c{smem, nullptr, nullptr, ctl, s_scale, s_shift, tmem_base, u_begin, u_end, warp, lane, (int)rank,
-                 {tc::mapa(tc::smem_u32(&ctl->tmem_empty[0]), 0), tc::mapa(tc::smem_u32(&ctl->tmem_empty[1]), 0)}};
-        epilogue_loop<1, 0, false>(p, c, &tmap_a);
+        const EpiCtx c = epi_ctx<true>(L, ctl, tmem_base, u_begin, u_end);
+        epilogue_loop<1, 0, false>(p, c, &tmap_out);
     }
-
-    tc::tc_fence_before();
-    tc::cluster_sync_all();
-    if (warp == 2) {
-        tc::tc_fence_after();
-        tc::tmem_dealloc_2cta(tmem_base, kTmemCols);
-    }
+    gemm_teardown<true>(tmem_base);
 }
 
 // conv_gemm_kernel on CTA pairs (tcgen05 cta_group::2) for the DSAM stages (epilogue modes 1 and 3): the two CTAs of a
 // cluster take adjacent M tiles of the same N tile, so each stages only half of every B (weight) K block.
 __global__ void __launch_bounds__(kThreads, 1)
 conv_gemm_2cta_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
+                      const __grid_constant__ CUtensorMap tmap_out, const __grid_constant__ CUtensorMap tmap_gate,
                       const __grid_constant__ KParams p) {
-    extern __shared__ __align__(1024) uint8_t smem_raw[];
-    uint8_t* smem = smem_raw + ((1024u - (tc::smem_u32(smem_raw) & 1023u)) & 1023u);
+    uint8_t* smem = smem_base();
+    const SmemLayout<uint8_t*> L = smem_layout(kGemmPair, p, smem);
     const int a_bytes = kBlockM * p.kb_bytes;
-    const int b_bytes = (p.BLOCK_N / 2) * p.kb_bytes;          // this CTA's half of a B K block
-    const int stage_bytes = a_bytes + b_bytes;
-    SmemCtl* ctl = reinterpret_cast<SmemCtl*>(smem + (size_t)p.stages * stage_bytes);
-    int4* s_slices = reinterpret_cast<int4*>(reinterpret_cast<uint8_t*>(ctl) + sizeof(SmemCtl));
-    float* s_scale = reinterpret_cast<float*>(s_slices + p.n_slices);
-    float* s_shift = s_scale + p.BLOCK_N;
+    SmemCtl* ctl = reinterpret_cast<SmemCtl*>(L.ctl);
+    int4* s_slices = reinterpret_cast<int4*>(L.slices);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t rank = tc::cluster_ctarank();
     const bool leader = rank == 0;
     for (int i = threadIdx.x; i < p.n_slices; i += blockDim.x) s_slices[i] = p.slices[i];
-    if (warp == 0 && lane == 0) {
-        tc::prefetch_tmap(&tmap_a);
-        tc::prefetch_tmap(&tmap_b);
-    }
-    if (warp == 1 && lane == 0) {
-        for (int s = 0; s < p.stages; ++s) {
-            tc::mbar_init(&ctl->full[s], 1);
-            tc::mbar_init(&ctl->empty[s], 1);
-        }
-        for (int s = 0; s < 2; ++s) {
-            tc::mbar_init(&ctl->tmem_full[s], 1);
-            tc::mbar_init(&ctl->tmem_empty[s], 2 * kEpiWarps);
-        }
-        tc::fence_barrier_init();
-    }
-    tc::cluster_sync_all();
-    if (warp == 2) tc::tmem_alloc_2cta(&ctl->tmem_base, kTmemCols);
-    tc::tc_fence_before();
-    tc::cluster_sync_all();
-    tc::tc_fence_after();
-    const uint32_t tmem_base = ctl->tmem_base;
-
-    const int total_m = p.total_tiles / p.n_tiles_n;
-    const int n_units = ((total_m + 1) / 2) * p.n_tiles_n;
-    const int n_clusters = gridDim.x / 2, cid = blockIdx.x / 2;
-    const int per = n_units / n_clusters, rem = n_units % n_clusters;
-    const int u_begin = cid * per + min(cid, rem);
-    const int u_end = u_begin + per + (cid < rem ? 1 : 0);
+    const uint32_t tmem_base = gemm_prologue<true>(ctl, p, &tmap_a, &tmap_b, &tmap_out, &tmap_gate);
+    int u_begin, u_end;
+    work_range<true>(p, u_begin, u_end);
 
     if (warp == 0 && lane == 0) {
-        int stage = 0;
-        uint32_t phase = 0;
+        Ring st;
         for (int u = u_begin; u < u_end; ++u) {
             int img, ty, tx, nt;
             decode_tile(p, pair_tile(p, u, (int)rank), img, ty, tx, nt);
             const int x0 = tx * p.BX, y0 = ty * p.BY, pl0 = img * p.plane_per_img;
             for (int j = 0; j < p.n_slices; ++j) {
-                tc::mbar_wait(&ctl->empty[stage], phase ^ 1);
-                uint8_t* sa = smem + (size_t)stage * stage_bytes;
-                if (leader) tc::mbar_expect_tx(&ctl->full[stage], 2u * (uint32_t)stage_bytes);
+                tc::mbar_wait(&ctl->empty[st.i], st.ph ^ 1);
+                uint8_t* sa = L.ring + (size_t)st.i * L.stage;
+                if (leader) tc::mbar_expect_tx(&ctl->full[st.i], 2u * (uint32_t)L.stage);
                 const int4 sl = s_slices[j];
-                tc::tma_load_4d_2cta(sa, &tmap_a, &ctl->full[stage], sl.x, x0 + sl.y, y0 + sl.z, pl0 + sl.w);
-                tc::tma_load_2d_2cta(sa + a_bytes, &tmap_b, &ctl->full[stage], j * (p.kb_bytes >> 1),
+                tc::tma_load_4d_2cta(sa, &tmap_a, &ctl->full[st.i], sl.x, x0 + sl.y, y0 + sl.z, pl0 + sl.w);
+                tc::tma_load_2d_2cta(sa + a_bytes, &tmap_b, &ctl->full[st.i], j * (p.kb_bytes >> 1),
                                      nt * p.BLOCK_N + (int)rank * (p.BLOCK_N / 2));
-                if (++stage == p.stages) { stage = 0; phase ^= 1; }
+                st.next(p.stages);
             }
         }
     } else if (warp == 1 && leader) {
         // whole warp in uniform control flow, one elected lane issues (descriptors stay in uniform registers)
         const uint32_t idesc = tc::make_idesc_bf16(2 * kBlockM, p.BLOCK_N);
         const int k_per_block = p.kb_bytes >> 5;
-        int stage = 0, as = 0;
-        uint32_t phase = 0, aphase = 0;
+        Ring st, buf;
         for (int u = u_begin; u < u_end; ++u) {
-            tc::mbar_wait(&ctl->tmem_empty[as], aphase ^ 1);
+            tc::mbar_wait(&ctl->tmem_empty[buf.i], buf.ph ^ 1);
             tc::tc_fence_after();
-            const uint32_t d_tmem = tmem_base + (uint32_t)(as * p.BLOCK_N);
+            const uint32_t d_tmem = tmem_base + (uint32_t)(buf.i * p.BLOCK_N);
             for (int j = 0; j < p.n_slices; ++j) {
-                tc::mbar_wait(&ctl->full[stage], phase);
+                tc::mbar_wait(&ctl->full[st.i], st.ph);
                 tc::tc_fence_after();
-                const uint32_t sa = tc::smem_u32(smem + (size_t)stage * stage_bytes);
+                const uint32_t sa = tc::smem_u32(L.ring + (size_t)st.i * L.stage);
                 const uint64_t adesc = tc::make_kmajor_desc(sa, p.kb_bytes);
                 const uint64_t bdesc = tc::make_kmajor_desc(sa + a_bytes, p.kb_bytes);
                 if (tc::elect_one()) {
                     for (int k = 0; k < k_per_block; ++k)
                         tc::umma_bf16_2cta(d_tmem, adesc + (uint64_t)(k * 2), bdesc + (uint64_t)(k * 2), idesc, (j | k) != 0);
-                    tc::umma_commit_2cta(&ctl->empty[stage]);
-                    if (j == p.n_slices - 1) tc::umma_commit_2cta(&ctl->tmem_full[as]);
+                    tc::umma_commit_2cta(&ctl->empty[st.i]);
+                    if (j == p.n_slices - 1) tc::umma_commit_2cta(&ctl->tmem_full[buf.i]);
                 }
                 __syncwarp();
-                if (++stage == p.stages) { stage = 0; phase ^= 1; }
+                st.next(p.stages);
             }
-            if (++as == p.acc_stages) { as = 0; aphase ^= 1; }
+            buf.next(kAccStages);
         }
     } else if (warp >= 4) {
-        EpiCtx c{smem, nullptr, nullptr, ctl, s_scale, s_shift, tmem_base, u_begin, u_end, warp, lane, (int)rank,
-                 {tc::mapa(tc::smem_u32(&ctl->tmem_empty[0]), 0), tc::mapa(tc::smem_u32(&ctl->tmem_empty[1]), 0)}};
-        if (p.epi_mode == 3) epilogue_loop<3, 0, false>(p, c, &tmap_a);
-        else if (p.scale) epilogue_loop<1, 0, true>(p, c, &tmap_a);
-        else epilogue_loop<1, 0, false>(p, c, &tmap_a);
+        const EpiCtx c = epi_ctx<true>(L, ctl, tmem_base, u_begin, u_end);
+        if (p.epi_mode == 3) epilogue_loop<3, 0, false>(p, c, &tmap_out);
+        else if (p.scale) epilogue_loop<1, 0, true>(p, c, &tmap_out);
+        else epilogue_loop<1, 0, false>(p, c, &tmap_out);
     }
-
-    tc::tc_fence_before();
-    tc::cluster_sync_all();
-    if (warp == 2) {
-        tc::tc_fence_after();
-        tc::tmem_dealloc_2cta(tmem_base, kTmemCols);
-    }
+    gemm_teardown<true>(tmem_base);
 }
 
 // The same 3x3 convolution on a CTA PAIR (tcgen05 cta_group::2): the two CTAs of a cluster work on two consecutive
@@ -1063,73 +1027,48 @@ conv_gemm_2cta_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_c
 template <bool STATS>
 __global__ void __launch_bounds__(kThreads, 1)
 conv3x3_2cta_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
+                    const __grid_constant__ CUtensorMap tmap_out, const __grid_constant__ CUtensorMap tmap_gate,
                     const __grid_constant__ KParams p) {
-    extern __shared__ __align__(1024) uint8_t smem_raw[];
-    uint8_t* smem = smem_raw + ((1024u - (tc::smem_u32(smem_raw) & 1023u)) & 1023u);
-    const int b_bytes = (p.BLOCK_N / 2) * 128;                 // this CTA's half of a B tile
+    uint8_t* smem = smem_base();
+    const SmemLayout<uint8_t*> L = smem_layout(kConv3x3Pair, p, smem);
     uint8_t* s_a = smem;
-    uint8_t* s_b = s_a + (size_t)p.sa_stages * p.a_stage_bytes;
-    SmemCtl* ctl = reinterpret_cast<SmemCtl*>(s_b + (size_t)p.stages * b_bytes);
-    float* s_scale = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(ctl) + sizeof(SmemCtl));
-    float* s_shift = s_scale + p.BLOCK_N;
+    uint8_t* s_b = L.ring;
+    SmemCtl* ctl = reinterpret_cast<SmemCtl*>(L.ctl);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t rank = tc::cluster_ctarank();
     const bool leader = rank == 0;
-    if (warp == 0 && lane == 0) {
-        tc::prefetch_tmap(&tmap_a);
-        tc::prefetch_tmap(&tmap_b);
-    }
     if (warp == 1 && lane == 0) {
-        for (int s = 0; s < p.stages; ++s) {
-            tc::mbar_init(&ctl->full[s], 1);
-            tc::mbar_init(&ctl->empty[s], 1);
-        }
         for (int s = 0; s < p.sa_stages; ++s) {
             tc::mbar_init(&ctl->a_full[s], 1);
             tc::mbar_init(&ctl->a_empty[s], 1);
         }
-        for (int s = 0; s < 2; ++s) {
-            tc::mbar_init(&ctl->tmem_full[s], 1);
-            tc::mbar_init(&ctl->tmem_empty[s], 2 * kEpiWarps);     // the epilogue warps of BOTH CTAs
-        }
-        tc::fence_barrier_init();
     }
-    tc::cluster_sync_all();                                            // barriers of both CTAs exist before any remote use
-    if (warp == 2) tc::tmem_alloc_2cta(&ctl->tmem_base, kTmemCols);
-    tc::tc_fence_before();
-    tc::cluster_sync_all();
-    tc::tc_fence_after();
-    const uint32_t tmem_base = ctl->tmem_base;
-
-    // pairs of tiles (2u, 2u+1) are split contiguously over the clusters
-    const int n_pairs = (p.total_tiles + 1) / 2;
-    const int n_clusters = gridDim.x / 2, cid = blockIdx.x / 2;
-    const int per = n_pairs / n_clusters, rem = n_pairs % n_clusters;
-    const int u_begin = cid * per + min(cid, rem);
-    const int u_end = u_begin + per + (cid < rem ? 1 : 0);
+    const uint32_t tmem_base = gemm_prologue<true>(ctl, p, &tmap_a, &tmap_b, &tmap_out, &tmap_gate);
+    // pairs of tiles (2u, 2u+1) are split contiguously over the clusters (one N tile)
+    int u_begin, u_end;
+    work_range<true>(p, u_begin, u_end);
 
     if (warp == 0 && lane == 0) {
         // ================= TMA producer (both CTAs) =================
-        int sa = 0, sb = 0;
-        uint32_t pa = 0, pb = 0;
+        Ring ra, rb;
         for (int u = u_begin; u < u_end; ++u) {
             int img, ty, tx, nt;
             decode_tile(p, pair_tile(p, u, (int)rank), img, ty, tx, nt);
             const int x0 = tx * p.BX, y0 = ty;
             for (int dy = 0; dy < 3; ++dy) {
                 for (int cb = 0; cb < p.c_blocks; ++cb) {
-                    tc::mbar_wait(&ctl->a_empty[sa], pa ^ 1);
-                    if (leader) tc::mbar_expect_tx(&ctl->a_full[sa], 2u * (uint32_t)((kBlockM + 2) * 128));
-                    tc::tma_load_4d_2cta(s_a + (size_t)sa * p.a_stage_bytes, &tmap_a, &ctl->a_full[sa], cb * 64, x0 - 1,
+                    tc::mbar_wait(&ctl->a_empty[ra.i], ra.ph ^ 1);
+                    if (leader) tc::mbar_expect_tx(&ctl->a_full[ra.i], 2u * (uint32_t)((kBlockM + 2) * 128));
+                    tc::tma_load_4d_2cta(s_a + (size_t)ra.i * p.a_stage_bytes, &tmap_a, &ctl->a_full[ra.i], cb * 64, x0 - 1,
                                          y0 + dy - 1, img);
-                    if (++sa == p.sa_stages) { sa = 0; pa ^= 1; }
+                    ra.next(p.sa_stages);
                     for (int dx = 0; dx < 3; ++dx) {
-                        tc::mbar_wait(&ctl->empty[sb], pb ^ 1);
-                        if (leader) tc::mbar_expect_tx(&ctl->full[sb], 2u * (uint32_t)b_bytes);
-                        tc::tma_load_2d_2cta(s_b + (size_t)sb * b_bytes, &tmap_b, &ctl->full[sb],
+                        tc::mbar_wait(&ctl->empty[rb.i], rb.ph ^ 1);
+                        if (leader) tc::mbar_expect_tx(&ctl->full[rb.i], 2u * (uint32_t)L.stage);
+                        tc::tma_load_2d_2cta(s_b + (size_t)rb.i * L.stage, &tmap_b, &ctl->full[rb.i],
                                              ((dy * 3 + dx) * p.c_blocks + cb) * 64, (int)rank * (p.BLOCK_N / 2));
-                        if (++sb == p.stages) { sb = 0; pb ^= 1; }
+                        rb.next(p.stages);
                     }
                 }
             }
@@ -1138,79 +1077,79 @@ conv3x3_2cta_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
         // ================= MMA issuer (leader CTA only): whole warp in uniform control flow, one elected lane issues (keeps the
         // descriptors in uniform registers: no per-MMA ELECT/R2UR waterfall) =================
         const uint32_t idesc = tc::make_idesc_bf16(2 * kBlockM, p.BLOCK_N);
-        int sa = 0, sb = 0, as = 0;
-        uint32_t pa = 0, pb = 0, aphase = 0;
+        Ring ra, rb, buf;
         for (int u = u_begin; u < u_end; ++u) {
-            tc::mbar_wait(&ctl->tmem_empty[as], aphase ^ 1);
+            tc::mbar_wait(&ctl->tmem_empty[buf.i], buf.ph ^ 1);
             tc::tc_fence_after();
-            const uint32_t d_tmem = tmem_base + (uint32_t)(as * p.BLOCK_N);
+            const uint32_t d_tmem = tmem_base + (uint32_t)(buf.i * p.BLOCK_N);
             uint32_t started = 0;
             for (int dy = 0; dy < 3; ++dy) {
                 for (int cb = 0; cb < p.c_blocks; ++cb) {
-                    tc::mbar_wait(&ctl->a_full[sa], pa);
-                    const uint32_t a_base = tc::smem_u32(s_a + (size_t)sa * p.a_stage_bytes);
+                    tc::mbar_wait(&ctl->a_full[ra.i], ra.ph);
+                    const uint32_t a_base = tc::smem_u32(s_a + (size_t)ra.i * p.a_stage_bytes);
                     for (int dx = 0; dx < 3; ++dx) {
-                        tc::mbar_wait(&ctl->full[sb], pb);
+                        tc::mbar_wait(&ctl->full[rb.i], rb.ph);
                         tc::tc_fence_after();
                         const uint64_t adesc = tc::make_kmajor_desc(a_base + (uint32_t)(dx * 128), 128);
-                        const uint64_t bdesc = tc::make_kmajor_desc(tc::smem_u32(s_b + (size_t)sb * b_bytes), 128);
+                        const uint64_t bdesc = tc::make_kmajor_desc(tc::smem_u32(s_b + (size_t)rb.i * L.stage), 128);
                         if (tc::elect_one()) {
 #pragma unroll
                             for (int k = 0; k < 4; ++k)
                                 tc::umma_bf16_2cta(d_tmem, adesc + (uint64_t)(k * 2), bdesc + (uint64_t)(k * 2), idesc,
                                                    (started | k) ? 1u : 0u);
-                            tc::umma_commit_2cta(&ctl->empty[sb]);
+                            tc::umma_commit_2cta(&ctl->empty[rb.i]);
                             if (dx == 2) {
-                                tc::umma_commit_2cta(&ctl->a_empty[sa]);
-                                if (dy == 2 && cb == p.c_blocks - 1) tc::umma_commit_2cta(&ctl->tmem_full[as]);
+                                tc::umma_commit_2cta(&ctl->a_empty[ra.i]);
+                                if (dy == 2 && cb == p.c_blocks - 1) tc::umma_commit_2cta(&ctl->tmem_full[buf.i]);
                             }
                         }
                         __syncwarp();
                         started = 1;
-                        if (++sb == p.stages) { sb = 0; pb ^= 1; }
+                        rb.next(p.stages);
                     }
-                    if (++sa == p.sa_stages) { sa = 0; pa ^= 1; }
+                    ra.next(p.sa_stages);
                 }
             }
-            if (++as == p.acc_stages) { as = 0; aphase ^= 1; }
+            buf.next(kAccStages);
         }
     } else if (warp >= 4) {
         // ================= epilogue (both CTAs, each on its own 128 TMEM lanes) =================
-        EpiCtx c{smem, nullptr, nullptr, ctl, s_scale, s_shift, tmem_base, u_begin, u_end, warp, lane, (int)rank,
-                 {tc::mapa(tc::smem_u32(&ctl->tmem_empty[0]), 0), tc::mapa(tc::smem_u32(&ctl->tmem_empty[1]), 0)}};
-        if (STATS) epilogue_loop<2, 3, false>(p, c, &tmap_a);
-        else if (p.scale) epilogue_loop<2, 1, true>(p, c, &tmap_a);
-        else epilogue_loop<2, 1, false>(p, c, &tmap_a);
+        const EpiCtx c = epi_ctx<true>(L, ctl, tmem_base, u_begin, u_end);
+        if (STATS) epilogue_loop<2, 3, false>(p, c, &tmap_out);
+        else if (p.scale) epilogue_loop<2, 1, true>(p, c, &tmap_out);
+        else epilogue_loop<2, 1, false>(p, c, &tmap_out);
     }
-
-    tc::tc_fence_before();
-    tc::cluster_sync_all();                       // the peer's smem / TMEM stay alive until the leader's MMAs are done
-    if (warp == 2) {
-        tc::tc_fence_after();
-        tc::tmem_dealloc_2cta(tmem_base, kTmemCols);
-    }
+    gemm_teardown<true>(tmem_base);
 }
 
 // ---- host side ------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+using GemmKernel = void (*)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, KParams);
 
-EncodeTiledFn get_encode_fn() {
-    static EncodeTiledFn fn = nullptr;
-    if (!fn) {
-        void* ptr = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &qres) == cudaSuccess &&
-            qres == cudaDriverEntryPointSuccess)
-            fn = (EncodeTiledFn)ptr;
+// the statistics epilogue (act 3, train-mode BatchNorm) lives in its own instantiations: it needs 17 more registers, which
+// the inference kernels should not pay for
+GemmKernel gemm_kernel(GemmKind kind, bool stats) {
+    switch (kind) {
+    case kGemm:
+        if (stats) return conv_gemm_kernel<true>;
+        return conv_gemm_kernel<false>;
+    case kGemmPair:
+        return conv_gemm_2cta_kernel;
+    case kConv3x3:
+        if (stats) return conv3x3_kernel<true>;
+        return conv3x3_kernel<false>;
+    case kConv3x3Pair:
+        if (stats) return conv3x3_2cta_kernel<true>;
+        return conv3x3_2cta_kernel<false>;
+    case kDsam:
+        break;
     }
-    return fn;
+    return dsam_fwd_kernel;
 }
 
 }  // namespace
 
 extern "C" int rgbd_conv_gemm(const rgbd_conv_gemm_desc* d, rgbd_stream_t stream) {
+    // ---- validate
     RGBD_CHECK_ARG(d, "conv_gemm: null descriptor");
     RGBD_CHECK_ARG(d->a && d->w && (d->slices || d->conv3x3_reuse || d->dsam_masked), "conv_gemm: null operand pointer");
     RGBD_CHECK_ARG(d->kb_elems == 64 || d->kb_elems == 32, "conv_gemm: kb_elems must be 64 or 32 (got %d)", d->kb_elems);
@@ -1258,65 +1197,9 @@ extern "C" int rgbd_conv_gemm(const rgbd_conv_gemm_desc* d, rgbd_stream_t stream
     if (d->epi_mode == 0)
         RGBD_CHECK_ARG(d->block_n % 64 == 0, "conv_gemm: the channels-last epilogue needs BLOCK_N %% 64 == 0 (got %d)", d->block_n);
     RGBD_CHECK_ARG(d->epi_mode == 0 || !d->gate, "conv_gemm: gate is only supported by epilogue mode 0");
-    EncodeTiledFn encode = get_encode_fn();
-    if (!encode) {
-        rgbd_set_error("conv_gemm: cuTensorMapEncodeTiled is not available from the driver");
-        return RGBD_ERR_CUDA;
-    }
+
+    // ---- plan: kernel, buffers, stage count, grid
     const int kb_bytes = d->kb_elems * 2;
-    const CUtensorMapSwizzle swz = kb_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
-
-    CUtensorMap tmap_a, tmap_b;
-    {
-        cuuint64_t dims[4] = {(cuuint64_t)d->a_c, (cuuint64_t)d->a_x, (cuuint64_t)d->a_y, (cuuint64_t)d->a_planes};
-        cuuint64_t strides[3] = {(cuuint64_t)d->a_c * 2, (cuuint64_t)d->a_c * 2 * d->a_x,
-                                 (cuuint64_t)d->a_c * 2 * d->a_x * d->a_y};
-        cuuint32_t box[4] = {(cuuint32_t)d->kb_elems, (cuuint32_t)(d->conv3x3_reuse ? d->bx + 2 : d->bx), (cuuint32_t)d->by, 1};
-        cuuint32_t estr[4] = {1, 1, 1, 1};
-        CUresult r = encode(&tmap_a, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(d->a), dims, strides, box, estr,
-                            CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) {
-            rgbd_set_error("conv_gemm: cuTensorMapEncodeTiled(A) failed with %d", (int)r);
-            return RGBD_ERR_CUDA;
-        }
-    }
-    const long long k_total = d->conv3x3_reuse ? 9ll * d->a_c
-                              : d->dsam_masked ? 9ll * d->a_c * d->m3_n_seg : (long long)d->n_slices * d->kb_elems;
-    {
-        cuuint64_t dims[2] = {(cuuint64_t)k_total, (cuuint64_t)d->n_pad};
-        cuuint64_t strides[1] = {(cuuint64_t)k_total * 2};
-        cuuint32_t box[2] = {(cuuint32_t)d->kb_elems, (cuuint32_t)d->block_n};
-        cuuint32_t estr[2] = {1, 1};
-        CUresult r = encode(&tmap_b, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(d->w), dims, strides, box, estr,
-                            CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) {
-            rgbd_set_error("conv_gemm: cuTensorMapEncodeTiled(B) failed with %d", (int)r);
-            return RGBD_ERR_CUDA;
-        }
-    }
-
-    CUtensorMap tmap_out = tmap_a, tmap_gate = tmap_a;   // placeholders unless epilogue mode 0 uses them
-    if (d->epi_mode == 0) {
-        cuuint64_t dims[4] = {(cuuint64_t)d->n_pad, (cuuint64_t)d->out_w, (cuuint64_t)d->out_h, (cuuint64_t)d->n_img};
-        cuuint64_t strides[3] = {(cuuint64_t)d->n_pad * 2, (cuuint64_t)d->n_pad * 2 * d->out_w,
-                                 (cuuint64_t)d->n_pad * 2 * d->out_w * d->out_h};
-        cuuint32_t box[4] = {64, (cuuint32_t)d->bx, (cuuint32_t)d->by, 1};
-        cuuint32_t estr[4] = {1, 1, 1, 1};
-        CUresult r = encode(&tmap_out, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, d->out, dims, strides, box, estr,
-                            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r == CUDA_SUCCESS && d->gate)
-            r = encode(&tmap_gate, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(d->gate), dims, strides, box, estr,
-                       CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                       CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) {
-            rgbd_set_error("conv_gemm: cuTensorMapEncodeTiled(out/gate) failed with %d", (int)r);
-            return RGBD_ERR_CUDA;
-        }
-    }
-
     KParams p;
     p.n_img = d->n_img;
     p.BX = d->bx; p.BY = d->by;
@@ -1330,15 +1213,11 @@ extern "C" int rgbd_conv_gemm(const rgbd_conv_gemm_desc* d, rgbd_stream_t stream
     p.next_c_pad = d->next_c_pad; p.next_n_seg = d->next_n_seg; p.next_masked_segs = d->next_masked_segs;
     p.kb_bytes = kb_bytes;
     p.c_blocks = d->a_c / 64;
-    p.sa_stages = 0;
-    p.a_stage_bytes = 0;
     p.N = d->n; p.N_pad = d->n_pad; p.BLOCK_N = d->block_n; p.n_tiles_n = d->n_pad / d->block_n;
     p.plane_per_img = d->plane_per_img;
     p.tile_order = d->tile_order;
     p.slices = reinterpret_cast<const int4*>(d->slices);
     p.epi_mode = d->epi_mode; p.act = d->act;
-    const bool stats = d->epi_mode == 2 && d->act == 3;
-    p.acc_stages = 2;
     p.scale = d->scale; p.shift = d->shift; p.variant = d->variant;
     p.gate = reinterpret_cast<const __nv_bfloat16*>(d->gate);
     p.out = d->out; p.residual = d->residual; p.pool = d->pool; p.pool_sq = d->pool_sq;
@@ -1349,178 +1228,79 @@ extern "C" int rgbd_conv_gemm(const rgbd_conv_gemm_desc* d, rgbd_stream_t stream
     const long long total = (long long)p.n_img * p.tiles_x * p.tiles_y * p.n_tiles_n;
     RGBD_CHECK_ARG(total < (1ll << 31), "conv_gemm: too many tiles");
     p.total_tiles = (int)total;
+    const int total_m = p.total_tiles / p.n_tiles_n;
+    p.b_resident = 0; p.b_res_bytes = 0;
+    p.staging_bytes = d->epi_mode == 0 ? (p.BLOCK_N / 64) * kBlockM * 128 : 0;
+    p.gate_bytes = (d->epi_mode == 0 && d->gate) ? p.staging_bytes : 0;
+    p.sa_stages = 0; p.a_stage_bytes = 0;
+    GemmKind kind;
+    if (d->conv3x3_reuse) {
+        p.gate_bytes = 0;                                 // the 3x3 kernels take no gate
+        p.sa_stages = 3;
+        p.a_stage_bytes = 17 * 1024;                      // (128+2) rows x 128 B, rounded up to the swizzle period
+        const bool pair = d->epi_mode == 2 && p.n_tiles_n == 1 && p.BLOCK_N % 32 == 0 && (p.BLOCK_N / 2) % 8 == 0 && p.total_tiles >= 2;
+        kind = pair ? kConv3x3Pair : kConv3x3;
+    } else if (d->dsam_masked) {
+        kind = kDsam;
+    } else {
+        const int b_total = p.n_slices * p.BLOCK_N * kb_bytes;
+        p.b_resident = (p.n_tiles_n == 1 && b_total <= 100 * 1024) ? 1 : 0;
+        p.b_res_bytes = p.b_resident ? b_total : 0;
+        const bool pair = (d->epi_mode == 1 || d->epi_mode == 3) && !p.b_resident && total_m >= 2 && (p.BLOCK_N / 2) % 16 == 0;
+        kind = pair ? kGemmPair : kGemm;
+    }
+    const bool pair = kind == kGemmPair || kind == kConv3x3Pair || kind == kDsam;
+    const bool stats = d->epi_mode == 2 && d->act == 3;
 
     RgbdDeviceInfo di;
     if (int rc = rgbd_device_info(&di)) return rc;
     const int num_sms = di.num_sms, max_smem = di.max_smem;
     RGBD_ONCE_PER_DEVICE(di.device, {
-        RGBD_CHECK_CUDA(cudaFuncSetAttribute(conv_gemm_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-        RGBD_CHECK_CUDA(cudaFuncSetAttribute(conv3x3_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-        RGBD_CHECK_CUDA(cudaFuncSetAttribute(conv3x3_2cta_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-        // the statistics epilogue (act 3, train-mode BatchNorm) lives in its own instantiations: it needs 17 more registers,
-        // which the inference kernels should not pay for
-        RGBD_CHECK_CUDA(cudaFuncSetAttribute(conv_gemm_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-        RGBD_CHECK_CUDA(cudaFuncSetAttribute(conv3x3_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-        RGBD_CHECK_CUDA(cudaFuncSetAttribute(conv3x3_2cta_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-        RGBD_CHECK_CUDA(cudaFuncSetAttribute(conv_gemm_2cta_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-        RGBD_CHECK_CUDA(cudaFuncSetAttribute(dsam_fwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-        RGBD_CHECK_CUDA(cudaFuncSetAttribute(dsam_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
+        for (int k = kGemm; k <= kDsam; ++k)
+            for (int st = 0; st < 2; ++st)
+                RGBD_CHECK_CUDA(cudaFuncSetAttribute(gemm_kernel((GemmKind)k, st), cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
     });
-    const int grid = p.total_tiles < num_sms ? p.total_tiles : num_sms;
-    if (d->conv3x3_reuse) {
-        p.b_resident = 0; p.b_res_bytes = 0;
-        p.staging_bytes = d->epi_mode == 0 ? (p.BLOCK_N / 64) * kBlockM * 128 : 0;
-        p.gate_bytes = 0;
-        p.sa_stages = 3;
-        p.a_stage_bytes = 17 * 1024;                      // (128+2) rows x 128 B, rounded up to the swizzle period
-        const int b_stage = p.BLOCK_N * 128;
-        const int fixed3 = 1024 + (int)sizeof(SmemCtl) + 64 + p.staging_bytes + 2 * p.BLOCK_N * (int)sizeof(float) +
-                           p.sa_stages * p.a_stage_bytes;
-        int sb = (max_smem - fixed3) / b_stage;
-        if (sb > kMaxStages) sb = kMaxStages;
-        RGBD_CHECK_ARG(sb >= 2, "conv_gemm: not enough shared memory for the 3x3 A-reuse pipeline");
-        p.stages = sb;
-        const int smem3 = fixed3 + sb * b_stage;
-        static const bool no_pair = getenv("RGBD_NO_CTA_PAIR") != nullptr;
-        if (d->epi_mode == 2 && p.n_tiles_n == 1 && p.BLOCK_N % 32 == 0 && (p.BLOCK_N / 2) % 8 == 0 && p.total_tiles >= 2 && !no_pair) {
-            // CTA-pair kernel: each CTA stages half of every B tile (box rows = BLOCK_N/2)
-            CUtensorMap tmap_b2;
-            cuuint64_t dims[2] = {(cuuint64_t)k_total, (cuuint64_t)d->n_pad};
-            cuuint64_t strides[1] = {(cuuint64_t)k_total * 2};
-            cuuint32_t box[2] = {64, (cuuint32_t)(p.BLOCK_N / 2)};
-            cuuint32_t estr[2] = {1, 1};
-            CUresult r = encode(&tmap_b2, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(d->w), dims, strides, box, estr,
-                                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-            if (r != CUDA_SUCCESS) {
-                rgbd_set_error("conv_gemm: cuTensorMapEncodeTiled(B half) failed with %d", (int)r);
-                return RGBD_ERR_CUDA;
-            }
-            const int b_half = (p.BLOCK_N / 2) * 128;
-            const int fixed2 = 1024 + (int)sizeof(SmemCtl) + 64 + 2 * p.BLOCK_N * (int)sizeof(float) + p.sa_stages * p.a_stage_bytes;
-            int sb2 = (max_smem - fixed2) / b_half;
-            if (sb2 > kMaxStages) sb2 = kMaxStages;
-            p.stages = sb2;
-            const int n_pairs = (p.total_tiles + 1) / 2;
-            int clusters = num_sms / 2;
-            if (clusters > n_pairs) clusters = n_pairs;
-            cudaLaunchConfig_t cfg = {};
-            cfg.gridDim = dim3(2 * clusters);
-            cfg.blockDim = dim3(kThreads);
-            cfg.dynamicSmemBytes = fixed2 + sb2 * b_half;
-            cfg.stream = (cudaStream_t)stream;
-            cudaLaunchAttribute attr[1];
-            attr[0].id = cudaLaunchAttributeClusterDimension;
-            attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-            cfg.attrs = attr;
-            cfg.numAttrs = 1;
-            if (stats) RGBD_CHECK_CUDA(cudaLaunchKernelEx(&cfg, conv3x3_2cta_kernel<true>, tmap_a, tmap_b2, p));
-            else RGBD_CHECK_CUDA(cudaLaunchKernelEx(&cfg, conv3x3_2cta_kernel<false>, tmap_a, tmap_b2, p));
-            return RGBD_OK;
-        }
-        if (stats) conv3x3_kernel<true><<<grid, kThreads, smem3, (cudaStream_t)stream>>>(tmap_a, tmap_b, tmap_out, tmap_gate, p);
-        else conv3x3_kernel<false><<<grid, kThreads, smem3, (cudaStream_t)stream>>>(tmap_a, tmap_b, tmap_out, tmap_gate, p);
-        RGBD_CHECK_LAUNCH();
-        return RGBD_OK;
-    }
-    if (d->dsam_masked) {
-        p.b_resident = 0; p.b_res_bytes = 0; p.staging_bytes = 0; p.gate_bytes = 0;
-        CUtensorMap tmap_b2;
-        cuuint64_t dims[2] = {(cuuint64_t)k_total, (cuuint64_t)d->n_pad};
-        cuuint64_t strides[1] = {(cuuint64_t)k_total * 2};
-        cuuint32_t box[2] = {64, (cuuint32_t)(p.BLOCK_N / 2)};
-        cuuint32_t estr[2] = {1, 1};
-        CUresult r = encode(&tmap_b2, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(d->w), dims, strides, box, estr,
-                            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) {
-            rgbd_set_error("conv_gemm: cuTensorMapEncodeTiled(B half) failed with %d", (int)r);
-            return RGBD_ERR_CUDA;
-        }
-        const int b_half = (p.BLOCK_N / 2) * 128;
-        const char* tmem_e = getenv("RGBD_DSAM_TMEM");                  // A/B switch (read per launch)
-        const bool tmem_env = tmem_e == nullptr || tmem_e[0] != (char)48;
-        const bool tmem_a = tmem_env && p.BLOCK_N <= 256 && p.m3_masked_segs <= 4;   // masked copies in tensor memory
-        if (tmem_a) p.acc_stages = 1;
-        const int fixedm = 1024 + (int)sizeof(SmemCtl) + 64 + 2 * p.BLOCK_N * (int)sizeof(float) +
-                           (kDsamRaw + (tmem_a ? 0 : 2 * p.m3_masked_segs)) * kBlockM * 128;
-        int sbm = (max_smem - fixedm) / b_half;
-        if (sbm > kMaxStages) sbm = kMaxStages;
-        RGBD_CHECK_ARG(sbm >= 2, "conv_gemm: not enough shared memory for the masked DSAM pipeline");
-        p.stages = sbm;
-        const int total_m = p.total_tiles / p.n_tiles_n;
+    // dynamic shared memory: the layout, the alignment slack and 64 bytes
+    p.stages = 0;
+    const SmemLayout<size_t> fixed = smem_layout(kind, p, (size_t)0);
+    p.stages = (max_smem - 1024 - (int)fixed.end - 64) / fixed.stage;
+    if (p.stages > kMaxStages) p.stages = kMaxStages;
+    RGBD_CHECK_ARG(p.stages >= 2, "conv_gemm: not enough shared memory for 2 pipeline stages");
+    int smem_bytes = 1024 + (int)smem_layout(kind, p, (size_t)0).end + 64;
+    // the slice-table kernels always take (almost) the whole SM so exactly one CTA (and its 512 TMEM columns) is resident
+    if ((kind == kGemm || kind == kGemmPair) && smem_bytes < 160 * 1024) smem_bytes = 160 * 1024;
+    int grid = p.total_tiles < num_sms ? p.total_tiles : num_sms;
+    if (pair) {
         const int n_units = ((total_m + 1) / 2) * p.n_tiles_n;
-        int clusters = num_sms / 2;
-        if (clusters > n_units) clusters = n_units;
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3(2 * clusters);
-        cfg.blockDim = dim3(kDsamThreads);
-        cfg.dynamicSmemBytes = fixedm + sbm * b_half;
-        cfg.stream = (cudaStream_t)stream;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = 1;
-        if (tmem_a) RGBD_CHECK_CUDA(cudaLaunchKernelEx(&cfg, dsam_fwd_kernel<true>, tmap_a, tmap_b2, p));
-        else RGBD_CHECK_CUDA(cudaLaunchKernelEx(&cfg, dsam_fwd_kernel<false>, tmap_a, tmap_b2, p));
-        return RGBD_OK;
+        const int clusters = num_sms / 2 < n_units ? num_sms / 2 : n_units;
+        grid = 2 * clusters;
     }
-    const int b_total = p.n_slices * p.BLOCK_N * kb_bytes;
-    p.b_resident = (p.n_tiles_n == 1 && b_total <= 100 * 1024) ? 1 : 0;
-    p.b_res_bytes = p.b_resident ? b_total : 0;
-    const int stage_bytes = kBlockM * kb_bytes + (p.b_resident ? 0 : p.BLOCK_N * kb_bytes);
-    p.staging_bytes = d->epi_mode == 0 ? (p.BLOCK_N / 64) * kBlockM * 128 : 0;
-    p.gate_bytes = (d->epi_mode == 0 && d->gate) ? p.staging_bytes : 0;
-    const int fixed = 1024 + (int)sizeof(SmemCtl) + p.n_slices * 16 + 64 + p.staging_bytes + p.gate_bytes +
-                      2 * p.BLOCK_N * (int)sizeof(float) + p.b_res_bytes;
-    int stages = (max_smem - fixed) / stage_bytes;
-    if (stages > kMaxStages) stages = kMaxStages;
-    RGBD_CHECK_ARG(stages >= 2, "conv_gemm: not enough shared memory for 2 stages");
-    p.stages = stages;
-    // always take (almost) the whole SM so exactly one CTA (and its 512 TMEM columns) is resident
-    int smem_bytes = fixed + stages * stage_bytes;
-    if (smem_bytes < 160 * 1024) smem_bytes = 160 * 1024;
-    static const bool no_pair_g = getenv("RGBD_NO_CTA_PAIR") != nullptr;
-    const int total_m = p.total_tiles / p.n_tiles_n;
-    if ((d->epi_mode == 1 || d->epi_mode == 3) && !p.b_resident && !no_pair_g && total_m >= 2 && (p.BLOCK_N / 2) % 16 == 0) {
-        CUtensorMap tmap_b2;
-        cuuint64_t dims[2] = {(cuuint64_t)k_total, (cuuint64_t)d->n_pad};
-        cuuint64_t strides[1] = {(cuuint64_t)k_total * 2};
-        cuuint32_t box[2] = {(cuuint32_t)d->kb_elems, (cuuint32_t)(p.BLOCK_N / 2)};
-        cuuint32_t estr[2] = {1, 1};
-        CUresult r = encode(&tmap_b2, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(d->w), dims, strides, box, estr,
-                            CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) {
-            rgbd_set_error("conv_gemm: cuTensorMapEncodeTiled(B half) failed with %d", (int)r);
-            return RGBD_ERR_CUDA;
-        }
-        const int stage2 = kBlockM * kb_bytes + (p.BLOCK_N / 2) * kb_bytes;
-        const int fixed2 = 1024 + (int)sizeof(SmemCtl) + p.n_slices * 16 + 64 + 2 * p.BLOCK_N * (int)sizeof(float);
-        int st2 = (max_smem - fixed2) / stage2;
-        if (st2 > kMaxStages) st2 = kMaxStages;
-        p.stages = st2;
-        const int n_units = ((total_m + 1) / 2) * p.n_tiles_n;
-        int clusters = num_sms / 2;
-        if (clusters > n_units) clusters = n_units;
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3(2 * clusters);
-        cfg.blockDim = dim3(kThreads);
-        int smem2 = fixed2 + st2 * stage2;
-        if (smem2 < 160 * 1024) smem2 = 160 * 1024;
-        cfg.dynamicSmemBytes = smem2;
-        cfg.stream = (cudaStream_t)stream;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = 1;
-        RGBD_CHECK_CUDA(cudaLaunchKernelEx(&cfg, conv_gemm_2cta_kernel, tmap_a, tmap_b2, p));
-        return RGBD_OK;
+
+    // ---- encode the tensor maps
+    const CUtensorMapSwizzle swz = kb_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
+    const long long a_px = 2ll * d->a_c, a_row = a_px * d->a_x;
+    CUtensorMap tmap_a, tmap_b;
+    if (int rc = encode_bf16_map(&tmap_a, "conv_gemm(A)", d->a, {d->a_c, d->a_x, d->a_y, d->a_planes}, {a_px, a_row, a_row * d->a_y},
+                                 {d->kb_elems, d->conv3x3_reuse ? d->bx + 2 : d->bx, d->by, 1}, swz))
+        return rc;
+    // B: [N_pad][K], K-major; a CTA pair stages half of the BLOCK_N rows in each CTA
+    const long long k_total = d->conv3x3_reuse ? 9ll * d->a_c
+                              : d->dsam_masked ? 9ll * d->a_c * d->m3_n_seg : (long long)d->n_slices * d->kb_elems;
+    if (int rc = encode_bf16_map(&tmap_b, "conv_gemm(B)", d->w, {k_total, d->n_pad}, {k_total * 2},
+                                 {d->kb_elems, pair ? p.BLOCK_N / 2 : p.BLOCK_N}, swz))
+        return rc;
+    CUtensorMap tmap_out = tmap_a, tmap_gate = tmap_a;   // placeholders unless epilogue mode 0 uses them
+    if (d->epi_mode == 0) {
+        const long long o_px = 2ll * d->n_pad, o_row = o_px * d->out_w;
+        if (int rc = encode_bf16_map(&tmap_out, "conv_gemm(out)", d->out, {d->n_pad, d->out_w, d->out_h, d->n_img},
+                                     {o_px, o_row, o_row * d->out_h}, {64, d->bx, d->by, 1}, CU_TENSOR_MAP_SWIZZLE_128B))
+            return rc;
+        if (d->gate)
+            if (int rc = encode_bf16_map(&tmap_gate, "conv_gemm(gate)", d->gate, {d->n_pad, d->out_w, d->out_h, d->n_img},
+                                         {o_px, o_row, o_row * d->out_h}, {64, d->bx, d->by, 1}, CU_TENSOR_MAP_SWIZZLE_128B))
+                return rc;
     }
-    if (stats) conv_gemm_kernel<true><<<grid, kThreads, smem_bytes, (cudaStream_t)stream>>>(tmap_a, tmap_b, tmap_out, tmap_gate, p);
-    else conv_gemm_kernel<false><<<grid, kThreads, smem_bytes, (cudaStream_t)stream>>>(tmap_a, tmap_b, tmap_out, tmap_gate, p);
-    RGBD_CHECK_LAUNCH();
-    return RGBD_OK;
+
+    return launch_kernel(gemm_kernel(kind, stats), grid, kind == kDsam ? kDsamThreads : kThreads, smem_bytes, pair,
+                         (cudaStream_t)stream, tmap_a, tmap_b, tmap_out, tmap_gate, p);
 }

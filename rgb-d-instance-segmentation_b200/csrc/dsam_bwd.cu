@@ -15,6 +15,7 @@
 #include "common.cuh"
 #include "rgbd_b200.h"
 #include "tc_ptx.cuh"
+#include "tma_host.cuh"
 #include <stdlib.h>
 
 namespace {
@@ -218,31 +219,6 @@ __global__ void __launch_bounds__(256) dsam_dbias_kernel(const float* __restrict
     }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn wg_encode_fn() {
-    static EncodeTiledFn fn = nullptr;
-    if (!fn) {
-        void* ptr = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &qres) == cudaSuccess &&
-            qres == cudaDriverEntryPointSuccess)
-            fn = (EncodeTiledFn)ptr;
-    }
-    return fn;
-}
-
-bool make_pix_map(EncodeTiledFn enc, CUtensorMap* m, const void* base, long long pix, int rows, int planes, int box_rows) {
-    cuuint64_t dims[3] = {(cuuint64_t)pix, (cuuint64_t)rows, (cuuint64_t)planes};
-    cuuint64_t strides[2] = {(cuuint64_t)pix * 2, (cuuint64_t)pix * 2 * rows};
-    cuuint32_t box[3] = {64, (cuuint32_t)box_rows, 1};
-    cuuint32_t estr[3] = {1, 1, 1};
-    return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), dims, strides, box, estr,
-               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
 }  // namespace
 
 extern "C" int rgbd_cast_bf16_pitched(const float* src, void* dst_bf16, long long rows, int W, int W_pitch,
@@ -284,11 +260,6 @@ extern "C" int rgbd_dsam_wgrad(const void* g_bf16, int g_w_pitch, const void* xt
     RGBD_CHECK_ARG(B >= 1 && N_out >= 1 && C_pad >= 32 && C_pad % 32 == 0 && Ho >= 1 && Wo >= 1 && n_seg >= 1 && n_seg <= 8,
                    "dsam_wgrad: bad geometry");
     RGBD_CHECK_ARG(g_w_pitch % 8 == 0 && x_w_pitch % 8 == 0 && g_w_pitch >= Wo, "dsam_wgrad: row pitches must be multiples of 8");
-    EncodeTiledFn enc = wg_encode_fn();
-    if (!enc) {
-        rgbd_set_error("dsam_wgrad: cuTensorMapEncodeTiled is not available from the driver");
-        return RGBD_ERR_CUDA;
-    }
     WgradParams p;
     p.B = B; p.Ho = Ho; p.Wo = Wo; p.N_out = N_out; p.Cp = C_pad;
     p.n_seg = n_seg;
@@ -331,13 +302,15 @@ extern "C" int rgbd_dsam_wgrad(const void* g_bf16, int g_w_pitch, const void* xt
     if (stages > kMaxStagesW) stages = kMaxStagesW;
     RGBD_CHECK_ARG(stages >= 2, "dsam_wgrad: not enough shared memory");
     p.stages = stages;
+    // channel-major operands: (pixels, channels, planes), pixels innermost
     CUtensorMap m_g, m_x;
-    const int x_planes = B * n_seg * p.n_par;
-    if (!make_pix_map(enc, &m_g, g_bf16, (long long)Ho * g_w_pitch, N_out, B, kBlockM) ||
-        !make_pix_map(enc, &m_x, xt_bf16, (long long)x_h * x_w_pitch, C_pad, x_planes, p.BLOCK_N)) {
-        rgbd_set_error("dsam_wgrad: cuTensorMapEncodeTiled failed");
-        return RGBD_ERR_CUDA;
-    }
+    const long long g_pix = (long long)Ho * g_w_pitch, x_pix = (long long)x_h * x_w_pitch;
+    if (int rc = encode_bf16_map(&m_g, "dsam_wgrad", g_bf16, {g_pix, N_out, B}, {g_pix * 2, g_pix * 2 * N_out}, {64, kBlockM, 1},
+                                 CU_TENSOR_MAP_SWIZZLE_128B))
+        return rc;
+    if (int rc = encode_bf16_map(&m_x, "dsam_wgrad", xt_bf16, {x_pix, C_pad, B * n_seg * p.n_par},
+                                 {x_pix * 2, x_pix * 2 * C_pad}, {64, p.BLOCK_N, 1}, CU_TENSOR_MAP_SWIZZLE_128B))
+        return rc;
     RGBD_CHECK_CUDA(cudaMemsetAsync(dw, 0, sizeof(float) * (size_t)N_out * n_seg * p.taps * C_pad, (cudaStream_t)stream));
     int smem_bytes = 1024 + stages * stage_bytes + (int)sizeof(WCtl) + 64;
     if (smem_bytes < 120 * 1024) smem_bytes = 120 * 1024;     // one CTA per SM (TMEM allocation)

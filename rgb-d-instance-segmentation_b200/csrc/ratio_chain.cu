@@ -14,6 +14,7 @@
 #include "common.cuh"
 #include "rgbd_b200.h"
 #include "tc_ptx.cuh"
+#include "tma_host.cuh"
 
 namespace {
 
@@ -274,42 +275,6 @@ ratio_chain_kernel(const __grid_constant__ CUtensorMap tmap_x1, const __grid_con
     }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn encode_fn() {
-    static EncodeTiledFn fn = nullptr;
-    if (!fn) {
-        void* ptr = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &qres) == cudaSuccess &&
-            qres == cudaDriverEntryPointSuccess)
-            fn = (EncodeTiledFn)ptr;
-    }
-    return fn;
-}
-
-bool make_nhwc_map(EncodeTiledFn enc, CUtensorMap* m, const void* base, int c, int w, int h, int n, int bx, int by) {
-    cuuint64_t dims[4] = {(cuuint64_t)c, (cuuint64_t)w, (cuuint64_t)h, (cuuint64_t)n};
-    cuuint64_t strides[3] = {(cuuint64_t)c * 2, (cuuint64_t)c * 2 * w, (cuuint64_t)c * 2 * w * h};
-    cuuint32_t box[4] = {64, (cuuint32_t)bx, (cuuint32_t)by, 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(base), dims, strides, box, estr,
-               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
-bool make_weight_map(EncodeTiledFn enc, CUtensorMap* m, const void* base, int k, int n) {
-    cuuint64_t dims[2] = {(cuuint64_t)k, (cuuint64_t)n};
-    cuuint64_t strides[1] = {(cuuint64_t)k * 2};
-    cuuint32_t box[2] = {64, (cuuint32_t)n};
-    cuuint32_t estr[2] = {1, 1};
-    return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
-               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
 }  // namespace
 
 extern "C" int rgbd_ratio_chain(const void* x1_bf16, const void* w2_bf16, const void* w3_bf16, const void* w4_bf16,
@@ -318,18 +283,16 @@ extern "C" int rgbd_ratio_chain(const void* x1_bf16, const void* w2_bf16, const 
     RGBD_CHECK_ARG(x1_bf16 && w2_bf16 && w3_bf16 && w4_bf16 && sh2 && sh3 && sh4 && out_bf16, "ratio_chain: null pointer");
     RGBD_CHECK_ARG(B >= 1 && H >= 1 && W >= 1, "ratio_chain: bad geometry");
     RGBD_CHECK_ARG(bx >= 1 && by >= 1 && bx * by == kBlockM && bx <= 256 && by <= 256, "ratio_chain: box must cover 128 pixels");
-    EncodeTiledFn enc = encode_fn();
-    if (!enc) {
-        rgbd_set_error("ratio_chain: cuTensorMapEncodeTiled is not available from the driver");
-        return RGBD_ERR_CUDA;
-    }
+    const char* who = "ratio_chain";
+    const CUtensorMapSwizzle sw128 = CU_TENSOR_MAP_SWIZZLE_128B;
+    const long long x1_row = 192 * 2 * (long long)W, o_row = 128 * 2 * (long long)W;
     CUtensorMap m_x1, m_w2, m_w3, m_w4, m_out;
-    if (!make_nhwc_map(enc, &m_x1, x1_bf16, 192, W, H, B, bx, by) || !make_nhwc_map(enc, &m_out, out_bf16, 128, W, H, B, bx, by) ||
-        !make_weight_map(enc, &m_w2, w2_bf16, 192, 128) || !make_weight_map(enc, &m_w3, w3_bf16, 128, 64) ||
-        !make_weight_map(enc, &m_w4, w4_bf16, 64, 128)) {
-        rgbd_set_error("ratio_chain: cuTensorMapEncodeTiled failed");
-        return RGBD_ERR_CUDA;
-    }
+    if (int rc = encode_bf16_map(&m_x1, who, x1_bf16, {192, W, H, B}, {192 * 2, x1_row, x1_row * H}, {64, bx, by, 1}, sw128)) return rc;
+    if (int rc = encode_bf16_map(&m_out, who, out_bf16, {128, W, H, B}, {128 * 2, o_row, o_row * H}, {64, bx, by, 1}, sw128)) return rc;
+    // (n, k) weight matrices, one box of 64 K elements x all n rows
+    if (int rc = encode_bf16_map(&m_w2, who, w2_bf16, {192, 128}, {192 * 2}, {64, 128}, sw128)) return rc;
+    if (int rc = encode_bf16_map(&m_w3, who, w3_bf16, {128, 64}, {128 * 2}, {64, 64}, sw128)) return rc;
+    if (int rc = encode_bf16_map(&m_w4, who, w4_bf16, {64, 128}, {64 * 2}, {64, 128}, sw128)) return rc;
     ChainParams p;
     p.n_img = B; p.BX = bx; p.BY = by;
     p.tiles_x = ceil_div(W, bx);

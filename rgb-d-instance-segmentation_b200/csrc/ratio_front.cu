@@ -19,6 +19,7 @@
 #include "common.cuh"
 #include "rgbd_b200.h"
 #include "tc_ptx.cuh"
+#include "tma_host.cuh"
 
 namespace {
 
@@ -408,66 +409,6 @@ ratio_front_kernel(const __grid_constant__ CUtensorMap tmap_r, const __grid_cons
     }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn encode_fn() {
-    static EncodeTiledFn fn = nullptr;
-    if (!fn) {
-        void* ptr = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &qres) == cudaSuccess &&
-            qres == cudaDriverEntryPointSuccess)
-            fn = (EncodeTiledFn)ptr;
-    }
-    return fn;
-}
-
-bool make_nhwc_map(EncodeTiledFn enc, CUtensorMap* m, const void* base, int c, int w, int h, int n, int bx, int by) {
-    cuuint64_t dims[4] = {(cuuint64_t)c, (cuuint64_t)w, (cuuint64_t)h, (cuuint64_t)n};
-    cuuint64_t strides[3] = {(cuuint64_t)c * 2, (cuuint64_t)c * 2 * w, (cuuint64_t)c * 2 * w * h};
-    cuuint32_t box[4] = {64, (cuuint32_t)bx, (cuuint32_t)by, 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(base), dims, strides, box, estr,
-               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
-// (n, k) bf16 weight matrix, box = 64 K elements x n/2 rows (one CTA's half)
-bool make_weight_half_map(EncodeTiledFn enc, CUtensorMap* m, const void* base, int k, int n) {
-    cuuint64_t dims[2] = {(cuuint64_t)k, (cuuint64_t)n};
-    cuuint64_t strides[1] = {(cuuint64_t)k * 2};
-    cuuint32_t box[2] = {64, (cuuint32_t)(n / 2)};
-    cuuint32_t estr[2] = {1, 1};
-    return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
-               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
-// pixel-pair view: dims (inner, pairs, rows, images) with a 2-pixel stride in dimension 1 (overlapping when the inner
-// extent exceeds it: the sliding window over x)
-bool make_pair_map(EncodeTiledFn enc, CUtensorMap* m, const void* base, int inner_elems, int pixel_bytes, long long row_bytes,
-                   long long img_bytes, int pairs, int rows, int n, int box_inner, CUtensorMapSwizzle swz) {
-    cuuint64_t dims[4] = {(cuuint64_t)inner_elems, (cuuint64_t)pairs, (cuuint64_t)rows, (cuuint64_t)n};
-    cuuint64_t strides[3] = {(cuuint64_t)(2 * pixel_bytes), (cuuint64_t)row_bytes, (cuuint64_t)img_bytes};
-    cuuint32_t box[4] = {(cuuint32_t)box_inner, 64, 1, 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(base), dims, strides, box, estr,
-               CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
-bool make_weight_half_map64(EncodeTiledFn enc, CUtensorMap* m, const void* base, int k, int n) {   // 32-element K blocks, SW64
-    cuuint64_t dims[2] = {(cuuint64_t)k, (cuuint64_t)n};
-    cuuint64_t strides[1] = {(cuuint64_t)k * 2};
-    cuuint32_t box[2] = {32, (cuuint32_t)(n / 2)};
-    cuuint32_t estr[2] = {1, 1};
-    return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
-               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
 template <bool EM>
 int launch_front(const CUtensorMap& m_r, const CUtensorMap& m_r1, const CUtensorMap& m_w1, const CUtensorMap& m_w2,
                  const CUtensorMap& m_w3, const CUtensorMap& m_w4, const CUtensorMap& m_out, const CUtensorMap& m_out1,
@@ -484,18 +425,8 @@ int launch_front(const CUtensorMap& m_r, const CUtensorMap& m_r1, const CUtensor
     const int n_units = (p.total_tiles + 1) / 2;
     int clusters = num_sms / 2;
     if (clusters > n_units) clusters = n_units;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(2 * clusters);
-    cfg.blockDim = dim3(kThreads);
-    cfg.dynamicSmemBytes = smem_bytes;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    RGBD_CHECK_CUDA(cudaLaunchKernelEx(&cfg, ratio_front_kernel<EM>, m_r, m_r1, m_w1, m_w2, m_w3, m_w4, m_out, m_out1, p));
-    return RGBD_OK;
+    return launch_kernel(ratio_front_kernel<EM>, 2 * clusters, kThreads, smem_bytes, true, stream, m_r, m_r1, m_w1, m_w2, m_w3,
+                         m_w4, m_out, m_out1, p);
 }
 
 }  // namespace
@@ -509,35 +440,36 @@ extern "C" int rgbd_ratio_front(const void* r_bf16, const void* w1_bf16, const v
     RGBD_CHECK_ARG(bx >= 1 && by >= 1 && bx * by == kBlockM && bx <= 256 && by <= 256, "ratio_front: box must cover 128 pixels");
     if (compact_operand)
         RGBD_CHECK_ARG(bx == kBlockM && by == 1 && W % 2 == 0, "ratio_front: the compact operand needs a 128x1 box and an even width");
-    EncodeTiledFn enc = encode_fn();
-    if (!enc) {
-        rgbd_set_error("ratio_front: cuTensorMapEncodeTiled is not available from the driver");
-        return RGBD_ERR_CUDA;
-    }
+    const char* who = "ratio_front";
+    const CUtensorMapSwizzle sw64 = CU_TENSOR_MAP_SWIZZLE_64B, sw128 = CU_TENSOR_MAP_SWIZZLE_128B;
     CUtensorMap m_r, m_r1, m_w1, m_w2, m_w3, m_w4, m_out, m_out1;
-    bool ok = make_weight_half_map(enc, &m_w2, w2_bf16, 192, 128) && make_weight_half_map(enc, &m_w3, w3_bf16, 128, 64) &&
-              make_weight_half_map(enc, &m_w4, w4_bf16, 64, 128);
+    // (n, k) weight matrices: boxes of 64 K elements x n/2 rows (one CTA's half)
+    if (int rc = encode_bf16_map(&m_w2, who, w2_bf16, {192, 128}, {192 * 2}, {64, 64}, sw128)) return rc;
+    if (int rc = encode_bf16_map(&m_w3, who, w3_bf16, {128, 64}, {128 * 2}, {64, 32}, sw128)) return rc;
+    if (int rc = encode_bf16_map(&m_w4, who, w4_bf16, {64, 128}, {64 * 2}, {64, 64}, sw128)) return rc;
     if (compact_operand) {
+        // pixel-pair views: dims (inner, pairs, rows, images) with a 2-pixel stride in dimension 1 (overlapping when the inner
+        // extent exceeds it: the sliding window over x)
         const int Wp = rgbd_ratio_stem_compact_width(W);
         const long long row_bytes = (long long)Wp * 8, plane = (long long)(H + 6) * row_bytes;
         const uint8_t* e = reinterpret_cast<const uint8_t*>(r_bf16);
-        ok = ok && make_pair_map(enc, &m_r, e, 32, 8, row_bytes, 2 * plane, W / 2, H + 6, B, 32, CU_TENSOR_MAP_SWIZZLE_64B) &&
-             make_pair_map(enc, &m_r1, e + plane, 32, 8, row_bytes, 2 * plane, W / 2, H + 6, B, 32, CU_TENSOR_MAP_SWIZZLE_64B) &&
-             make_weight_half_map64(enc, &m_w1, w1_bf16, 224, 192);
+        if (int rc = encode_bf16_map(&m_r, who, e, {32, W / 2, H + 6, B}, {16, row_bytes, 2 * plane}, {32, 64, 1, 1}, sw64)) return rc;
+        if (int rc = encode_bf16_map(&m_r1, who, e + plane, {32, W / 2, H + 6, B}, {16, row_bytes, 2 * plane}, {32, 64, 1, 1}, sw64))
+            return rc;
+        if (int rc = encode_bf16_map(&m_w1, who, w1_bf16, {224, 192}, {224 * 2}, {32, 96}, sw64)) return rc;   // 32-element K blocks
         uint8_t* o = reinterpret_cast<uint8_t*>(out_bf16);
-        ok = ok && make_pair_map(enc, &m_out, o, 128, 256, (long long)W * 256, (long long)H * W * 256, W / 2, H, B, 64,
-                                 CU_TENSOR_MAP_SWIZZLE_128B) &&
-             make_pair_map(enc, &m_out1, o + 256, 128, 256, (long long)W * 256, (long long)H * W * 256, W / 2, H, B, 64,
-                           CU_TENSOR_MAP_SWIZZLE_128B);
+        const long long o_row = (long long)W * 256, o_img = (long long)H * W * 256;
+        if (int rc = encode_bf16_map(&m_out, who, o, {128, W / 2, H, B}, {512, o_row, o_img}, {64, 64, 1, 1}, sw128)) return rc;
+        if (int rc = encode_bf16_map(&m_out1, who, o + 256, {128, W / 2, H, B}, {512, o_row, o_img}, {64, 64, 1, 1}, sw128)) return rc;
     } else {
-        ok = ok && make_nhwc_map(enc, &m_r, r_bf16, 64, W, H + 6, B, bx, by) && make_nhwc_map(enc, &m_out, out_bf16, 128, W, H, B, bx, by) &&
-             make_weight_half_map(enc, &m_w1, w1_bf16, 256, 192);
+        const long long r_row = 64 * 2 * (long long)W, o_row = 128 * 2 * (long long)W;
+        if (int rc = encode_bf16_map(&m_r, who, r_bf16, {64, W, H + 6, B}, {64 * 2, r_row, r_row * (H + 6)}, {64, bx, by, 1}, sw128))
+            return rc;
+        if (int rc = encode_bf16_map(&m_out, who, out_bf16, {128, W, H, B}, {128 * 2, o_row, o_row * H}, {64, bx, by, 1}, sw128))
+            return rc;
+        if (int rc = encode_bf16_map(&m_w1, who, w1_bf16, {256, 192}, {256 * 2}, {64, 96}, sw128)) return rc;
         m_r1 = m_r;
         m_out1 = m_out;
-    }
-    if (!ok) {
-        rgbd_set_error("ratio_front: cuTensorMapEncodeTiled failed");
-        return RGBD_ERR_CUDA;
     }
     FrontParams p;
     p.n_img = B; p.BX = bx; p.BY = by;

@@ -9,7 +9,6 @@
 // work, bound by the FMA issue rate, not by memory.
 #include "common.cuh"
 #include "rgbd_b200.h"
-#include <stdlib.h>
 
 namespace {
 
@@ -39,8 +38,7 @@ __global__ void __launch_bounds__(256) window_attention_table_kernel(const float
     add[i] = x;
 }
 
-template <typename T> struct Ld;
-template <> struct Ld<float> {
+struct Ld {
     static __device__ __forceinline__ void row(const float* p, float (&x)[kHd]) {
 #pragma unroll
         for (int i = 0; i < kHd / 4; ++i) {
@@ -54,40 +52,11 @@ template <> struct Ld<float> {
         for (int i = 0; i < kHd / 4; ++i) reinterpret_cast<float4*>(p)[i] = make_float4(x[4 * i], x[4 * i + 1], x[4 * i + 2], x[4 * i + 3]);
     }
 };
-template <> struct Ld<__nv_bfloat16> {
-    static __device__ __forceinline__ void row(const __nv_bfloat16* p, float (&x)[kHd]) {
-#pragma unroll
-        for (int i = 0; i < kHd / 8; ++i) {
-            const uint4 v = __ldg(reinterpret_cast<const uint4*>(p) + i);
-            const uint32_t u[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-                x[8 * i + 2 * e] = __uint_as_float(u[e] << 16);
-                x[8 * i + 2 * e + 1] = __uint_as_float(u[e] & 0xffff0000u);
-            }
-        }
-    }
-    static __device__ __forceinline__ float one(const __nv_bfloat16* p) { return __bfloat162float(*p); }
-    static __device__ __forceinline__ void store(__nv_bfloat16* p, const float (&x)[kHd]) {
-#pragma unroll
-        for (int i = 0; i < kHd / 8; ++i) {
-            uint4 v;
-            uint32_t* u = reinterpret_cast<uint32_t*>(&v);
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-                const __nv_bfloat162 t = __floats2bfloat162_rn(x[8 * i + 2 * e], x[8 * i + 2 * e + 1]);
-                u[e] = *reinterpret_cast<const uint32_t*>(&t);
-            }
-            reinterpret_cast<uint4*>(p)[i] = v;
-        }
-    }
-};
 
-template <typename T>
-__global__ void __launch_bounds__(kWarps * 32) window_attention_kernel(const T* __restrict__ q, const T* __restrict__ k,
-                                                                     const T* __restrict__ v, const float* __restrict__ add,
-                                                                     T* __restrict__ out, long long n_units, int heads, int N, int nW,
-                                                                     float sqrt_d) {
+__global__ void __launch_bounds__(kWarps * 32) window_attention_kernel(const float* __restrict__ q, const float* __restrict__ k,
+                                                                     const float* __restrict__ v, const float* __restrict__ add,
+                                                                     float* __restrict__ out, long long n_units, int heads, int N,
+                                                                     int nW, float sqrt_d) {
     extern __shared__ float s_kv[];                          // per warp: K [N][32], V [N][32] as fp32
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const long long unit = (long long)blockIdx.x * kWarps + warp;
@@ -97,18 +66,18 @@ __global__ void __launch_bounds__(kWarps * 32) window_attention_kernel(const T* 
     const int C = heads * kHd;
     float* sk = s_kv + (size_t)warp * 2 * N * kHd;
     float* sv = sk + N * kHd;
-    const T* kb = k + (size_t)win * N * C + h * kHd;
-    const T* vb = v + (size_t)win * N * C + h * kHd;
+    const float* kb = k + (size_t)win * N * C + h * kHd;
+    const float* vb = v + (size_t)win * N * C + h * kHd;
     for (int i = lane; i < N * kHd; i += 32) {
         const int j = i >> 5, d = i & 31;
-        sk[i] = Ld<T>::one(kb + (size_t)j * C + d);
-        sv[i] = Ld<T>::one(vb + (size_t)j * C + d);
+        sk[i] = Ld::one(kb + (size_t)j * C + d);
+        sv[i] = Ld::one(vb + (size_t)j * C + d);
     }
     __syncwarp();
     const float* add_wh = add + ((size_t)(win % nW) * heads + h) * N * kTabPitch;
     for (int r = lane; r < N; r += 32) {
         float qv[kHd], o[kHd];
-        Ld<T>::row(q + ((size_t)win * N + r) * C + h * kHd, qv);
+        Ld::row(q + ((size_t)win * N + r) * C + h * kHd, qv);
 #pragma unroll
         for (int d = 0; d < kHd; ++d) o[d] = 0.f;
         float m = -INFINITY, l = 0.f;
@@ -163,7 +132,7 @@ __global__ void __launch_bounds__(kWarps * 32) window_attention_kernel(const T* 
         const float inv = 1.0f / l;
 #pragma unroll
         for (int d = 0; d < kHd; ++d) o[d] *= inv;
-        Ld<T>::store(out + ((size_t)win * N + r) * C + h * kHd, o);
+        Ld::store(out + ((size_t)win * N + r) * C + h * kHd, o);
     }
 }
 
@@ -524,9 +493,7 @@ extern "C" int rgbd_window_attention(const void* q, const void* k, const void* v
     RgbdDeviceInfo di;
     if (int rc = rgbd_device_info(&di)) return rc;
     RGBD_ONCE_PER_DEVICE(di.device, {
-        RGBD_CHECK_CUDA(cudaFuncSetAttribute(window_attention_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             kWarps * 2 * kMaxN * kHd * (int)sizeof(float)));
-        RGBD_CHECK_CUDA(cudaFuncSetAttribute(window_attention_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        RGBD_CHECK_CUDA(cudaFuncSetAttribute(window_attention_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                              kWarps * 2 * kMaxN * kHd * (int)sizeof(float)));
     });
     cudaStream_t s = (cudaStream_t)stream;
@@ -535,14 +502,11 @@ extern "C" int rgbd_window_attention(const void* q, const void* k, const void* v
     window_attention_table_kernel<<<(unsigned)((n_tab + 255) / 256), 256, 0, s>>>(bias, mask, add, nW, heads, N);
     RGBD_CHECK_LAUNCH();
     const float sqrt_d = sqrtf((float)head_dim);
-    if (dtype == RGBD_DTYPE_BF16 && !getenv("RGBD_WINATTN_CUDA_CORES"))
+    if (dtype == RGBD_DTYPE_BF16)
         window_attention_mma_kernel<<<(unsigned)blocks, kWarps * 32, 0, s>>>(
             (const __nv_bfloat16*)q, (const __nv_bfloat16*)k, (const __nv_bfloat16*)v, add, (__nv_bfloat16*)out, n_units, heads, N, nW, sqrt_d);
-    else if (dtype == RGBD_DTYPE_BF16)
-        window_attention_kernel<__nv_bfloat16><<<(unsigned)blocks, kWarps * 32, smem, s>>>(
-            (const __nv_bfloat16*)q, (const __nv_bfloat16*)k, (const __nv_bfloat16*)v, add, (__nv_bfloat16*)out, n_units, heads, N, nW, sqrt_d);
     else
-        window_attention_kernel<float><<<(unsigned)blocks, kWarps * 32, smem, s>>>((const float*)q, (const float*)k, (const float*)v, add,
+        window_attention_kernel<<<(unsigned)blocks, kWarps * 32, smem, s>>>((const float*)q, (const float*)k, (const float*)v, add,
                                                                                   (float*)out, n_units, heads, N, nW, sqrt_d);
     RGBD_CHECK_LAUNCH();
     return RGBD_OK;
