@@ -181,13 +181,20 @@ int rgbd_conv_gemm(const rgbd_conv_gemm_desc* desc_host, rgbd_stream_t stream);
  * rgbd_dsam_dbias: db[t][n] = sum over images that use region t (t < variant[b]) of sum_pixels g[b][n]; db overwritten.
  * rgbd_dsam_wgrad: dw[n][seg][tap][C_pad] (fp32, overwritten) = sum_pixels g[b][n][oy][ox] * x_t[b][seg][tap-shifted pixel][c];
  *   g_bf16: (B, N_out, Ho, g_w_pitch); xt_bf16: output of rgbd_dsam_pack_t with plane height x_h and the SAME row pitch.
- * The input gradient runs through rgbd_conv_gemm with epi_mode 3. */
-int rgbd_cast_bf16_pitched(const float* src, void* dst_bf16, long long rows, int W, int W_pitch, rgbd_stream_t stream);
-int rgbd_dsam_pack_t(const float* feat, const uint8_t* codes, void* out_bf16, int B, int C, int C_pad, int H, int W,
-                     int W2_pitch, int n_seg, int masked_segs, int parity_split, rgbd_stream_t stream);
+ * Split precision (DSAModule.grad_precision "fp32"): dst_lo / out_lo, when not NULL, receive the lo parts
+ *   bf16(v - float(bf16(v))) in the layout of the hi output (pitch and pad zero, masked pixels +0); rgbd_dsam_wgrad given
+ *   both g_lo and xt_lo accumulates G_hi.X_hi + G_lo.X_hi + G_hi.X_lo (~2^-16 relative instead of ~2^-8); NULL lo
+ *   pointers select the bf16 operands alone.
+ * The input gradient runs through rgbd_conv_gemm with epi_mode 3 (split precision: G packed by rgbd_dsam_pack with
+ * hi_lo = 1, weights [W_hi | W_hi | W_lo] per K block). */
+int rgbd_cast_bf16_pitched(const float* src, void* dst_bf16, void* dst_lo, long long rows, int W, int W_pitch,
+                           rgbd_stream_t stream);
+int rgbd_dsam_pack_t(const float* feat, const uint8_t* codes, void* out_bf16, void* out_lo, int B, int C, int C_pad, int H,
+                     int W, int W2_pitch, int n_seg, int masked_segs, int parity_split, rgbd_stream_t stream);
 int rgbd_dsam_dbias(const float* g, const int* variant, float* db, int B, int N, int HW, int n_bias, rgbd_stream_t stream);
-int rgbd_dsam_wgrad(const void* g_bf16, int g_w_pitch, const void* xt_bf16, int x_w_pitch, int x_h, float* dw, int B,
-                    int N_out, int C_pad, int Ho, int Wo, int n_seg, int parity_split, rgbd_stream_t stream);
+int rgbd_dsam_wgrad(const void* g_bf16, const void* g_lo, int g_w_pitch, const void* xt_bf16, const void* xt_lo, int x_w_pitch,
+                    int x_h, float* dw, int B, int N_out, int C_pad, int Ho, int Wo, int n_seg, int parity_split,
+                    rgbd_stream_t stream);
 
 /* Fused point-wise middle of EnhancedDepthImageRatioPredictor.forward (CM:1466-1470): feature_fusion (1x1 192->128 +
  * folded BN + ReLU), attention (1x1 128->64 + ReLU, 1x1 64->128 + sigmoid) and the gating multiply, as three chained

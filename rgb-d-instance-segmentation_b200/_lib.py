@@ -65,12 +65,12 @@ SIGNATURES = {
     "rgbd_ratio_stem_pack": (C.c_int, [C.c_void_p, C.c_longlong, C.c_longlong, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
                                        C.c_void_p]),
     "rgbd_conv_gemm": (C.c_int, [C.POINTER(ConvGemmDesc), C.c_void_p]),
-    "rgbd_cast_bf16_pitched": (C.c_int, [C.c_void_p, C.c_void_p, C.c_longlong, C.c_int, C.c_int, C.c_void_p]),
-    "rgbd_dsam_pack_t": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
-                                   C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "rgbd_cast_bf16_pitched": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong, C.c_int, C.c_int, C.c_void_p]),
+    "rgbd_dsam_pack_t": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
+                                   C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "rgbd_dsam_dbias": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
-    "rgbd_dsam_wgrad": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int,
-                                  C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "rgbd_dsam_wgrad": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p,
+                                  C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "rgbd_ratio_chain": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                    C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "rgbd_ratio_front": (C.c_int, [C.c_void_p] * 10 + [C.c_int] * 6 + [C.c_void_p]),

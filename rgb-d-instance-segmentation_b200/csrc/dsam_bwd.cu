@@ -12,6 +12,11 @@
 // (= conv padding; the pitch padding of G is zero, so pad columns never contribute).  One CTA tile = (segment, tap, 128 output channels, BLOCK_N input
 // channels, image range); tcgen05.mma accumulates in TMEM over the whole K loop; the epilogue adds the fp32 tile
 // into dW with red.global (split-K over images keeps all SMs busy).
+//
+// Split-precision mode (hi_lo, DSAModule.grad_precision == "fp32"): both operands also come as bf16 lo parts
+// lo = bf16(v - float(bf16(v))).  A pipeline stage then holds four boxes under one mbarrier -- G_hi, G_lo, X_hi, X_lo --
+// and the MMA warp issues G_hi.X_hi + G_lo.X_hi + G_hi.X_lo into the same TMEM accumulator, so every hi tile is loaded
+// once per K block.  The three products leave out lo.lo and the rounding of lo, each at most 2^-16 |g||x|.
 #include "common.cuh"
 #include "rgbd_b200.h"
 #include "tc_ptx.cuh"
@@ -29,6 +34,7 @@ struct WgradParams {
     int n_seg, n_par, taps;
     int m_tiles, n_tiles, BLOCK_N, ksplit;
     int N_out, Cp, stages;
+    int hi_lo;                         // 1: split-precision operands (G_lo, X_lo boxes after G_hi, X_hi in every stage)
     int taps_tbl[9][2];                // (plane, flattened pixel offset) per tap
     float* dw;                         // [N_out][n_seg][taps][Cp]
     int total_tiles;
@@ -53,15 +59,23 @@ __device__ __forceinline__ void decode_wtile(const WgradParams& p, int t, int& k
 
 __global__ void __launch_bounds__(kThreads, 1)
 dsam_wgrad_kernel(const __grid_constant__ CUtensorMap tmap_g, const __grid_constant__ CUtensorMap tmap_x,
+                  const __grid_constant__ CUtensorMap tmap_g_lo, const __grid_constant__ CUtensorMap tmap_x_lo,
                   const __grid_constant__ WgradParams p) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     uint8_t* smem = smem_raw + ((1024u - (tc::smem_u32(smem_raw) & 1023u)) & 1023u);
-    const int a_bytes = kBlockM * 128, b_bytes = p.BLOCK_N * 128, stage_bytes = a_bytes + b_bytes;
+    // stage layout: [G_hi | G_lo | X_hi | X_lo] in split mode, [G | X] otherwise (every box a multiple of 4 KB, so each
+    // stays 1024-byte aligned for the 128-byte swizzle)
+    const int n_op = p.hi_lo ? 2 : 1;
+    const int a_bytes = kBlockM * 128, b_bytes = p.BLOCK_N * 128, x_off = n_op * a_bytes, stage_bytes = n_op * (a_bytes + b_bytes);
     WCtl* ctl = reinterpret_cast<WCtl*>(smem + (size_t)p.stages * stage_bytes);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     if (warp == 0 && lane == 0) {
         tc::prefetch_tmap(&tmap_g);
         tc::prefetch_tmap(&tmap_x);
+        if (p.hi_lo) {
+            tc::prefetch_tmap(&tmap_g_lo);
+            tc::prefetch_tmap(&tmap_x_lo);
+        }
         for (int s = 0; s < p.stages; ++s) {
             tc::mbar_init(&ctl->full[s], 1);
             tc::mbar_init(&ctl->empty[s], 1);
@@ -91,7 +105,11 @@ dsam_wgrad_kernel(const __grid_constant__ CUtensorMap tmap_g, const __grid_const
                     uint8_t* sa = smem + (size_t)stage * stage_bytes;
                     tc::mbar_expect_tx(&ctl->full[stage], (uint32_t)stage_bytes);
                     tc::tma_load_3d(sa, &tmap_g, &ctl->full[stage], kb * 64, mt * kBlockM, b);
-                    tc::tma_load_3d(sa + a_bytes, &tmap_x, &ctl->full[stage], kb * 64 + off, nt * p.BLOCK_N, plane);
+                    tc::tma_load_3d(sa + x_off, &tmap_x, &ctl->full[stage], kb * 64 + off, nt * p.BLOCK_N, plane);
+                    if (p.hi_lo) {
+                        tc::tma_load_3d(sa + a_bytes, &tmap_g_lo, &ctl->full[stage], kb * 64, mt * kBlockM, b);
+                        tc::tma_load_3d(sa + x_off + b_bytes, &tmap_x_lo, &ctl->full[stage], kb * 64 + off, nt * p.BLOCK_N, plane);
+                    }
                     if (++stage == p.stages) { stage = 0; phase ^= 1; }
                 }
             }
@@ -112,11 +130,22 @@ dsam_wgrad_kernel(const __grid_constant__ CUtensorMap tmap_g, const __grid_const
                 tc::mbar_wait(&ctl->full[stage], phase);
                 tc::tc_fence_after();
                 const uint32_t sa = tc::smem_u32(smem + (size_t)stage * stage_bytes);
-                const uint64_t adesc = tc::make_kmajor_desc(sa, 128), bdesc = tc::make_kmajor_desc(sa + a_bytes, 128);
+                const uint64_t adesc = tc::make_kmajor_desc(sa, 128), bdesc = tc::make_kmajor_desc(sa + x_off, 128);
                 if (tc::elect_one()) {
 #pragma unroll
                     for (int k = 0; k < 4; ++k)
                         tc::umma_bf16(tmem, adesc + (uint64_t)(k * 2), bdesc + (uint64_t)(k * 2), idesc, (j | k) != 0);
+                    if (p.hi_lo) {
+                        // G_lo . X_hi, then G_hi . X_lo, into the same accumulator
+                        const uint64_t adesc_lo = tc::make_kmajor_desc(sa + a_bytes, 128);
+                        const uint64_t bdesc_lo = tc::make_kmajor_desc(sa + x_off + b_bytes, 128);
+#pragma unroll
+                        for (int k = 0; k < 4; ++k)
+                            tc::umma_bf16(tmem, adesc_lo + (uint64_t)(k * 2), bdesc + (uint64_t)(k * 2), idesc, 1u);
+#pragma unroll
+                        for (int k = 0; k < 4; ++k)
+                            tc::umma_bf16(tmem, adesc + (uint64_t)(k * 2), bdesc_lo + (uint64_t)(k * 2), idesc, 1u);
+                    }
                     tc::umma_commit(&ctl->empty[stage]);
                 }
                 __syncwarp();
@@ -162,39 +191,53 @@ dsam_wgrad_kernel(const __grid_constant__ CUtensorMap tmap_g, const __grid_const
 }
 
 // ---- operand staging ---------------------------------------------------------------------------------------
-// G (B,N,Ho,Wo) fp32 -> bf16 with the row pitch padded to a multiple of 8 pixels (TMA strides are 16-byte units)
+// G (B,N,Ho,Wo) fp32 -> bf16 with the row pitch padded to a multiple of 8 pixels (TMA strides are 16-byte units).
+// dst_lo (optional): the lo part bf16(v - float(bf16(v))) in the same layout (split-precision weight gradient).
 __global__ void __launch_bounds__(256) cast_pitched_kernel(const float* __restrict__ src, __nv_bfloat16* __restrict__ dst,
-                                                           long long rows, int W, int Wp) {
+                                                           __nv_bfloat16* __restrict__ dst_lo, long long rows, int W, int Wp) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const long long total = rows * Wp;
     if (i >= total) return;
     const long long r = i / Wp;
     const int x = (int)(i - r * Wp);
-    dst[i] = __float2bfloat16(x < W ? src[r * W + x] : 0.f);
+    const float v = x < W ? src[r * W + x] : 0.f;
+    const __nv_bfloat16 h = __float2bfloat16(v);
+    dst[i] = h;
+    if (dst_lo) dst_lo[i] = __float2bfloat16(v - __bfloat162float(h));
 }
 
 // masked, parity-split, pixel-contiguous input: out[b][seg][par][c][y2][x2 (pitch W2p)] = bf16(F[b][c][y][x] * bit(code,seg)).
 // TMA needs the innermost (x) start coordinate 16-byte aligned, so the x-1 tap cannot be a box shifted by one pixel:
 // planes 4 and 5 are copies of the px=1 planes (py=0 / py=1) shifted right by one pixel (x2 -> x2+1).
+// out_lo (optional): the lo parts bf16(v - float(bf16(v))) in the identical layout; masked-out pixels are +0 in both.
 __global__ void __launch_bounds__(256) dsam_pack_t_kernel(const float* __restrict__ feat, const uint8_t* __restrict__ codes,
-                                                          __nv_bfloat16* __restrict__ out, int C, int Cp, int H, int W,
-                                                          int H2, int W2p, int n_seg, int masked_segs, int split) {
+                                                          __nv_bfloat16* __restrict__ out, __nv_bfloat16* __restrict__ out_lo,
+                                                          int C, int Cp, int H, int W, int H2, int W2p, int n_seg,
+                                                          int masked_segs, int split) {
     const int b = blockIdx.z, c = blockIdx.y;
     const int n_par = split ? 6 : 1;
     const size_t plane = (size_t)H * W;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < H * W; i += gridDim.x * blockDim.x) {
         const int y = i / W, x = i - y * W;
         const float v = feat[((size_t)b * C + c) * plane + i];
+        const __nv_bfloat16 vh = __float2bfloat16(v);
+        const __nv_bfloat16 vl = __float2bfloat16(v - __bfloat162float(vh));
+        const __nv_bfloat16 zero = __float2bfloat16(0.f);
         const unsigned code = codes[(size_t)b * plane + i];
         const int par = split ? ((y & 1) * 2 + (x & 1)) : 0;
         const int yy = split ? (y >> 1) : y, xx = split ? (x >> 1) : x;
         for (int s = 0; s < n_seg; ++s) {
             const bool keep = s >= masked_segs || ((code >> s) & 1u);
-            const __nv_bfloat16 h = __float2bfloat16(keep ? v : 0.f);
+            const __nv_bfloat16 h = keep ? vh : zero, l = keep ? vl : zero;
             const size_t pl = ((size_t)b * n_seg + s) * n_par;
-            out[(((pl + par) * Cp + c) * H2 + yy) * W2p + xx] = h;
-            if (split && (x & 1) && xx + 1 < W2p)
-                out[(((pl + 4 + (y & 1)) * Cp + c) * H2 + yy) * W2p + xx + 1] = h;
+            const size_t o = (((pl + par) * Cp + c) * H2 + yy) * W2p + xx;
+            out[o] = h;
+            if (out_lo) out_lo[o] = l;
+            if (split && (x & 1) && xx + 1 < W2p) {
+                const size_t o2 = (((pl + 4 + (y & 1)) * Cp + c) * H2 + yy) * W2p + xx + 1;
+                out[o2] = h;
+                if (out_lo) out_lo[o2] = l;
+            }
         }
     }
 }
@@ -221,25 +264,25 @@ __global__ void __launch_bounds__(256) dsam_dbias_kernel(const float* __restrict
 
 }  // namespace
 
-extern "C" int rgbd_cast_bf16_pitched(const float* src, void* dst_bf16, long long rows, int W, int W_pitch,
+extern "C" int rgbd_cast_bf16_pitched(const float* src, void* dst_bf16, void* dst_lo, long long rows, int W, int W_pitch,
                                       rgbd_stream_t stream) {
     RGBD_CHECK_ARG(src && dst_bf16 && rows >= 1 && W >= 1 && W_pitch >= W && W_pitch % 8 == 0, "cast_bf16_pitched: bad arguments");
     const long long total = rows * W_pitch;
-    cast_pitched_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(src, (__nv_bfloat16*)dst_bf16, rows, W,
-                                                                                         W_pitch);
+    cast_pitched_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(src, (__nv_bfloat16*)dst_bf16,
+                                                                                         (__nv_bfloat16*)dst_lo, rows, W, W_pitch);
     RGBD_CHECK_LAUNCH();
     return RGBD_OK;
 }
 
-extern "C" int rgbd_dsam_pack_t(const float* feat, const uint8_t* codes, void* out_bf16, int B, int C, int C_pad, int H, int W,
-                                int W2_pitch, int n_seg, int masked_segs, int parity_split, rgbd_stream_t stream) {
+extern "C" int rgbd_dsam_pack_t(const float* feat, const uint8_t* codes, void* out_bf16, void* out_lo, int B, int C, int C_pad,
+                                int H, int W, int W2_pitch, int n_seg, int masked_segs, int parity_split, rgbd_stream_t stream) {
     RGBD_CHECK_ARG(feat && codes && out_bf16, "dsam_pack_t: null pointer");
     RGBD_CHECK_ARG(B >= 1 && C >= 1 && C_pad >= C && H >= 1 && W >= 1 && W2_pitch % 8 == 0, "dsam_pack_t: bad geometry");
     const int H2 = parity_split ? (H + 1) / 2 : H;
     RGBD_CHECK_ARG(W2_pitch >= (parity_split ? (W + 1) / 2 : W), "dsam_pack_t: pitch too small");
     dim3 grid(min(ceil_div(H * W, 256), 64), C, B);
-    dsam_pack_t_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(feat, codes, (__nv_bfloat16*)out_bf16, C, C_pad, H, W, H2,
-                                                              W2_pitch, n_seg, masked_segs, parity_split ? 1 : 0);
+    dsam_pack_t_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(feat, codes, (__nv_bfloat16*)out_bf16, (__nv_bfloat16*)out_lo, C,
+                                                              C_pad, H, W, H2, W2_pitch, n_seg, masked_segs, parity_split ? 1 : 0);
     RGBD_CHECK_LAUNCH();
     return RGBD_OK;
 }
@@ -253,16 +296,18 @@ extern "C" int rgbd_dsam_dbias(const float* g, const int* variant, float* db, in
     return RGBD_OK;
 }
 
-extern "C" int rgbd_dsam_wgrad(const void* g_bf16, int g_w_pitch, const void* xt_bf16, int x_w_pitch, int x_h, float* dw,
-                               int B, int N_out, int C_pad, int Ho, int Wo, int n_seg, int parity_split,
-                               rgbd_stream_t stream) {
+extern "C" int rgbd_dsam_wgrad(const void* g_bf16, const void* g_lo, int g_w_pitch, const void* xt_bf16, const void* xt_lo,
+                               int x_w_pitch, int x_h, float* dw, int B, int N_out, int C_pad, int Ho, int Wo, int n_seg,
+                               int parity_split, rgbd_stream_t stream) {
     RGBD_CHECK_ARG(g_bf16 && xt_bf16 && dw, "dsam_wgrad: null pointer");
+    RGBD_CHECK_ARG((g_lo == nullptr) == (xt_lo == nullptr), "dsam_wgrad: give both lo parts (split precision) or neither");
     RGBD_CHECK_ARG(B >= 1 && N_out >= 1 && C_pad >= 32 && C_pad % 32 == 0 && Ho >= 1 && Wo >= 1 && n_seg >= 1 && n_seg <= 8,
                    "dsam_wgrad: bad geometry");
     RGBD_CHECK_ARG(g_w_pitch % 8 == 0 && x_w_pitch % 8 == 0 && g_w_pitch >= Wo, "dsam_wgrad: row pitches must be multiples of 8");
     WgradParams p;
     p.B = B; p.Ho = Ho; p.Wo = Wo; p.N_out = N_out; p.Cp = C_pad;
     p.n_seg = n_seg;
+    p.hi_lo = g_lo ? 1 : 0;
     p.n_par = parity_split ? 6 : 1;
     p.taps = parity_split ? 9 : 1;
     RGBD_CHECK_ARG(g_w_pitch == x_w_pitch && x_h >= Ho, "dsam_wgrad: G and X^T must share the row pitch (got %d / %d)", g_w_pitch,
@@ -279,15 +324,21 @@ extern "C" int rgbd_dsam_wgrad(const void* g_bf16, int g_w_pitch, const void* xt
         }
         p.taps_tbl[tap][0] = par; p.taps_tbl[tap][1] = off;
     }
-    p.BLOCK_N = C_pad <= 256 ? C_pad : 0;
-    if (!p.BLOCK_N)
-        for (int bn = 256; bn >= 32; bn -= 32)
-            if (C_pad % bn == 0) { p.BLOCK_N = bn; break; }
-    p.n_tiles = C_pad / p.BLOCK_N;
-    p.m_tiles = ceil_div(N_out, kBlockM);
     RgbdDeviceInfo di;
     if (int rc = rgbd_device_info(&di)) return rc;
     const int num_sms = di.num_sms, max_smem = di.max_smem;
+    // BLOCK_N: the widest multiple of 32 (at most 256) that divides C_pad.  Split mode doubles the stage bytes; there the
+    // widest one that still leaves 3 pipeline stages (BLOCK_N 128 at 227 KB: 64 KB stages; 256 would leave 2).
+    const int n_op = p.hi_lo ? 2 : 1;
+    auto stages_for = [&](int bn) {
+        const int s = (max_smem - 2048 - (int)sizeof(WCtl)) / (n_op * (kBlockM * 128 + bn * 128));
+        return s < kMaxStagesW ? s : kMaxStagesW;
+    };
+    p.BLOCK_N = 32;
+    for (int bn = 256; bn > 32; bn -= 32)
+        if (C_pad % bn == 0 && (!p.hi_lo || stages_for(bn) >= 3)) { p.BLOCK_N = bn; break; }
+    p.n_tiles = C_pad / p.BLOCK_N;
+    p.m_tiles = ceil_div(N_out, kBlockM);
     RGBD_ONCE_PER_DEVICE(di.device, {
         RGBD_CHECK_CUDA(cudaFuncSetAttribute(dsam_wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
     });
@@ -297,25 +348,31 @@ extern "C" int rgbd_dsam_wgrad(const void* g_bf16, int g_w_pitch, const void* xt
     p.ksplit = ksplit;
     p.total_tiles = base_tiles * ksplit;
     p.dw = dw;
-    const int stage_bytes = kBlockM * 128 + p.BLOCK_N * 128;
-    int stages = (max_smem - 2048 - (int)sizeof(WCtl)) / stage_bytes;
-    if (stages > kMaxStagesW) stages = kMaxStagesW;
+    const int stage_bytes = n_op * (kBlockM * 128 + p.BLOCK_N * 128);
+    const int stages = stages_for(p.BLOCK_N);
     RGBD_CHECK_ARG(stages >= 2, "dsam_wgrad: not enough shared memory");
     p.stages = stages;
     // channel-major operands: (pixels, channels, planes), pixels innermost
-    CUtensorMap m_g, m_x;
+    // (the lo maps describe the same layout at the lo base pointers; the bf16 mode passes the hi maps again, unread)
+    CUtensorMap m_g, m_x, m_g_lo, m_x_lo;
     const long long g_pix = (long long)Ho * g_w_pitch, x_pix = (long long)x_h * x_w_pitch;
-    if (int rc = encode_bf16_map(&m_g, "dsam_wgrad", g_bf16, {g_pix, N_out, B}, {g_pix * 2, g_pix * 2 * N_out}, {64, kBlockM, 1},
-                                 CU_TENSOR_MAP_SWIZZLE_128B))
-        return rc;
-    if (int rc = encode_bf16_map(&m_x, "dsam_wgrad", xt_bf16, {x_pix, C_pad, B * n_seg * p.n_par},
-                                 {x_pix * 2, x_pix * 2 * C_pad}, {64, p.BLOCK_N, 1}, CU_TENSOR_MAP_SWIZZLE_128B))
-        return rc;
+    const void* g_ptrs[2] = {g_bf16, p.hi_lo ? g_lo : g_bf16};
+    const void* x_ptrs[2] = {xt_bf16, p.hi_lo ? xt_lo : xt_bf16};
+    CUtensorMap* g_maps[2] = {&m_g, &m_g_lo};
+    CUtensorMap* x_maps[2] = {&m_x, &m_x_lo};
+    for (int h = 0; h < 2; ++h) {
+        if (int rc = encode_bf16_map(g_maps[h], "dsam_wgrad", g_ptrs[h], {g_pix, N_out, B}, {g_pix * 2, g_pix * 2 * N_out},
+                                     {64, kBlockM, 1}, CU_TENSOR_MAP_SWIZZLE_128B))
+            return rc;
+        if (int rc = encode_bf16_map(x_maps[h], "dsam_wgrad", x_ptrs[h], {x_pix, C_pad, B * n_seg * p.n_par},
+                                     {x_pix * 2, x_pix * 2 * C_pad}, {64, p.BLOCK_N, 1}, CU_TENSOR_MAP_SWIZZLE_128B))
+            return rc;
+    }
     RGBD_CHECK_CUDA(cudaMemsetAsync(dw, 0, sizeof(float) * (size_t)N_out * n_seg * p.taps * C_pad, (cudaStream_t)stream));
     int smem_bytes = 1024 + stages * stage_bytes + (int)sizeof(WCtl) + 64;
     if (smem_bytes < 120 * 1024) smem_bytes = 120 * 1024;     // one CTA per SM (TMEM allocation)
     const int grid = p.total_tiles < num_sms ? p.total_tiles : num_sms;
-    dsam_wgrad_kernel<<<grid, kThreads, smem_bytes, (cudaStream_t)stream>>>(m_g, m_x, p);
+    dsam_wgrad_kernel<<<grid, kThreads, smem_bytes, (cudaStream_t)stream>>>(m_g, m_x, m_g_lo, m_x_lo, p);
     RGBD_CHECK_LAUNCH();
     return RGBD_OK;
 }

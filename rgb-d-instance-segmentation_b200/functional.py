@@ -509,26 +509,35 @@ def project_group_norm(x: torch.Tensor, conv_w: torch.Tensor, conv_b: Optional[t
     return out
 
 
-def cast_bf16_pitched(src: torch.Tensor, w_pitch: int) -> torch.Tensor:
-    """(..., W) fp32 -> (..., w_pitch) bf16, zero padded (TMA row strides must be multiples of 16 bytes)."""
+def cast_bf16_pitched(src: torch.Tensor, w_pitch: int, lo: bool = False):
+    """(..., W) fp32 -> (..., w_pitch) bf16, zero padded (TMA row strides must be multiples of 16 bytes).  With ``lo``
+    returns (hi, lo): hi = bf16(v) and lo = bf16(v - hi) in the same layout (split-precision operands)."""
     lib = _lib.load()
     _req(src, "src", torch.float32)
     W = src.shape[-1]
     rows = src.numel() // W
     out = torch.empty(*src.shape[:-1], w_pitch, device=src.device, dtype=torch.bfloat16)
-    check(lib.rgbd_cast_bf16_pitched(src.data_ptr(), out.data_ptr(), rows, W, w_pitch, _stream()), "rgbd_cast_bf16_pitched")
+    out_lo = torch.empty_like(out) if lo else None
+    check(lib.rgbd_cast_bf16_pitched(src.data_ptr(), out.data_ptr(), out_lo.data_ptr() if lo else None, rows, W, w_pitch,
+                                     _stream()), "rgbd_cast_bf16_pitched")
     _count(1)
-    return out
+    return (out, out_lo) if lo else out
 
 
 def dsam_pack_t(feat: torch.Tensor, codes: torch.Tensor, out: torch.Tensor, c_pad: int, w2_pitch: int, n_seg: int,
-                masked_segs: int, parity_split: bool) -> None:
+                masked_segs: int, parity_split: bool, out_lo: Optional[torch.Tensor] = None) -> None:
+    """``out_lo`` (same shape as ``out``, zeroed like it): also write the lo parts bf16(v - bf16(v))."""
     lib = _lib.load()
     _req(feat, "feat", torch.float32)
     _req(codes, "codes", torch.uint8)
     _req(out, "packed", torch.bfloat16)
+    if out_lo is not None:
+        _req(out_lo, "packed_lo", torch.bfloat16)
+        if out_lo.shape != out.shape:
+            raise RgbdB200Error(f"dsam_pack_t: out_lo must be {tuple(out.shape)}, got {tuple(out_lo.shape)}")
     B, Cc, H, W = feat.shape
-    check(lib.rgbd_dsam_pack_t(feat.data_ptr(), codes.data_ptr(), out.data_ptr(), B, Cc, c_pad, H, W, w2_pitch, n_seg,
+    check(lib.rgbd_dsam_pack_t(feat.data_ptr(), codes.data_ptr(), out.data_ptr(),
+                               out_lo.data_ptr() if out_lo is not None else None, B, Cc, c_pad, H, W, w2_pitch, n_seg,
                                masked_segs, 1 if parity_split else 0, _stream()), "rgbd_dsam_pack_t")
     _count(1)
 
@@ -545,16 +554,26 @@ def dsam_dbias(g: torch.Tensor, variant: Optional[torch.Tensor], n_bias: int) ->
 
 
 def dsam_wgrad(g_bf16: torch.Tensor, xt: torch.Tensor, n_out: int, c_pad: int, out_hw: Tuple[int, int], n_seg: int,
-               parity_split: bool) -> torch.Tensor:
-    """dW[n][seg][tap][c_pad] fp32.  g_bf16: (B, n_out, Ho, Wp); xt: (B, n_seg, n_par, c_pad, H2, W2p)."""
+               parity_split: bool, g_lo: Optional[torch.Tensor] = None, xt_lo: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """dW[n][seg][tap][c_pad] fp32.  g_bf16: (B, n_out, Ho, Wp); xt: (B, n_seg, n_par, c_pad, H2, W2p).  With both lo
+    parts (``cast_bf16_pitched(lo=True)``, ``dsam_pack_t(out_lo=...)``): split precision, g_hi.x_hi + g_lo.x_hi + g_hi.x_lo."""
     lib = _lib.load()
     _req(g_bf16, "g", torch.bfloat16)
     _req(xt, "x_t", torch.bfloat16)
+    if (g_lo is None) != (xt_lo is None):
+        raise RgbdB200Error("dsam_wgrad: give both lo parts (split precision) or neither")
+    if g_lo is not None:
+        _req(g_lo, "g_lo", torch.bfloat16)
+        _req(xt_lo, "x_t_lo", torch.bfloat16)
+        if g_lo.shape != g_bf16.shape or xt_lo.shape != xt.shape:
+            raise RgbdB200Error("dsam_wgrad: lo parts must have the shapes of the hi parts")
     B = g_bf16.shape[0]
     taps = 9 if parity_split else 1
     dw = torch.empty(n_out, n_seg, taps, c_pad, device=g_bf16.device, dtype=torch.float32)
-    check(lib.rgbd_dsam_wgrad(g_bf16.data_ptr(), g_bf16.shape[-1], xt.data_ptr(), xt.shape[-1], xt.shape[-2], dw.data_ptr(), B,
-                              n_out, c_pad, out_hw[0], out_hw[1], n_seg, 1 if parity_split else 0, _stream()),
+    check(lib.rgbd_dsam_wgrad(g_bf16.data_ptr(), g_lo.data_ptr() if g_lo is not None else None, g_bf16.shape[-1],
+                              xt.data_ptr(), xt_lo.data_ptr() if xt_lo is not None else None, xt.shape[-1], xt.shape[-2],
+                              dw.data_ptr(), B, n_out, c_pad, out_hw[0], out_hw[1], n_seg, 1 if parity_split else 0,
+                              _stream()),
           "rgbd_dsam_wgrad")
     _count(1)
     return dw

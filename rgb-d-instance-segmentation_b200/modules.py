@@ -179,8 +179,14 @@ class DSAModule(_PackedCacheMixin, nn.Module):
 
     #: "bf16": bf16 operands, fp32 accumulate (what torch.autocast gives the reference; ~1e-3 relative).
     #: "fp32": split precision -- activations and weights as bf16 hi + lo parts, three tensor-core products per term
-    #: (~2^-16 relative, inside the 1e-4 fp32 bar) at three times the GEMM work.  Forward only; gradients stay bf16.
+    #: (~2^-16 relative, inside the 1e-4 fp32 bar) at three times the GEMM work.  Forward only: the backward follows
+    #: ``grad_precision``.
     precision = "bf16"
+    #: Operands of the weight and input gradient GEMMs (dW, dx), independent of ``precision``; the forward output does
+    #: not depend on it.  "bf16": bf16 G, x and weights, fp32 accumulate (~2^-8 relative).  "fp32": the same split as the
+    #: forward -- G, x * bit_t and the weights as bf16 hi + lo, products hi.hi + lo.hi + hi.lo (the three terms left out
+    #: are each at most 2^-16 |g||x|) at three times the GEMM work.  dbias and the identity residual are fp32 sums in both.
+    grad_precision = "bf16"
 
     def __init__(self, in_channels, out_channels, num_depth_regions=3):
         super().__init__()
@@ -308,10 +314,18 @@ class DSAModule(_PackedCacheMixin, nn.Module):
         return self._stage_forward_impl(rgb_features, codes, bias_variant, residual)
 
     # ---- backward (K3b) ----------------------------------------------------------------------------
+    def _split_grad(self) -> bool:
+        if self.grad_precision not in ("bf16", "fp32"):
+            raise ValueError(f"DSAModule.grad_precision must be 'bf16' or 'fp32', got {self.grad_precision!r}")
+        return self.grad_precision == "fp32"
+
     def _refresh_bwd(self):
-        """Per input-parity class: transposed weights [(channel block, segment, 32 ch)][(tap, n)] and tap offsets."""
+        """Per input-parity class: transposed weights [(channel block, segment, 32 ch)][(tap, n)] and tap offsets.  Split
+        precision (``grad_precision == "fp32"``): every 64-row K block becomes three, [W_hi | W_hi | W_lo], read against
+        the G planes (hi, lo, hi)."""
         srcs = [p for p in self.parameters()]
-        if not self._ver_bwd.stale(srcs) and self._packed_bwd:
+        split = self._split_grad()
+        if not self._ver_bwd.stale(srcs) and self._packed_bwd and self._packed_bwd.get("split") == split:
             return self._packed_bwd
         dev = srcs[0].device
         c_in, c_out, R = self.in_channels, self.out_channels, self.num_depth_regions
@@ -334,11 +348,19 @@ class DSAModule(_PackedCacheMixin, nn.Module):
                     wt = torch.zeros(c32, np64, device=dev)
                     wt[:c_in, :c_out] = w[:, :, dy, dx].t()                 # (c, n)
                     wd[:, sg, :, ti, :] = wt.reshape(c32 // 32, 32, np64)
-            wd = wd.reshape(c32 // 32 * n_seg * 32, len(taps) * np64).to(torch.bfloat16).contiguous()
-            sl = torch.tensor([(nb * 64, xo, yo, 0) for (dy, yo, dx, xo) in taps for nb in range(np64 // 64)],
+            wd = wd.reshape(c32 // 32 * n_seg * 32, len(taps) * np64)
+            if split:
+                w_hi = wd.reshape(wd.shape[0], len(taps) * np64 // 64, 64).to(torch.bfloat16)
+                w_lo = (wd.reshape(w_hi.shape) - w_hi.float()).to(torch.bfloat16)
+                wd = torch.stack([w_hi, w_hi, w_lo], dim=2).reshape(wd.shape[0], 3 * len(taps) * np64).contiguous()
+                planes = (0, 1, 0)
+            else:
+                wd = wd.to(torch.bfloat16).contiguous()
+                planes = (0,)
+            sl = torch.tensor([(nb * 64, xo, yo, pl) for (dy, yo, dx, xo) in taps for nb in range(np64 // 64) for pl in planes],
                               device=dev, dtype=torch.int32).contiguous()
             classes.append({"py": py, "px": px, "w": wd, "slices": sl})
-        self._packed_bwd = {"classes": classes, "n_seg": n_seg, "c32": c32, "np64": np64}
+        self._packed_bwd = {"classes": classes, "n_seg": n_seg, "c32": c32, "np64": np64, "split": split}
         return self._packed_bwd
 
     def _stage_backward_impl(self, x: torch.Tensor, codes: torch.Tensor, variant: torch.Tensor, g: torch.Tensor, need_dx: bool):
@@ -346,20 +368,24 @@ class DSAModule(_PackedCacheMixin, nn.Module):
         c_pad, kb, n_pad, n_seg = self._geometry()
         B, _, H, W = x.shape
         _, _, Ho, Wo = g.shape
+        split = self._split_grad()
         x = x.detach().contiguous().float()
         # ---- bias gradients: images use the first variant[b] biases
         db = Fn.dsam_dbias(g, variant, R + 1)
-        # ---- weight gradients: GEMM over the output pixels
-        gp = Fn.cast_bf16_pitched(g, _round_up(Wo, 8))
+        # ---- weight gradients: GEMM over the output pixels (split precision: hi and lo parts of both operands)
+        if split:
+            gp, gp_lo = Fn.cast_bf16_pitched(g, _round_up(Wo, 8), lo=True)
+        else:
+            gp, gp_lo = Fn.cast_bf16_pitched(g, _round_up(Wo, 8)), None
         H2, W2 = ((H + 1) // 2, (W + 1) // 2) if self._proj else (H, W)
-        key = (B, H, W, str(x.device))
+        key = (B, H, W, str(x.device), split)
         if key not in self._ws_t:
             _evict(self._ws_t)
-            self._ws_t[key] = torch.zeros(B, n_seg, 6 if self._proj else 1, c_pad, H2, _round_up(W2, 8),
+            self._ws_t[key] = torch.zeros(2 if split else 1, B, n_seg, 6 if self._proj else 1, c_pad, H2, _round_up(W2, 8),
                                           device=x.device, dtype=torch.bfloat16)
-        xt = self._ws_t[key]
-        Fn.dsam_pack_t(x, codes, xt, c_pad, xt.shape[-1], n_seg, R + 1, self._proj)
-        dw = Fn.dsam_wgrad(gp, xt, c_out, c_pad, (Ho, Wo), n_seg, self._proj)       # (c_out, n_seg, taps, c_pad)
+        xt, xt_lo = self._ws_t[key][0], (self._ws_t[key][1] if split else None)
+        Fn.dsam_pack_t(x, codes, xt, c_pad, xt.shape[-1], n_seg, R + 1, self._proj, out_lo=xt_lo)
+        dw = Fn.dsam_wgrad(gp, xt, c_out, c_pad, (Ho, Wo), n_seg, self._proj, g_lo=gp_lo, xt_lo=xt_lo)   # (c_out, n_seg, taps, c_pad)
         k = 3 if self._proj else 1
         grads = []
         for t in range(R + 1):
@@ -372,12 +398,14 @@ class DSAModule(_PackedCacheMixin, nn.Module):
         if need_dx:
             pk = self._refresh_bwd()
             np64 = pk["np64"]
-            gcl = torch.empty(B, Ho, Wo, np64, device=x.device, dtype=torch.bfloat16)
-            Fn.dsam_pack(g, codes.reshape(-1)[:B * Ho * Wo].reshape(B, Ho, Wo), gcl, np64, 1, 0, False)   # plain NCHW -> channels-last
+            n_pl = 2 if split else 1                          # split precision: planes (G_hi, G_lo) per image
+            gcl = torch.empty(B, n_pl, Ho, Wo, np64, device=x.device, dtype=torch.bfloat16)
+            Fn.dsam_pack(g, codes.reshape(-1)[:B * Ho * Wo].reshape(B, Ho, Wo), gcl, np64, 1, 0, False,   # plain NCHW -> channels-last
+                         hi_lo=split)
             dx = torch.empty_like(x)
             direct = g if not self._proj else None            # identity residual (out = enh + F)
             for cl in pk["classes"]:
-                Fn.conv_gemm(gcl, (B, Ho, Wo, np64), 1, cl["w"], cl["slices"], 64, B, (H2, W2), _best_box(H2, W2), c_in, None,
+                Fn.conv_gemm(gcl, (B * n_pl, Ho, Wo, np64), n_pl, cl["w"], cl["slices"], 64, B, (H2, W2), _best_box(H2, W2), c_in, None,
                              epi_mode=3, out=dx, residual=direct, codes=codes, in_hw=(H, W), parity=(cl["py"], cl["px"]),
                              m3_stride=2 if self._proj else 1, m3_masked_segs=R + 1, m3_n_seg=n_seg,
                              block_n=32 * n_seg)
@@ -896,11 +924,14 @@ class DepthGuidance(nn.Module):
     stages -> DGGM injection fused with the branch sum.  Child names match the reference's pixel-level
     module (``ratio_predictor, dsam0, dsam1, dsam2, depth_gradient_injection``)."""
 
-    def __init__(self, color_channels: Sequence[int] = (96, 192, 384, 768), precision: str = "bf16"):
+    def __init__(self, color_channels: Sequence[int] = (96, 192, 384, 768), precision: str = "bf16",
+                 grad_precision: str = "bf16"):
         super().__init__()
         c = list(color_channels)
         assert len(c) == 4
         assert precision in ("bf16", "fp32")
+        if grad_precision not in ("bf16", "fp32"):
+            raise ValueError(f"grad_precision must be 'bf16' or 'fp32', got {grad_precision!r}")
         self.ratio_predictor = EnhancedDepthImageRatioPredictor(3)
         self.dsam0 = DSAModule(in_channels=c[0], out_channels=c[1], num_depth_regions=3)
         self.dsam1 = DSAModule(in_channels=c[1], out_channels=c[2], num_depth_regions=3)
@@ -908,6 +939,7 @@ class DepthGuidance(nn.Module):
         self.depth_gradient_injection = DepthGradientInjectionResidual(c, 3)
         for d in (self.dsam0, self.dsam1, self.dsam2):
             d.precision = precision            # DSAM convolutions; DGGM is fp32 arithmetic in either mode
+            d.grad_precision = grad_precision  # DSAM dW and dx; independent of the forward's precision
 
     def forward(self, pixel_values: torch.Tensor, color_feature_map: Sequence[torch.Tensor],
                 ratios: Optional[torch.Tensor] = None, out: Optional[Sequence[torch.Tensor]] = None) -> List[torch.Tensor]:
