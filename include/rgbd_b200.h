@@ -303,6 +303,18 @@ int rgbd_postprocess_instances(const float* class_logits, const float* mask_logi
                                int Ht, int Wt, float threshold, void* workspace, uint8_t* out_masks, int* out_labels,
                                float* out_scores, int* out_query, int* out_count, int* out_segmentation,
                                rgbd_stream_t stream);
+/* Run-length encoding of int32 label maps, the `return_coco_annotation=True` output of the same HF routine
+ * (`convert_segmentation_to_rle`): for every value present, in ascending order, its maximal runs in row-major order with
+ * 1-based starts.  seg (B,H,W) int32 with labels in [-1, L); label index k = id + 1.  CSR output, no host synchronisation:
+ * offsets (B, L+2): the runs of label k in image b are [offsets[b,k], offsets[b,k+1]) relative to base[b];
+ * base (B+1): exclusive scan of the per-image run totals, so the used runs of the batch are runs[0, base[B]);
+ * runs (B*H*W, 2): (start, end) of each run, 1-based and inclusive (length = end - start + 1);
+ * bad_count (1): pixels whose label lies outside [-1, L); they belong to no run and the caller must check this count.
+ * Deterministic: the output depends on the input alone.  L <= 4096, B <= 65535, B*H*W < 2^31.
+ * workspace: rgbd_label_map_rle_workspace_bytes(B, H, W, L) bytes (0 for invalid arguments). */
+size_t rgbd_label_map_rle_workspace_bytes(int B, int H, int W, int L);
+int rgbd_label_map_rle(const int* seg, int B, int H, int W, int L, void* workspace, int* offsets, int* base, int* runs,
+                       int* bad_count, rgbd_stream_t stream);
 /* Pairwise mask IoU, the core of the evaluator's segm mAP (mask2former/utils/model_essential_part.py:111-170 through
  * torchmetrics): pred (P,pixels) and gt (G,pixels) bytes 0/1 -> iou (P,G) fp32 (0 where the union is empty). */
 int rgbd_mask_iou(const uint8_t* pred_masks, const uint8_t* gt_masks, int P, int G, long long pixels, float* iou,

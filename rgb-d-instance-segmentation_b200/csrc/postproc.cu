@@ -16,6 +16,7 @@
 //                               bitmap written by pass 2), and the painted segmentation map (id of the last kept segment
 //                               covering a pixel)
 // The 384x384 upsampled logits (59 MB per image for 100 queries) are never materialised.
+// rgbd_label_map_rle: run-length encoding of the painted map (HF `return_coco_annotation=True`) in four sync-free passes.
 // rgbd_mask_iou: pairwise mask IoU (the evaluator's torchmetrics `iou_type="segm"` core) with 16-byte loads + popcount.
 // Compiled with -fmad=false: the interpolation is written as separate multiplies and adds like ATen's kernel.
 #include "common.cuh"
@@ -370,6 +371,199 @@ __global__ void __launch_bounds__(256) postproc_paint_kernel(PostGeom g, const i
     }
 }
 
+// ---- run-length encoding of int32 label maps (HF `convert_segmentation_to_rle`: per value present, ascending, the maximal
+// row-major runs as [start_1, len_1, ...] with 1-based starts).  Label k = id + 1 of id in [-1, L).  Each warp owns a subtile
+// of kRleSub consecutive pixels of one image and walks it in rounds of 32 pixels, lane order = pixel order.  A run STARTS at p
+// when p == 0 or seg[p-1] != seg[p] and ENDS at p when p == N-1 or seg[p+1] != seg[p].
+//   1. rle_count_kernel  starts per (label, subtile) -> table (B, K, n_sub); pixels outside [-1, L) are counted and skipped
+//   2. rle_scan_kernel   per image, exclusive scan of the table in label-major (label, subtile) order, in place: the first
+//                        start of label k in subtile s goes to slot table[b,k,s] relative to the image; offsets (B, K+1)
+//   3. rle_base_kernel   exclusive scan of the per-image totals -> base (B+1)
+//   4. rle_emit_kernel   slot of a start = cursor + (same-label starts in the lower lanes); the end of a run at p takes
+//                        (starts of its label at positions <= p) - 1, so a start and its end meet in one slot even when they
+//                        fall in different subtiles.  The cursor per (label, subtile) is owned by one warp: no atomics decide
+//                        an order, and the output depends on the input alone.
+constexpr int kRleWarps = 4;
+constexpr int kRleRounds = 32;
+constexpr int kRleSub = 32 * kRleRounds;        // pixels per warp
+constexpr int kRleMaxLabels = 4096;
+
+__device__ __forceinline__ bool rle_label(int v, int L, int& k) {
+    k = v + 1;
+    return v >= -1 && v < L;
+}
+
+__global__ void __launch_bounds__(kRleWarps * 32) rle_count_kernel(const int* __restrict__ seg, int N, int K, int n_sub,
+                                                                   int* __restrict__ table, int* __restrict__ bad) {
+    extern __shared__ int s_rle[];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int s = blockIdx.x * kRleWarps + warp, b = blockIdx.y;
+    if (s >= n_sub) return;
+    int* hist = s_rle + warp * K;
+    for (int k = lane; k < K; k += 32) hist[k] = 0;
+    __syncwarp();
+    const int* img = seg + (size_t)b * N;
+    unsigned n_bad = 0;
+    for (int r = 0; r < kRleRounds; ++r) {
+        const int p = s * kRleSub + r * 32 + lane;
+        if (s * kRleSub + r * 32 >= N) break;                      // warp-uniform
+        int k = -1;
+        bool start = false, ok = false;
+        if (p < N) {
+            const int v = __ldg(img + p);
+            ok = rle_label(v, K - 1, k);
+            start = ok && (p == 0 || __ldg(img + p - 1) != v);
+        }
+        n_bad += __popc(__ballot_sync(0xffffffffu, p < N && !ok));
+        if (!__ballot_sync(0xffffffffu, start)) continue;         // most rounds of a real map: no run starts here
+        // one key for every lane that takes no part: __match_any_sync costs grow with the number of distinct keys
+        const unsigned grp = __match_any_sync(0xffffffffu, start ? k : -1);
+        if (start && (__ffs(grp) - 1) == lane) hist[k] += __popc(grp);
+        __syncwarp();
+    }
+    __syncwarp();
+    for (int k = lane; k < K; k += 32) table[((size_t)b * K + k) * n_sub + s] = hist[k];
+    if (lane == 0 && n_bad) atomicAdd(bad, (int)n_bad);            // a count, not an order
+}
+
+constexpr int kScanThreads = 1024;
+constexpr int kScanItems = 8;
+
+// Exclusive scan of one value per thread over a block of kScanThreads threads; `total` = the block's sum in every thread.
+// Ends with a barrier, so s_warp (kScanThreads / 32 ints) can be reused by the next call.
+__device__ __forceinline__ int block_exclusive_scan(int x, int* s_warp, int& total) {
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    int incl = x;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const int y = __shfl_up_sync(0xffffffffu, incl, d);
+        if (lane >= d) incl += y;
+    }
+    if (lane == 31) s_warp[warp] = incl;
+    __syncthreads();
+    if (warp == 0) {
+        int w = s_warp[lane];
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const int y = __shfl_up_sync(0xffffffffu, w, d);
+            if (lane >= d) w += y;
+        }
+        s_warp[lane] = w;
+    }
+    __syncthreads();
+    const int ex = (warp ? s_warp[warp - 1] : 0) + incl - x;
+    total = s_warp[kScanThreads / 32 - 1];
+    __syncthreads();
+    return ex;
+}
+
+__global__ void __launch_bounds__(kScanThreads) rle_scan_kernel(int K, int n_sub, int* __restrict__ table,
+                                                                int* __restrict__ offsets) {
+    __shared__ int s_warp[kScanThreads / 32];
+    const int b = blockIdx.x;
+    const long long M = (long long)K * n_sub;
+    int* t = table + (size_t)b * M;
+    int* off = offsets + (size_t)b * (K + 1);
+    int carry = 0;
+    for (long long c0 = 0; c0 < M; c0 += (long long)kScanThreads * kScanItems) {
+        const long long i0 = c0 + (long long)threadIdx.x * kScanItems;
+        int v[kScanItems], sum = 0;
+#pragma unroll
+        for (int e = 0; e < kScanItems; ++e) {
+            v[e] = i0 + e < M ? t[i0 + e] : 0;
+            sum += v[e];
+        }
+        int total;
+        int run = carry + block_exclusive_scan(sum, s_warp, total);
+#pragma unroll
+        for (int e = 0; e < kScanItems; ++e) {
+            const long long i = i0 + e;
+            if (i < M) {
+                t[i] = run;
+                if (i % n_sub == 0) off[i / n_sub] = run;
+            }
+            run += v[e];
+        }
+        carry += total;
+    }
+    if (threadIdx.x == 0) off[K] = carry;
+}
+
+__global__ void __launch_bounds__(kScanThreads) rle_base_kernel(int B, int K, const int* __restrict__ offsets,
+                                                                int* __restrict__ base) {
+    __shared__ int s_warp[kScanThreads / 32];
+    int carry = 0;
+    for (int c0 = 0; c0 < B; c0 += kScanThreads) {
+        const int i = c0 + threadIdx.x;
+        int total;
+        const int ex = block_exclusive_scan(i < B ? offsets[(size_t)i * (K + 1) + K] : 0, s_warp, total);
+        if (i < B) base[i] = carry + ex;
+        carry += total;
+    }
+    if (threadIdx.x == 0) base[B] = carry;
+}
+
+__global__ void __launch_bounds__(kRleWarps * 32) rle_emit_kernel(const int* __restrict__ seg, int N, int K, int n_sub,
+                                                                  const int* __restrict__ table, const int* __restrict__ base,
+                                                                  int2* __restrict__ runs) {
+    extern __shared__ int s_rle[];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int s = blockIdx.x * kRleWarps + warp, b = blockIdx.y;
+    if (s >= n_sub) return;
+    int* cur = s_rle + warp * K;
+    const int b0 = base[b];
+    for (int k = lane; k < K; k += 32) cur[k] = b0 + table[((size_t)b * K + k) * n_sub + s];
+    __syncwarp();
+    const int* img = seg + (size_t)b * N;
+    const unsigned le = 0xffffffffu >> (31 - lane);                // lanes <= this one
+    for (int r = 0; r < kRleRounds; ++r) {
+        const int p = s * kRleSub + r * 32 + lane;
+        if (s * kRleSub + r * 32 >= N) break;                      // warp-uniform
+        int k = -1;
+        bool start = false, end = false;
+        if (p < N) {
+            const int v = __ldg(img + p);
+            if (rle_label(v, K - 1, k)) {
+                start = p == 0 || __ldg(img + p - 1) != v;
+                end = p == N - 1 || __ldg(img + p + 1) != v;
+            }
+        }
+        if (!__ballot_sync(0xffffffffu, start || end)) continue;  // warp-uniform: nothing to write this round
+        const unsigned grp = __match_any_sync(0xffffffffu, (start || end) ? k : -1);
+        const unsigned starts = grp & __ballot_sync(0xffffffffu, start);
+        int c = 0;
+        if (start || end) {
+            c = cur[k];
+            const int slot = c + __popc(starts & le) - 1;
+            if (start) runs[slot].x = p + 1;
+            if (end) runs[slot].y = p + 1;
+        }
+        __syncwarp();
+        if ((start || end) && (__ffs(grp) - 1) == lane) cur[k] = c + __popc(starts);
+        __syncwarp();
+    }
+}
+
+struct RleLayout {
+    int K, n_sub;
+    size_t table, total;
+};
+
+// The argument rules of rgbd_label_map_rle; the workspace query applies them too (0 bytes = invalid).
+bool rle_args_ok(int B, int H, int W, int L) {
+    return B >= 1 && H >= 1 && W >= 1 && L >= 0 && L <= kRleMaxLabels && B <= 65535 &&
+           (long long)B * H * W < (1ll << 31);
+}
+
+RleLayout rle_layout(int B, int H, int W, int L) {   // valid arguments only (rle_args_ok)
+    RleLayout l;
+    l.K = L + 1;
+    l.n_sub = ceil_div(H * W, kRleSub);
+    l.table = 0;
+    l.total = ((size_t)B * l.K * l.n_sub * 4 + 255) / 256 * 256;
+    return l;
+}
+
 __global__ void __launch_bounds__(256) fill_int_kernel(int* __restrict__ p, size_t n, int v) {
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) p[i] = v;
 }
@@ -528,6 +722,42 @@ extern "C" int rgbd_postprocess_instances(const float* class_logits, const float
     RGBD_CHECK_LAUNCH();
     RGBD_CHECK_ARG(B <= 65535, "postprocess: at most 65535 images per call");
     postproc_paint_kernel<<<dim3(ceil_div(Ht * Wt, 256 * 4), B), 256, 0, s>>>(g, inv_slot, out_count, bitmap, out_masks, out_segmentation);
+    RGBD_CHECK_LAUNCH();
+    return RGBD_OK;
+}
+
+extern "C" size_t rgbd_label_map_rle_workspace_bytes(int B, int H, int W, int L) {
+    return rle_args_ok(B, H, W, L) ? rle_layout(B, H, W, L).total : 0;
+}
+
+extern "C" int rgbd_label_map_rle(const int* seg, int B, int H, int W, int L, void* workspace, int* offsets, int* base,
+                                  int* runs, int* bad_count, rgbd_stream_t stream) {
+    RGBD_CHECK_ARG(seg && workspace && offsets && base && runs && bad_count, "label_map_rle: null pointer");
+    RGBD_CHECK_ARG(B >= 1 && H >= 1 && W >= 1, "label_map_rle: bad geometry B=%d H=%d W=%d", B, H, W);
+    RGBD_CHECK_ARG(L >= 0 && L <= kRleMaxLabels, "label_map_rle: L = %d labels outside [0, %d]", L, kRleMaxLabels);
+    RGBD_CHECK_ARG((long long)B * H * W < (1ll << 31), "label_map_rle: B*H*W must be below 2^31");
+    RGBD_CHECK_ARG(B <= 65535, "label_map_rle: at most 65535 images per call");
+    cudaStream_t s = (cudaStream_t)stream;
+    const RleLayout l = rle_layout(B, H, W, L);
+    const int N = H * W;
+    int* table = reinterpret_cast<int*>(reinterpret_cast<uint8_t*>(workspace) + l.table);
+    const size_t smem = (size_t)kRleWarps * l.K * sizeof(int);
+    RgbdDeviceInfo di;
+    if (int rc = rgbd_device_info(&di)) return rc;
+    RGBD_ONCE_PER_DEVICE(di.device, {
+        const int cap = kRleWarps * (kRleMaxLabels + 1) * (int)sizeof(int);
+        RGBD_CHECK_CUDA(cudaFuncSetAttribute(rle_count_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, cap));
+        RGBD_CHECK_CUDA(cudaFuncSetAttribute(rle_emit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, cap));
+    });
+    const dim3 grid(ceil_div(l.n_sub, kRleWarps), B);
+    RGBD_CHECK_CUDA(cudaMemsetAsync(bad_count, 0, sizeof(int), s));
+    rle_count_kernel<<<grid, kRleWarps * 32, smem, s>>>(seg, N, l.K, l.n_sub, table, bad_count);
+    RGBD_CHECK_LAUNCH();
+    rle_scan_kernel<<<B, kScanThreads, 0, s>>>(l.K, l.n_sub, table, offsets);
+    RGBD_CHECK_LAUNCH();
+    rle_base_kernel<<<1, kScanThreads, 0, s>>>(B, l.K, offsets, base);
+    RGBD_CHECK_LAUNCH();
+    rle_emit_kernel<<<grid, kRleWarps * 32, smem, s>>>(seg, N, l.K, l.n_sub, table, base, reinterpret_cast<int2*>(runs));
     RGBD_CHECK_LAUNCH();
     return RGBD_OK;
 }

@@ -832,6 +832,67 @@ def post_process_instances(class_logits: torch.Tensor, mask_logits: torch.Tensor
     return InstanceBatch(masks, labels, scores, query, count, seg)
 
 
+@dataclass
+class RunLengths:
+    """Device-side result of ``label_map_rle`` (CSR).  The runs of label ``k = id + 1`` in image ``b`` are
+    ``runs[base[b] + offsets[b, k] : base[b] + offsets[b, k + 1]]``; the batch uses ``runs[:base[B]]``."""
+    offsets: torch.Tensor              # (B, L+2) i32, relative to the image's base
+    base: torch.Tensor                 # (B+1,) i32
+    runs: torch.Tensor                 # (B*H*W, 2) i32: (start, end), 1-based, end inclusive
+    bad: torch.Tensor                  # (1,) i32: pixels whose label lies outside [-1, L)
+
+
+def _rle_workspace_bytes(B: int, H: int, W: int, L: int) -> int:
+    ws_bytes = int(_lib.load().rgbd_label_map_rle_workspace_bytes(B, H, W, L))
+    if ws_bytes == 0:
+        raise RgbdB200Error(f"label_map_rle: unsupported shape (B,H,W)={(B, H, W)} or label count {L} "
+                            "(at most 4096 labels, 65535 images, B*H*W < 2^31)")
+    return ws_bytes
+
+
+def _rle_outputs(B: int, H: int, W: int, L: int, device) -> RunLengths:
+    i32 = dict(device=device, dtype=torch.int32)
+    return RunLengths(torch.empty(B, L + 2, **i32), torch.empty(B + 1, **i32), torch.empty(B * H * W, 2, **i32),
+                      torch.empty(1, **i32))
+
+
+def label_map_rle_buffers(B: int, H: int, W: int, n_labels: int, device) -> Tuple[RunLengths, torch.Tensor]:
+    """Output tensors and workspace of ``label_map_rle`` for (B,H,W) maps, to pass as ``out`` / ``workspace``."""
+    ws_bytes = _rle_workspace_bytes(B, H, W, int(n_labels))          # checks the arguments before anything is allocated
+    return _rle_outputs(B, H, W, int(n_labels), device), torch.empty(ws_bytes, device=device, dtype=torch.uint8)
+
+
+def label_map_rle(seg: torch.Tensor, n_labels: int, out: Optional[RunLengths] = None,
+                  workspace: Optional[torch.Tensor] = None) -> RunLengths:
+    """Run-length encoding of (B,H,W) int32 label maps with labels in [-1, n_labels) (HF ``convert_segmentation_to_rle``
+    per image), without host synchronisation.  Out-of-range pixels are counted in ``bad``, never encoded: check it.
+    ``out`` / ``workspace`` (from ``label_map_rle_buffers``) are used in place when given; either one may be given alone."""
+    lib = _lib.load()
+    _req(seg, "seg", torch.int32)
+    if seg.dim() != 3:
+        raise RgbdB200Error("label_map_rle: expected a (B,H,W) int32 label map")
+    B, H, W = seg.shape
+    L = int(n_labels)
+    ws_bytes = _rle_workspace_bytes(B, H, W, L)
+    if out is None:
+        out = _rle_outputs(B, H, W, L, seg.device)
+    if workspace is None:
+        workspace = torch.empty(ws_bytes, device=seg.device, dtype=torch.uint8)
+    want = [(out.offsets, (B, L + 2)), (out.base, (B + 1,)), (out.runs, (B * H * W, 2)), (out.bad, (1,))]
+    for t, shape in want:
+        _req(t, "label_map_rle output", torch.int32)
+        if tuple(t.shape) != shape:
+            raise RgbdB200Error(f"label_map_rle: output of shape {tuple(t.shape)}, expected {shape}")
+    _req(workspace, "label_map_rle workspace", torch.uint8)
+    if workspace.numel() < ws_bytes:
+        raise RgbdB200Error("label_map_rle: workspace too small")
+    check(lib.rgbd_label_map_rle(seg.data_ptr(), B, H, W, L, workspace.data_ptr(), out.offsets.data_ptr(),
+                                 out.base.data_ptr(), out.runs.data_ptr(), out.bad.data_ptr(), _stream()),
+          "rgbd_label_map_rle")
+    _count(4)                                           # count, scan, base, emit
+    return out
+
+
 def mask_iou(pred_masks: torch.Tensor, gt_masks: torch.Tensor) -> torch.Tensor:
     """(P,H,W) x (G,H,W) 0/1 masks (bool or uint8) -> (P,G) float32 IoU."""
     lib = _lib.load()

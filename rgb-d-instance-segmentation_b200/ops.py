@@ -141,6 +141,22 @@ def _(class_logits, mask_logits, threshold, target_h, target_w):
             e((B, Q), dtype=torch.int32), e((B,), dtype=torch.int32), e((B, target_h, target_w), dtype=torch.int32)]
 
 
+@torch.library.custom_op(f"{NAMESPACE}::label_map_rle", mutates_args=())
+def label_map_rle(seg: Tensor, n_labels: int) -> List[Tensor]:
+    """HF ``convert_segmentation_to_rle`` per image of (B,H,W) int32 maps, as CSR: [offsets (B,L+2), base (B+1), runs
+    (B*H*W,2) 1-based inclusive (start, end), out-of-range pixel count (1)]."""
+    r = Fn.label_map_rle(seg, n_labels)
+    return [r.offsets, r.base, r.runs, r.bad]
+
+
+@label_map_rle.register_fake
+def _(seg, n_labels):
+    B, H, W = seg.shape
+    e = seg.new_empty
+    i32 = dict(dtype=torch.int32)
+    return [e((B, n_labels + 2), **i32), e((B + 1,), **i32), e((B * H * W, 2), **i32), e((1,), **i32)]
+
+
 @torch.library.custom_op(f"{NAMESPACE}::mask_iou", mutates_args=())
 def mask_iou(pred_masks: Tensor, gt_masks: Tensor) -> Tensor:
     """(P,H,W) x (G,H,W) 0/1 masks -> (P,G) IoU (segm mAP of model_essential_part.py:111-170)."""
@@ -213,5 +229,5 @@ def _(x, weight, bias, eps, bf16_out=False):
 
 
 REGISTERED = ("dggm_forward", "dggm_backward_params", "gradient_features", "pack_pixel_values", "to_grayscale",
-              "depth_decompose", "post_process_instances", "mask_iou", "msda_forward", "attention_mask", "window_attention",
+              "depth_decompose", "post_process_instances", "label_map_rle", "mask_iou", "msda_forward", "attention_mask", "window_attention",
               "masked_cross_attention", "layer_norm")

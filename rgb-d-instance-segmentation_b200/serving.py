@@ -8,6 +8,8 @@ What ``predictor.predictor`` / ``process_prediction`` do per image in the refere
            hot path CM:324-355 on this library's kernels; by default also the two decoder_ops kernels inside the stock
            decoders: deformable-attention sampling and the masked-attention mask)
         -> device post-processing (K5)  --D2H-->  pinned segmentation map + per-segment labels / scores / counts
+           (``return_coco_annotation=True``: the map is run-length encoded on the device, and only the small CSR tables,
+           then the used runs, are copied)
 
 The device part of a step is replayed as one CUDA graph per staging buffer (``cuda_graph``), so the host only issues two copies
 and a graph launch per batch.  Only ~1.2 MB per 480x640 frame crosses the host link on the way in and the painted instance map on the way out; encoder
@@ -56,7 +58,7 @@ class RgbdInstanceSegmenter:
 
     def __init__(self, model, batch: int, frame_hw: Tuple[int, int], threshold: float = 0.5,
                  target_size: Optional[Tuple[int, int]] = None, autocast_dtype: Optional[torch.dtype] = torch.bfloat16,
-                 fast_decoder_ops: bool = True, cuda_graph: Optional[bool] = None):
+                 fast_decoder_ops: bool = True, cuda_graph: Optional[bool] = None, return_coco_annotation: bool = False):
         p = next(model.parameters())
         if not p.is_cuda:
             raise RgbdB200Error("RgbdInstanceSegmenter: the model must live on a CUDA device (no CPU path)")
@@ -96,17 +98,38 @@ class RgbdInstanceSegmenter:
                         torch.empty(B, H, W, dtype=torch.uint8, device=dev)) for _ in range(2)]
         self.pv = [torch.empty(B, 10, H, W, dtype=torch.float32, device=dev) for _ in range(2)]
         self.out_dev: List[Optional[Fn.InstanceBatch]] = [None, None]
-        self.out_host = [{"segmentation": torch.empty(B, Ht, Wt, dtype=torch.int32).pin_memory(),
+        #: HF's run-length lists instead of painted maps: the maps are encoded inside the step (and its graph), the
+        #: download carries only the small CSR tables, and ``result`` copies the used runs.  The encoder's outputs and
+        #: workspace are allocated here, outside the graphs' shared memory pool: ``result`` reads a buffer's runs after the
+        #: other buffer's graph has started, and that graph may reuse whatever memory the first one freed during capture.
+        self.return_coco_annotation = bool(return_coco_annotation)
+        self.rle_dev = [Fn.label_map_rle_buffers(B, Ht, Wt, Q, dev) for _ in range(2)] if return_coco_annotation else None
+        if self.return_coco_annotation:
+            tables = {"offsets": torch.empty(B, Q + 2, dtype=torch.int32), "base": torch.empty(B + 1, dtype=torch.int32),
+                      "bad": torch.empty(1, dtype=torch.int32)}
+        else:
+            tables = {"segmentation": torch.empty(B, Ht, Wt, dtype=torch.int32)}
+        self.out_host = [{**{k: v.pin_memory() for k, v in tables.items()},
                           "labels": torch.empty(B, Q, dtype=torch.int32).pin_memory(),
                           "scores": torch.empty(B, Q, dtype=torch.float32).pin_memory(),
                           "count": torch.empty(B, dtype=torch.int32).pin_memory()} for _ in range(2)]
         self.s_in, self.s_out = torch.cuda.Stream(device=dev), torch.cuda.Stream(device=dev)
+        self.s_runs = torch.cuda.Stream(device=dev) if self.return_coco_annotation else None
+        self._runs_host: Optional[torch.Tensor] = None      # pinned, grown on demand, reused by every ``result``
         self.h2d_bytes_per_step = B * H * W * 4
-        self.d2h_bytes_per_step = sum(t.numel() * t.element_size() for t in self.out_host[0].values())
+        self._table_d2h_bytes = sum(t.numel() * t.element_size() for t in self.out_host[0].values())
+        #: bytes of runs the last ``result`` copied (8 per run; 0 with ``return_coco_annotation`` off)
+        self.runs_d2h_bytes = 0
         self._ev_in = [None, None]
         self._ev_free = [None, None]
         self._ev_d2h = [None, None]
         self._step = 0
+
+    @property
+    def d2h_bytes_per_step(self) -> int:
+        """Bytes copied device -> host per step: the pinned download of the step, plus, with ``return_coco_annotation``,
+        the runs of the step whose ``result`` was read last (the run count depends on the frames)."""
+        return self._table_d2h_bytes + self.runs_d2h_bytes
 
     # ---- one device step ---------------------------------------------------------------------------
     @property
@@ -155,6 +178,8 @@ class RgbdInstanceSegmenter:
             self.out_dev[b] = Fn.post_process_instances(out.class_queries_logits.float().contiguous(),
                                                         out.masks_queries_logits.float().contiguous(),
                                                         self.threshold, self.target, want_segmentation=True)
+            if self.return_coco_annotation:
+                Fn.label_map_rle(self.out_dev[b].segmentation, self.Q, *self.rle_dev[b])
 
     def submit(self, rgb_u8: Optional[torch.Tensor] = None, depth_u8: Optional[torch.Tensor] = None) -> int:
         """Enqueue one batch (host uint8 tensors (B,H,W,3) / (B,H,W); ``None`` re-sends what the staging buffer holds).
@@ -183,7 +208,13 @@ class RgbdInstanceSegmenter:
         with torch.cuda.stream(self.s_out):
             self.s_out.wait_event(self._ev_free[b])
             oh = self.out_host[b]
-            oh["segmentation"].copy_(r.segmentation, non_blocking=True)
+            if self.return_coco_annotation:
+                e = self.rle_dev[b][0]
+                oh["offsets"].copy_(e.offsets, non_blocking=True)
+                oh["base"].copy_(e.base, non_blocking=True)
+                oh["bad"].copy_(e.bad, non_blocking=True)
+            else:
+                oh["segmentation"].copy_(r.segmentation, non_blocking=True)
             oh["labels"].copy_(r.labels, non_blocking=True)
             oh["scores"].copy_(r.scores, non_blocking=True)
             oh["count"].copy_(r.count, non_blocking=True)
@@ -200,10 +231,29 @@ class RgbdInstanceSegmenter:
     def result(self, b: int, copy: bool = True) -> List[Dict]:
         """HF-shaped results of buffer ``b`` (``post_process_instance_segmentation`` return structure, PR:701-703).  The pinned
         staging buffer is reused by the second-next ``submit``: the maps are copied out unless ``copy=False`` (then they are
-        views that stay valid only until that submit)."""
+        views that stay valid only until that submit).
+
+        With ``return_coco_annotation`` "segmentation" is HF's run-length list of lists, and this call copies the used runs
+        of buffer ``b`` from the device (8 bytes per run) after the table download.  That is valid only because ``result(b)``
+        is called before the second-next ``submit``, which would overwrite them: the same rule as for the staging buffers."""
         self._ev_d2h[b].synchronize()
         oh = self.out_host[b]
-        seg = oh["segmentation"].clone() if copy else oh["segmentation"]
+        if self.return_coco_annotation:
+            if int(oh["bad"][0]):
+                raise RgbdB200Error(f"RgbdInstanceSegmenter: {int(oh['bad'][0])} painted pixels outside [-1, {self.Q})")
+            n_runs = int(oh["base"][self.B])
+            if self._runs_host is None or self._runs_host.shape[0] < n_runs:
+                cap = max(n_runs, 2 * (0 if self._runs_host is None else self._runs_host.shape[0]), 1)
+                self._runs_host = torch.empty(cap, 2, dtype=torch.int32).pin_memory()
+            runs = self._runs_host[:n_runs]
+            with torch.cuda.stream(self.s_runs):       # not behind the next step's work on the main / download streams
+                runs.copy_(self.rle_dev[b][0].runs[:n_runs], non_blocking=True)
+            self.s_runs.synchronize()
+            self.runs_d2h_bytes = n_runs * 8
+            from .postprocess import rle_lists_from_csr
+            seg = rle_lists_from_csr(oh["offsets"].numpy(), oh["base"].numpy(), runs.numpy())
+        else:
+            seg = oh["segmentation"].clone() if copy else oh["segmentation"]
         res = []
         for i in range(self.B):
             n = int(oh["count"][i])
