@@ -315,6 +315,20 @@ int rgbd_postprocess_instances(const float* class_logits, const float* mask_logi
 size_t rgbd_label_map_rle_workspace_bytes(int B, int H, int W, int L);
 int rgbd_label_map_rle(const int* seg, int B, int H, int W, int L, void* workspace, int* offsets, int* base, int* runs,
                        int* bad_count, rgbd_stream_t stream);
+/* pycocotools RLE of every kept segment of a painted map: segment s of image b (s < count[b]) gets exactly the "counts"
+ * string of `pycocotools.mask.encode(np.asfortranarray((seg[b] == s).astype(np.uint8)))`, size [H, W]: column-major
+ * counts, alternating 0-runs and 1-runs and starting with 0-runs, compressed by `rleToString` (ASCII 48..111).
+ * seg (B,H,W) int32 with ids in [-1, L), -1 = background; count (B) int32.  CSR output, no host synchronisation:
+ * offsets (B, L+1): segment s's characters are chars[base[b] + offsets[b,s], base[b] + offsets[b,s+1]); segments
+ * s >= count[b] are empty; base (B+1): exclusive scan of the per-image character totals;
+ * chars (rgbd_instance_rle_capacity(B, H, W, L)) bytes; bad_count (1): pixels whose id lies outside [-1, L) or in
+ * [count[b], L), plus 1 per image whose count lies outside [0, L] (that image gets no segments).  The caller must check it.
+ * Deterministic: the output depends on the input alone.  L <= 4096, B <= 65535, 7*B*(2*H*W + L) < 2^31.
+ * workspace: rgbd_instance_rle_workspace_bytes(B, H, W, L) bytes; both queries return 0 for invalid arguments. */
+size_t rgbd_instance_rle_workspace_bytes(int B, int H, int W, int L);
+size_t rgbd_instance_rle_capacity(int B, int H, int W, int L);
+int rgbd_instance_rle(const int* seg, const int* count, int B, int H, int W, int L, void* workspace, int* offsets, int* base,
+                      uint8_t* chars, int* bad_count, rgbd_stream_t stream);
 /* Pairwise mask IoU, the core of the evaluator's segm mAP (mask2former/utils/model_essential_part.py:111-170 through
  * torchmetrics): pred (P,pixels) and gt (G,pixels) bytes 0/1 -> iou (P,G) fp32 (0 where the union is empty). */
 int rgbd_mask_iou(const uint8_t* pred_masks, const uint8_t* gt_masks, int P, int G, long long pixels, float* iou,

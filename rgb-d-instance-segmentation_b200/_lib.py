@@ -93,6 +93,9 @@ SIGNATURES = {
     "rgbd_postprocess_instances": (C.c_int, [C.c_void_p, C.c_void_p] + [C.c_int] * 7 + [C.c_float] + [C.c_void_p] * 8),
     "rgbd_label_map_rle_workspace_bytes": (C.c_size_t, [C.c_int] * 4),
     "rgbd_label_map_rle": (C.c_int, [C.c_void_p] + [C.c_int] * 4 + [C.c_void_p] * 6),
+    "rgbd_instance_rle_workspace_bytes": (C.c_size_t, [C.c_int] * 4),
+    "rgbd_instance_rle_capacity": (C.c_size_t, [C.c_int] * 4),
+    "rgbd_instance_rle": (C.c_int, [C.c_void_p] * 2 + [C.c_int] * 4 + [C.c_void_p] * 6),
     "rgbd_mask_iou": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_longlong, C.c_void_p, C.c_void_p]),
     "rgbd_ratio_tail": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, c_void_pp, c_void_pp,
                                   C.c_float, C.c_float, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),

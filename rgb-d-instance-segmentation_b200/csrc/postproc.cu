@@ -17,6 +17,8 @@
 //                               covering a pixel)
 // The 384x384 upsampled logits (59 MB per image for 100 queries) are never materialised.
 // rgbd_label_map_rle: run-length encoding of the painted map (HF `return_coco_annotation=True`) in four sync-free passes.
+// rgbd_instance_rle: pycocotools' compressed RLE string of every kept segment, from the same encoder run on the transposed
+// map, then a size, scan, base and emit pass over the runs; no host synchronisation either.
 // rgbd_mask_iou: pairwise mask IoU (the evaluator's torchmetrics `iou_type="segm"` core) with 16-byte loads + popcount.
 // Compiled with -fmad=false: the interpolation is written as separate multiplies and adds like ATen's kernel.
 #include "common.cuh"
@@ -564,6 +566,219 @@ RleLayout rle_layout(int B, int H, int W, int L) {   // valid arguments only (rl
     return l;
 }
 
+// ---- pycocotools RLE of the segments of a painted map (`pycocotools.mask.encode` of (map == s) in Fortran order, then
+// `rleToString`).  The map is transposed, so the label-major runs the rle_* kernels find in it are the 1-runs of each
+// segment in column-major order (position q = x*H + y).  Then, per image, one ITEM per run plus one TAIL item per
+// segment s in [0, L): with the image's run indices j counted from o1 = (its first non-background run), run j of segment s
+// is item (j - o1 + s) and the tail of s is item (offsets_r[s+2] - o1 + s), so items are placed without a search.
+// Run m of a segment gives counts 2m (zeros before it) and 2m+1 (its length); the tail gives count 2R = h*w - end_{R-1}
+// when that is > 0 (the whole [h*w] of an empty segment).  Each item reads its run and the two before it in the segment,
+// which is all the string's deltas (x - c[i-2] for i > 2) need, so a segment with h*w/2 runs is spread over threads.
+//   coco_transpose_kernel  (B,H,W) -> (B,W,H), 32x32 shared tiles with a padded row
+//   rgbd_label_map_rle     the four rle_* kernels on the transposed map, into the workspace
+//   coco_size_kernel       characters per item -> pos (B, H*W + L); run lengths of segments s >= count[b] -> bad
+//   coco_scan_kernel       per image, exclusive scan of pos in place over its items; total -> offsets[b, L]
+//   rle_base_kernel        exclusive scan of the per-image totals -> base (B+1)
+//   coco_emit_kernel       writes each item's characters at base[b] + pos; the first item of s writes offsets[b, s]
+constexpr int kCocoTile = 32;
+constexpr int kCocoThreads = 256;
+
+__global__ void __launch_bounds__(kCocoTile * 8) coco_transpose_kernel(const int* __restrict__ seg, int H, int W,
+                                                                       int tiles_w, int* __restrict__ seg_t) {
+    __shared__ int tile[kCocoTile][kCocoTile + 1];                 // +1: the column reads hit 32 different banks
+    const int b = blockIdx.y;
+    const int ty = blockIdx.x / tiles_w, tx = blockIdx.x - ty * tiles_w;
+    const int* src = seg + (size_t)b * H * W;
+    int* dst = seg_t + (size_t)b * H * W;
+    const int x = tx * kCocoTile + threadIdx.x;
+    for (int r = threadIdx.y; r < kCocoTile; r += 8) {
+        const int y = ty * kCocoTile + r;
+        if (y < H && x < W) tile[r][threadIdx.x] = __ldg(src + (size_t)y * W + x);
+    }
+    __syncthreads();
+    const int y = ty * kCocoTile + threadIdx.x;
+    for (int r = threadIdx.y; r < kCocoTile; r += 8) {
+        const int xo = tx * kCocoTile + r;
+        if (xo < W && y < H) dst[(size_t)xo * H + y] = tile[threadIdx.x][r];
+    }
+}
+
+// rleToString: 5-bit groups, low bits first, 0x20 = more follow, +48.  Returns the number of characters; writes them when
+// `out` is given.
+__device__ __forceinline__ int coco_put(int x, uint8_t* out) {
+    int n = 0;
+    bool more = true;
+    while (more) {
+        int c = x & 0x1f;
+        x >>= 5;                                                   // arithmetic: negative deltas end at x == -1
+        more = (c & 0x10) ? x != -1 : x != 0;
+        if (more) c |= 0x20;
+        if (out) out[n] = (uint8_t)(c + 48);
+        ++n;
+    }
+    return n;
+}
+
+// The counts of item t of image b as (up to) two string values, in order.  Returns the number of values (0, 1 or 2) and
+// sets the segment, whether this is the segment's first item, and the length of the run (0 for a tail).
+struct CocoItem {
+    int n_val, val[2], s, item, run_len;
+    bool first;
+};
+
+__device__ __forceinline__ CocoItem coco_item(int t, int N, int L, const int* __restrict__ off_r, const int2* __restrict__ runs,
+                                              const int* __restrict__ img_t) {
+    CocoItem it;
+    const int o1 = off_r[1], n_runs = off_r[L + 1] - o1;
+    int m, R;                                                      // run index in the segment; runs of the segment
+    int2 cur = make_int2(0, 0);
+    if (t < n_runs) {
+        cur = runs[o1 + t];
+        it.s = __ldg(img_t + cur.x - 1);
+        m = o1 + t - off_r[it.s + 1];
+        R = m + 1;
+        it.item = t + it.s;
+        it.run_len = cur.y - cur.x + 1;
+    } else {
+        it.s = t - n_runs;
+        R = off_r[it.s + 2] - off_r[it.s + 1];
+        m = R;                                                     // the tail sits where run R would
+        it.item = off_r[it.s + 2] - o1 + it.s;
+        it.run_len = 0;
+    }
+    it.first = m == 0;
+    const int j0 = off_r[it.s + 1];                                // run m of the segment is runs[j0 + m]
+    const int2 p1 = m >= 1 ? runs[j0 + m - 1] : make_int2(0, 0);
+    const int2 p2 = m >= 2 ? runs[j0 + m - 2] : make_int2(0, 0);
+    const int gap1 = p1.x - 1 - p2.y;                              // zeros before run m-1 (count 2m-2), when m >= 1
+    if (t < n_runs) {
+        const int gap = cur.x - 1 - p1.y;                          // count 2m
+        it.val[0] = m >= 2 ? gap - gap1 : gap;                     // delta when 2m > 2
+        it.val[1] = m >= 1 ? it.run_len - (p1.y - p1.x + 1) : it.run_len;   // count 2m+1: delta when 2m+1 > 2
+        it.n_val = 2;
+    } else {
+        const int tail = N - p1.y;                                 // count 2R: trailing zeros, h*w for an empty segment
+        it.val[0] = R >= 2 ? tail - gap1 : tail;
+        it.n_val = tail > 0 ? 1 : 0;
+    }
+    return it;
+}
+
+// image b's valid segment count: count[b] when it lies in [0, L], else 0 (and coco_scan_kernel counts it in bad)
+__device__ __forceinline__ int coco_n_segments(const int* __restrict__ count, int b, int L) {
+    const int n = count[b];
+    return n >= 0 && n <= L ? n : 0;
+}
+
+__global__ void __launch_bounds__(kCocoThreads) coco_size_kernel(int N, int L, const int* __restrict__ count,
+                                                                 const int* __restrict__ off_r, const int* __restrict__ base_r,
+                                                                 const int2* __restrict__ runs, const int* __restrict__ seg_t,
+                                                                 int* __restrict__ pos, int* __restrict__ bad) {
+    const int b = blockIdx.y;
+    const int t = blockIdx.x * kCocoThreads + threadIdx.x;
+    const int* o = off_r + (size_t)b * (L + 2);
+    const int n_items = o[L + 1] - o[1] + L;
+    int n_bad = 0;
+    if (t < n_items) {
+        const CocoItem it = coco_item(t, N, L, o, runs + base_r[b], seg_t + (size_t)b * N);
+        int n = 0;
+        if (it.s < coco_n_segments(count, b, L)) {
+#pragma unroll
+            for (int v = 0; v < 2; ++v) n += v < it.n_val ? coco_put(it.val[v], nullptr) : 0;
+        } else {
+            n_bad = it.run_len;                                    // painted pixels of an id >= count[b]
+        }
+        pos[(size_t)b * (N + L) + it.item] = n;
+    }
+#pragma unroll
+    for (int k = 16; k > 0; k >>= 1) n_bad += __shfl_xor_sync(0xffffffffu, n_bad, k);
+    if ((threadIdx.x & 31) == 0 && n_bad) atomicAdd(bad, n_bad);    // a count, not an order
+}
+
+// rle_scan_kernel's pattern over the image's items only: a checkerboard has ~h*w/2 of them, a real map a few per column
+__global__ void __launch_bounds__(kScanThreads) coco_scan_kernel(int N, int L, const int* __restrict__ count,
+                                                                 const int* __restrict__ off_r, int* __restrict__ pos,
+                                                                 int* __restrict__ offsets, int* __restrict__ bad) {
+    __shared__ int s_warp[kScanThreads / 32];
+    const int b = blockIdx.x;
+    const int* o = off_r + (size_t)b * (L + 2);
+    const int n_items = o[L + 1] - o[1] + L;
+    int* p = pos + (size_t)b * (N + L);
+    int carry = 0;
+    for (int c0 = 0; c0 < n_items; c0 += kScanThreads * kScanItems) {
+        const int i0 = c0 + threadIdx.x * kScanItems;
+        int v[kScanItems], sum = 0;
+#pragma unroll
+        for (int e = 0; e < kScanItems; ++e) {
+            v[e] = i0 + e < n_items ? p[i0 + e] : 0;
+            sum += v[e];
+        }
+        int total;
+        int run = carry + block_exclusive_scan(sum, s_warp, total);
+#pragma unroll
+        for (int e = 0; e < kScanItems; ++e) {
+            if (i0 + e < n_items) p[i0 + e] = run;
+            run += v[e];
+        }
+        carry += total;
+    }
+    if (threadIdx.x == 0) {
+        offsets[(size_t)b * (L + 1) + L] = carry;
+        if (count[b] < 0 || count[b] > L) atomicAdd(bad, 1);
+    }
+}
+
+__global__ void __launch_bounds__(kCocoThreads) coco_emit_kernel(int N, int L, const int* __restrict__ count,
+                                                                 const int* __restrict__ off_r, const int* __restrict__ base_r,
+                                                                 const int2* __restrict__ runs, const int* __restrict__ seg_t,
+                                                                 const int* __restrict__ pos, const int* __restrict__ base,
+                                                                 int* __restrict__ offsets, uint8_t* __restrict__ chars) {
+    const int b = blockIdx.y;
+    const int t = blockIdx.x * kCocoThreads + threadIdx.x;
+    const int* o = off_r + (size_t)b * (L + 2);
+    if (t >= o[L + 1] - o[1] + L) return;
+    const CocoItem it = coco_item(t, N, L, o, runs + base_r[b], seg_t + (size_t)b * N);
+    const int at = pos[(size_t)b * (N + L) + it.item];
+    if (it.first) offsets[(size_t)b * (L + 1) + it.s] = at;
+    if (it.s >= coco_n_segments(count, b, L)) return;
+    uint8_t* dst = chars + base[b] + at;
+#pragma unroll
+    for (int v = 0; v < 2; ++v) dst += v < it.n_val ? coco_put(it.val[v], dst) : 0;
+}
+
+struct CocoLayout {
+    RleLayout rle;
+    size_t seg_t, rle_ws, off_r, base_r, runs, pos, total;
+};
+
+// The argument rules of rgbd_instance_rle: those of rgbd_label_map_rle, and the character capacity (a count takes at most 7
+// characters, an image at most 2*H*W + L counts) must index with int32.
+bool coco_args_ok(int B, int H, int W, int L) {
+    return rle_args_ok(B, H, W, L) && 7ll * B * (2ll * H * W + L) < (1ll << 31);
+}
+
+size_t coco_capacity(int B, int H, int W, int L) { return 7ull * B * (2ull * H * W + L); }
+
+CocoLayout coco_layout(int B, int H, int W, int L) {   // valid arguments only (coco_args_ok)
+    CocoLayout l;
+    l.rle = rle_layout(B, W, H, L);
+    const size_t N = (size_t)H * W;
+    size_t o = 0;
+    auto take = [&](size_t bytes) {
+        const size_t at = o;
+        o += (bytes + 255) / 256 * 256;
+        return at;
+    };
+    l.seg_t = take((size_t)B * N * 4);
+    l.rle_ws = take(l.rle.total);
+    l.off_r = take((size_t)B * (L + 2) * 4);
+    l.base_r = take((size_t)(B + 1) * 4);
+    l.runs = take((size_t)B * N * 8);
+    l.pos = take((size_t)B * (N + L) * 4);
+    l.total = o;
+    return l;
+}
+
 __global__ void __launch_bounds__(256) fill_int_kernel(int* __restrict__ p, size_t n, int v) {
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) p[i] = v;
 }
@@ -758,6 +973,48 @@ extern "C" int rgbd_label_map_rle(const int* seg, int B, int H, int W, int L, vo
     rle_base_kernel<<<1, kScanThreads, 0, s>>>(B, l.K, offsets, base);
     RGBD_CHECK_LAUNCH();
     rle_emit_kernel<<<grid, kRleWarps * 32, smem, s>>>(seg, N, l.K, l.n_sub, table, base, reinterpret_cast<int2*>(runs));
+    RGBD_CHECK_LAUNCH();
+    return RGBD_OK;
+}
+
+extern "C" size_t rgbd_instance_rle_workspace_bytes(int B, int H, int W, int L) {
+    return coco_args_ok(B, H, W, L) ? coco_layout(B, H, W, L).total : 0;
+}
+
+extern "C" size_t rgbd_instance_rle_capacity(int B, int H, int W, int L) {
+    return coco_args_ok(B, H, W, L) ? coco_capacity(B, H, W, L) : 0;
+}
+
+extern "C" int rgbd_instance_rle(const int* seg, const int* count, int B, int H, int W, int L, void* workspace, int* offsets,
+                                 int* base, uint8_t* chars, int* bad_count, rgbd_stream_t stream) {
+    RGBD_CHECK_ARG(seg && count && workspace && offsets && base && chars && bad_count, "instance_rle: null pointer");
+    RGBD_CHECK_ARG(B >= 1 && H >= 1 && W >= 1, "instance_rle: bad geometry B=%d H=%d W=%d", B, H, W);
+    RGBD_CHECK_ARG(L >= 0 && L <= kRleMaxLabels, "instance_rle: L = %d labels outside [0, %d]", L, kRleMaxLabels);
+    RGBD_CHECK_ARG(B <= 65535, "instance_rle: at most 65535 images per call");
+    RGBD_CHECK_ARG(coco_args_ok(B, H, W, L), "instance_rle: 7*B*(2*H*W + L) characters must be below 2^31");
+    cudaStream_t s = (cudaStream_t)stream;
+    const CocoLayout l = coco_layout(B, H, W, L);
+    uint8_t* ws = reinterpret_cast<uint8_t*>(workspace);
+    int* seg_t = reinterpret_cast<int*>(ws + l.seg_t);
+    int* off_r = reinterpret_cast<int*>(ws + l.off_r);
+    int* base_r = reinterpret_cast<int*>(ws + l.base_r);
+    int* runs = reinterpret_cast<int*>(ws + l.runs);
+    int* pos = reinterpret_cast<int*>(ws + l.pos);
+    const int N = H * W;
+    const int tiles_w = ceil_div(W, kCocoTile);
+    coco_transpose_kernel<<<dim3(tiles_w * ceil_div(H, kCocoTile), B), dim3(kCocoTile, 8), 0, s>>>(seg, H, W, tiles_w, seg_t);
+    RGBD_CHECK_LAUNCH();
+    // the column-major runs: the label encoder on the (W, H) maps; it zeroes bad_count and counts ids outside [-1, L)
+    if (int rc = rgbd_label_map_rle(seg_t, B, W, H, L, ws + l.rle_ws, off_r, base_r, runs, bad_count, stream)) return rc;
+    const dim3 grid(ceil_div(N + L, kCocoThreads), B);
+    const int2* runs2 = reinterpret_cast<const int2*>(runs);
+    coco_size_kernel<<<grid, kCocoThreads, 0, s>>>(N, L, count, off_r, base_r, runs2, seg_t, pos, bad_count);
+    RGBD_CHECK_LAUNCH();
+    coco_scan_kernel<<<B, kScanThreads, 0, s>>>(N, L, count, off_r, pos, offsets, bad_count);
+    RGBD_CHECK_LAUNCH();
+    rle_base_kernel<<<1, kScanThreads, 0, s>>>(B, L, offsets, base);
+    RGBD_CHECK_LAUNCH();
+    coco_emit_kernel<<<grid, kCocoThreads, 0, s>>>(N, L, count, off_r, base_r, runs2, seg_t, pos, base, offsets, chars);
     RGBD_CHECK_LAUNCH();
     return RGBD_OK;
 }

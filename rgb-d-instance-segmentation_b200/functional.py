@@ -893,6 +893,75 @@ def label_map_rle(seg: torch.Tensor, n_labels: int, out: Optional[RunLengths] = 
     return out
 
 
+@dataclass
+class InstanceRle:
+    """Device-side result of ``instance_rle`` (CSR).  The pycocotools "counts" string of segment ``s`` of image ``b`` is
+    ``chars[base[b] + offsets[b, s] : base[b] + offsets[b, s + 1]]``; the batch uses ``chars[:base[B]]``."""
+    offsets: torch.Tensor              # (B, L+1) i32, relative to the image's base
+    base: torch.Tensor                 # (B+1,) i32
+    chars: torch.Tensor                # (capacity,) u8, ASCII 48..111
+    bad: torch.Tensor                  # (1,) i32: pixels outside [-1, L) or in [count[b], L), +1 per count outside [0, L]
+
+
+def _instance_rle_sizes(B: int, H: int, W: int, L: int) -> Tuple[int, int]:
+    lib = _lib.load()
+    ws_bytes = int(lib.rgbd_instance_rle_workspace_bytes(B, H, W, L))
+    capacity = int(lib.rgbd_instance_rle_capacity(B, H, W, L))
+    if ws_bytes == 0 or capacity == 0:
+        raise RgbdB200Error(f"instance_rle: unsupported shape (B,H,W)={(B, H, W)} or label count {L} "
+                            "(at most 4096 labels, 65535 images, 7*B*(2*H*W + L) < 2^31)")
+    return ws_bytes, capacity
+
+
+def _instance_rle_outputs(B: int, L: int, capacity: int, device) -> InstanceRle:
+    i32 = dict(device=device, dtype=torch.int32)
+    return InstanceRle(torch.empty(B, L + 1, **i32), torch.empty(B + 1, **i32),
+                       torch.empty(capacity, device=device, dtype=torch.uint8), torch.empty(1, **i32))
+
+
+def instance_rle_buffers(B: int, H: int, W: int, n_labels: int, device) -> Tuple[InstanceRle, torch.Tensor]:
+    """Output tensors and workspace of ``instance_rle`` for (B,H,W) maps, to pass as ``out`` / ``workspace``."""
+    ws_bytes, capacity = _instance_rle_sizes(B, H, W, int(n_labels))   # checks the arguments before anything is allocated
+    return (_instance_rle_outputs(B, int(n_labels), capacity, device),
+            torch.empty(ws_bytes, device=device, dtype=torch.uint8))
+
+
+def instance_rle(seg: torch.Tensor, count: torch.Tensor, n_labels: int, out: Optional[InstanceRle] = None,
+                 workspace: Optional[torch.Tensor] = None) -> InstanceRle:
+    """pycocotools RLE of the kept segments of (B,H,W) int32 painted maps, without host synchronisation: segment
+    ``s < count[b]`` gets the "counts" string of ``pycocotools.mask.encode(np.asfortranarray(seg[b] == s))``.  Pixels
+    outside [-1, n_labels) or in [count[b], n_labels) are counted in ``bad``, never encoded: check it.
+    ``out`` / ``workspace`` (from ``instance_rle_buffers``) are used in place when given; either one may be given alone."""
+    lib = _lib.load()
+    _req(seg, "seg", torch.int32)
+    _req(count, "count", torch.int32)
+    if seg.dim() != 3:
+        raise RgbdB200Error("instance_rle: expected a (B,H,W) int32 label map")
+    B, H, W = seg.shape
+    if tuple(count.shape) != (B,):
+        raise RgbdB200Error(f"instance_rle: count of shape {tuple(count.shape)}, expected {(B,)}")
+    L = int(n_labels)
+    ws_bytes, capacity = _instance_rle_sizes(B, H, W, L)
+    if out is None:
+        out = _instance_rle_outputs(B, L, capacity, seg.device)
+    if workspace is None:
+        workspace = torch.empty(ws_bytes, device=seg.device, dtype=torch.uint8)
+    want = [(out.offsets, (B, L + 1), torch.int32), (out.base, (B + 1,), torch.int32),
+            (out.chars, (capacity,), torch.uint8), (out.bad, (1,), torch.int32)]
+    for t, shape, dtype in want:
+        _req(t, "instance_rle output", dtype)
+        if tuple(t.shape) != shape:
+            raise RgbdB200Error(f"instance_rle: output of shape {tuple(t.shape)}, expected {shape}")
+    _req(workspace, "instance_rle workspace", torch.uint8)
+    if workspace.numel() < ws_bytes:
+        raise RgbdB200Error("instance_rle: workspace too small")
+    check(lib.rgbd_instance_rle(seg.data_ptr(), count.data_ptr(), B, H, W, L, workspace.data_ptr(),
+                                out.offsets.data_ptr(), out.base.data_ptr(), out.chars.data_ptr(), out.bad.data_ptr(),
+                                _stream()), "rgbd_instance_rle")
+    _count(9)                                           # transpose, 4 x rle_*, size, scan, base, emit
+    return out
+
+
 def mask_iou(pred_masks: torch.Tensor, gt_masks: torch.Tensor) -> torch.Tensor:
     """(P,H,W) x (G,H,W) 0/1 masks (bool or uint8) -> (P,G) float32 IoU."""
     lib = _lib.load()

@@ -157,6 +157,23 @@ def _(seg, n_labels):
     return [e((B, n_labels + 2), **i32), e((B + 1,), **i32), e((B * H * W, 2), **i32), e((1,), **i32)]
 
 
+@torch.library.custom_op(f"{NAMESPACE}::instance_rle", mutates_args=())
+def instance_rle(seg: Tensor, count: Tensor, n_labels: int) -> List[Tensor]:
+    """pycocotools RLE strings of the kept segments of (B,H,W) int32 painted maps, as CSR: [offsets (B,L+1), base (B+1),
+    chars (7*B*(2*H*W+L),) uint8, bad pixel count (1)]."""
+    r = Fn.instance_rle(seg, count, n_labels)
+    return [r.offsets, r.base, r.chars, r.bad]
+
+
+@instance_rle.register_fake
+def _(seg, count, n_labels):
+    B, H, W = seg.shape
+    e = seg.new_empty
+    i32 = dict(dtype=torch.int32)
+    return [e((B, n_labels + 1), **i32), e((B + 1,), **i32), e((7 * B * (2 * H * W + n_labels),), dtype=torch.uint8),
+            e((1,), **i32)]
+
+
 @torch.library.custom_op(f"{NAMESPACE}::mask_iou", mutates_args=())
 def mask_iou(pred_masks: Tensor, gt_masks: Tensor) -> Tensor:
     """(P,H,W) x (G,H,W) 0/1 masks -> (P,G) IoU (segm mAP of model_essential_part.py:111-170)."""
@@ -229,5 +246,5 @@ def _(x, weight, bias, eps, bf16_out=False):
 
 
 REGISTERED = ("dggm_forward", "dggm_backward_params", "gradient_features", "pack_pixel_values", "to_grayscale",
-              "depth_decompose", "post_process_instances", "label_map_rle", "mask_iou", "msda_forward", "attention_mask", "window_attention",
+              "depth_decompose", "post_process_instances", "label_map_rle", "instance_rle", "mask_iou", "msda_forward", "attention_mask", "window_attention",
               "masked_cross_attention", "layer_norm")

@@ -61,17 +61,74 @@ def _download_with_rle(r: "Fn.InstanceBatch", n_labels: int):
     return count.tolist(), labels.view(n, Q), scores.view(torch.float32).view(n, Q), rle
 
 
+def pycocotools_rle_from_csr(offsets, base, chars, count, size) -> List[List[Dict]]:
+    """pycocotools RLEs from the CSR tables of ``functional.instance_rle`` on the host: ``offsets`` (n, L+1) relative to
+    ``base`` (>= n entries), ``chars`` the used prefix of the characters (uint8 array or bytes), ``count`` the kept segments
+    per image and ``size`` the maps' (h, w).  Per image one ``{"size": [h, w], "counts": bytes}`` per segment, in id order:
+    what ``pycocotools.mask.encode`` returns for ``np.asfortranarray(map == s)``."""
+    offsets = np.asarray(offsets, dtype=np.int64)
+    base = np.asarray(base, dtype=np.int64)
+    buf = chars if isinstance(chars, bytes) else np.ascontiguousarray(chars, dtype=np.uint8).tobytes()
+    hw = [int(size[0]), int(size[1])]
+    out = []
+    for b in range(offsets.shape[0]):
+        bounds = (base[b] + offsets[b, :int(count[b]) + 1]).tolist()
+        out.append([{"size": list(hw), "counts": buf[lo:hi]} for lo, hi in zip(bounds[:-1], bounds[1:])])
+    return out
+
+
+def _download_with_pycocotools_rle(r: "Fn.InstanceBatch", n_labels: int, size):
+    """Encode the kept segments of ``r`` on the device, then read the small tables in one copy and the used characters in
+    one more.  Returns (count list, labels (n,Q), scores (n,Q), per-image pycocotools RLE lists)."""
+    n, Q = r.labels.shape
+    enc = Fn.instance_rle(r.segmentation, r.count, n_labels)
+    tables = torch.cat([r.count, r.labels.reshape(-1), r.scores.reshape(-1).view(torch.int32), enc.offsets.reshape(-1),
+                        enc.base, enc.bad]).cpu()   # the one synchronisation of the batch
+    sizes = [n, n * Q, n * Q, enc.offsets.numel(), n + 1, 1]
+    count, labels, scores, offsets, base, bad = torch.split(tables, sizes)
+    if int(bad[0]):
+        raise RgbdB200Error(f"post_process_instance_segmentation: {int(bad[0])} painted pixels outside the kept segments")
+    chars = enc.chars[:int(base[n])].cpu()
+    count = count.tolist()
+    rle = pycocotools_rle_from_csr(offsets.view(n, -1).numpy(), base.numpy(), chars.numpy(), count, size)
+    return count, labels.view(n, Q), scores.view(torch.float32).view(n, Q), rle
+
+
+def coco_results(results: Sequence[Dict], image_ids: Sequence[int]) -> List[Dict]:
+    """The COCO results list of ``results`` (from ``post_process_instance_segmentation(return_pycocotools_rle=True)`` or
+    ``RgbdInstanceSegmenter(return_pycocotools_rle=True).result``), one entry per segment, ready for ``json.dump`` and
+    ``COCO.loadRes``: ``{"image_id", "category_id", "segmentation": {"size", "counts": str}, "score"}``.  "category_id" is
+    the model's ``label_id``; mapping it to a dataset's category ids is the caller's."""
+    if len(results) != len(image_ids):
+        raise ValueError(f"coco_results: {len(results)} results for {len(image_ids)} image ids")
+    out = []
+    for res, image_id in zip(results, image_ids):
+        if len(res["segmentation"]) != len(res["segments_info"]):
+            raise ValueError("coco_results: expected one pycocotools RLE per segment (return_pycocotools_rle=True)")
+        for rle, info in zip(res["segmentation"], res["segments_info"]):
+            out.append({"image_id": image_id, "category_id": info["label_id"],
+                        "segmentation": {"size": list(rle["size"]), "counts": rle["counts"].decode("ascii")},
+                        "score": info["score"]})
+    return out
+
+
 def post_process_instance_segmentation(outputs, threshold: float = 0.5, mask_threshold: float = 0.5,
                                        overlap_mask_area_threshold: float = 0.8,
                                        target_sizes: Optional[Sequence[Tuple[int, int]]] = None,
                                        return_coco_annotation: bool = False,
-                                       return_binary_maps: bool = False) -> List[Dict]:
+                                       return_binary_maps: bool = False,
+                                       return_pycocotools_rle: bool = False) -> List[Dict]:
     """Drop-in for ``image_processor.post_process_instance_segmentation``.  ``mask_threshold`` and
     ``overlap_mask_area_threshold`` are accepted and unused, exactly as in HF's instance routine.
     ``return_coco_annotation=True`` returns HF's ``convert_segmentation_to_rle`` of the painted map as "segmentation": one
-    run-length list per value present (ascending, so -1 first when there is background), encoded on the device."""
+    run-length list per value present (ascending, so -1 first when there is background), encoded on the device.
+    ``return_pycocotools_rle=True`` (not an HF option) returns, as "segmentation", one pycocotools RLE
+    ``{"size": [h, w], "counts": bytes}`` per segment of ``segments_info``, equal to ``pycocotools.mask.encode`` of
+    (painted map == id) and encoded on the device; ``coco_results`` turns such results into a COCO results list."""
     if return_coco_annotation and return_binary_maps:
         raise ValueError("return_coco_annotation and return_binary_maps can not be both set to True.")
+    if return_pycocotools_rle and (return_coco_annotation or return_binary_maps):
+        raise ValueError("return_pycocotools_rle can not be combined with return_coco_annotation or return_binary_maps.")
     cls = outputs.class_queries_logits
     msk = outputs.masks_queries_logits
     if not (cls.is_cuda and msk.is_cuda):
@@ -90,6 +147,8 @@ def post_process_instance_segmentation(outputs, threshold: float = 0.5, mask_thr
                                       threshold, size, want_segmentation=not return_binary_maps)
         if return_coco_annotation:
             count, labels, scores, rle = _download_with_rle(r, msk.shape[1])
+        elif return_pycocotools_rle:
+            count, labels, scores, rle = _download_with_pycocotools_rle(r, msk.shape[1], size)
         else:
             count = r.count.cpu().tolist()             # the one synchronisation of the batch
             labels, scores = r.labels.cpu(), r.scores.cpu()
@@ -97,7 +156,7 @@ def post_process_instance_segmentation(outputs, threshold: float = 0.5, mask_thr
             n = count[k]
             info = [{"id": j, "label_id": int(labels[k, j]), "was_fused": False, "score": round(float(scores[k, j]), 6)}
                     for j in range(n)]
-            if return_coco_annotation:
+            if return_coco_annotation or return_pycocotools_rle:
                 seg = rle[k]
             elif return_binary_maps and n:
                 seg = r.masks[k, :n].float()

@@ -9,7 +9,8 @@ What ``predictor.predictor`` / ``process_prediction`` do per image in the refere
            decoders: deformable-attention sampling and the masked-attention mask)
         -> device post-processing (K5)  --D2H-->  pinned segmentation map + per-segment labels / scores / counts
            (``return_coco_annotation=True``: the map is run-length encoded on the device, and only the small CSR tables,
-           then the used runs, are copied)
+           then the used runs, are copied; ``return_pycocotools_rle=True``: the same with pycocotools' compressed strings, one
+           per segment, instead of runs)
 
 The device part of a step is replayed as one CUDA graph per staging buffer (``cuda_graph``), so the host only issues two copies
 and a graph launch per batch.  Only ~1.2 MB per 480x640 frame crosses the host link on the way in and the painted instance map on the way out; encoder
@@ -58,7 +59,10 @@ class RgbdInstanceSegmenter:
 
     def __init__(self, model, batch: int, frame_hw: Tuple[int, int], threshold: float = 0.5,
                  target_size: Optional[Tuple[int, int]] = None, autocast_dtype: Optional[torch.dtype] = torch.bfloat16,
-                 fast_decoder_ops: bool = True, cuda_graph: Optional[bool] = None, return_coco_annotation: bool = False):
+                 fast_decoder_ops: bool = True, cuda_graph: Optional[bool] = None, return_coco_annotation: bool = False,
+                 return_pycocotools_rle: bool = False):
+        if return_coco_annotation and return_pycocotools_rle:
+            raise ValueError("return_coco_annotation and return_pycocotools_rle can not be both set to True.")
         p = next(model.parameters())
         if not p.is_cuda:
             raise RgbdB200Error("RgbdInstanceSegmenter: the model must live on a CUDA device (no CPU path)")
@@ -103,9 +107,17 @@ class RgbdInstanceSegmenter:
         #: workspace are allocated here, outside the graphs' shared memory pool: ``result`` reads a buffer's runs after the
         #: other buffer's graph has started, and that graph may reuse whatever memory the first one freed during capture.
         self.return_coco_annotation = bool(return_coco_annotation)
-        self.rle_dev = [Fn.label_map_rle_buffers(B, Ht, Wt, Q, dev) for _ in range(2)] if return_coco_annotation else None
-        if self.return_coco_annotation:
-            tables = {"offsets": torch.empty(B, Q + 2, dtype=torch.int32), "base": torch.empty(B + 1, dtype=torch.int32),
+        #: ``return_pycocotools_rle``: the same scheme with one pycocotools RLE string per segment, and ``result`` copies the
+        #: used characters.
+        self.return_pycocotools_rle = bool(return_pycocotools_rle)
+        self.rle_dev = None
+        if return_coco_annotation:
+            self.rle_dev = [Fn.label_map_rle_buffers(B, Ht, Wt, Q, dev) for _ in range(2)]
+        elif return_pycocotools_rle:
+            self.rle_dev = [Fn.instance_rle_buffers(B, Ht, Wt, Q, dev) for _ in range(2)]
+        if self.rle_dev is not None:
+            n_off = Q + 2 if return_coco_annotation else Q + 1
+            tables = {"offsets": torch.empty(B, n_off, dtype=torch.int32), "base": torch.empty(B + 1, dtype=torch.int32),
                       "bad": torch.empty(1, dtype=torch.int32)}
         else:
             tables = {"segmentation": torch.empty(B, Ht, Wt, dtype=torch.int32)}
@@ -114,11 +126,13 @@ class RgbdInstanceSegmenter:
                           "scores": torch.empty(B, Q, dtype=torch.float32).pin_memory(),
                           "count": torch.empty(B, dtype=torch.int32).pin_memory()} for _ in range(2)]
         self.s_in, self.s_out = torch.cuda.Stream(device=dev), torch.cuda.Stream(device=dev)
-        self.s_runs = torch.cuda.Stream(device=dev) if self.return_coco_annotation else None
+        self.s_runs = torch.cuda.Stream(device=dev) if self.rle_dev is not None else None
         self._runs_host: Optional[torch.Tensor] = None      # pinned, grown on demand, reused by every ``result``
+        self._chars_host: Optional[torch.Tensor] = None     # the same for ``return_pycocotools_rle``
         self.h2d_bytes_per_step = B * H * W * 4
         self._table_d2h_bytes = sum(t.numel() * t.element_size() for t in self.out_host[0].values())
-        #: bytes of runs the last ``result`` copied (8 per run; 0 with ``return_coco_annotation`` off)
+        #: bytes the last ``result`` copied after the tables: 8 per run with ``return_coco_annotation``, 1 per character
+        #: with ``return_pycocotools_rle``, 0 with both off
         self.runs_d2h_bytes = 0
         self._ev_in = [None, None]
         self._ev_free = [None, None]
@@ -127,8 +141,9 @@ class RgbdInstanceSegmenter:
 
     @property
     def d2h_bytes_per_step(self) -> int:
-        """Bytes copied device -> host per step: the pinned download of the step, plus, with ``return_coco_annotation``,
-        the runs of the step whose ``result`` was read last (the run count depends on the frames)."""
+        """Bytes copied device -> host per step: the pinned download of the step, plus, with ``return_coco_annotation``
+        or ``return_pycocotools_rle``, the runs or characters of the step whose ``result`` was read last (their number
+        depends on the frames)."""
         return self._table_d2h_bytes + self.runs_d2h_bytes
 
     # ---- one device step ---------------------------------------------------------------------------
@@ -180,6 +195,8 @@ class RgbdInstanceSegmenter:
                                                         self.threshold, self.target, want_segmentation=True)
             if self.return_coco_annotation:
                 Fn.label_map_rle(self.out_dev[b].segmentation, self.Q, *self.rle_dev[b])
+            elif self.return_pycocotools_rle:
+                Fn.instance_rle(self.out_dev[b].segmentation, self.out_dev[b].count, self.Q, *self.rle_dev[b])
 
     def submit(self, rgb_u8: Optional[torch.Tensor] = None, depth_u8: Optional[torch.Tensor] = None) -> int:
         """Enqueue one batch (host uint8 tensors (B,H,W,3) / (B,H,W); ``None`` re-sends what the staging buffer holds).
@@ -208,7 +225,7 @@ class RgbdInstanceSegmenter:
         with torch.cuda.stream(self.s_out):
             self.s_out.wait_event(self._ev_free[b])
             oh = self.out_host[b]
-            if self.return_coco_annotation:
+            if self.rle_dev is not None:
                 e = self.rle_dev[b][0]
                 oh["offsets"].copy_(e.offsets, non_blocking=True)
                 oh["base"].copy_(e.base, non_blocking=True)
@@ -235,7 +252,9 @@ class RgbdInstanceSegmenter:
 
         With ``return_coco_annotation`` "segmentation" is HF's run-length list of lists, and this call copies the used runs
         of buffer ``b`` from the device (8 bytes per run) after the table download.  That is valid only because ``result(b)``
-        is called before the second-next ``submit``, which would overwrite them: the same rule as for the staging buffers."""
+        is called before the second-next ``submit``, which would overwrite them: the same rule as for the staging buffers.
+        With ``return_pycocotools_rle`` "segmentation" is one ``{"size": [h, w], "counts": bytes}`` per segment, and this
+        call copies the used characters of buffer ``b`` under the same rule (1 byte per character)."""
         self._ev_d2h[b].synchronize()
         oh = self.out_host[b]
         if self.return_coco_annotation:
@@ -252,6 +271,21 @@ class RgbdInstanceSegmenter:
             self.runs_d2h_bytes = n_runs * 8
             from .postprocess import rle_lists_from_csr
             seg = rle_lists_from_csr(oh["offsets"].numpy(), oh["base"].numpy(), runs.numpy())
+        elif self.return_pycocotools_rle:
+            if int(oh["bad"][0]):
+                raise RgbdB200Error(f"RgbdInstanceSegmenter: {int(oh['bad'][0])} painted pixels outside the kept segments")
+            n_chars = int(oh["base"][self.B])
+            if self._chars_host is None or self._chars_host.shape[0] < n_chars:
+                cap = max(n_chars, 2 * (0 if self._chars_host is None else self._chars_host.shape[0]), 1)
+                self._chars_host = torch.empty(cap, dtype=torch.uint8).pin_memory()
+            chars = self._chars_host[:n_chars]
+            with torch.cuda.stream(self.s_runs):       # not behind the next step's work on the main / download streams
+                chars.copy_(self.rle_dev[b][0].chars[:n_chars], non_blocking=True)
+            self.s_runs.synchronize()
+            self.runs_d2h_bytes = n_chars
+            from .postprocess import pycocotools_rle_from_csr
+            seg = pycocotools_rle_from_csr(oh["offsets"].numpy(), oh["base"].numpy(), chars.numpy(), oh["count"].tolist(),
+                                           self.target)
         else:
             seg = oh["segmentation"].clone() if copy else oh["segmentation"]
         res = []
